@@ -6,6 +6,7 @@ on a synthetic GTDB-representatives-shaped reference database (BASELINE.json con
     python bench.py --gpus N --steps K --warmup W                  # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W # the reference's CPU core (oracle/_ref)
     torchrun ... bench.py --gpus N ...                             # N > 1: one rank per GPU (NCCL)
+    python bench.py ... --dump-outputs DIR                         # + the last resident step's results as DIR/*.npy
 
 One "step" = one pass of the hot path over the whole database:
   value : sketches already resident in HBM -> ygpu_build_index + ygpu_pairwise_flag (+ NCCL gather
@@ -123,7 +124,7 @@ def independent_counts_torch(d_hashes, torch):
 
 # ------------------------------------------------------------------------------------------------
 # CPU arm: the reference core (oracle/_ref) -- or the oracle port when that binary is absent.
-#   --impl reference : ONE run of the unmodified reference executable on the FULL configuration (same genomes, same
+#   --impl reference : --steps runs of the unmodified reference executable on the FULL configuration (same genomes, same
 #                      seed as the GPU arm): the database is written as signature files and the stock CLI is run with
 #                      every host thread.  Throughput counts the phases that correspond to the GPU arm's e2e step (host
 #                      buffers -> pair list + retained set): its own index + matrix + greedy timers; its JSON read
@@ -192,7 +193,8 @@ def reference_cache_key(args, binary: str, cores: int) -> str:
         stamp = f"{os.path.getsize(binary)}:{int(os.path.getmtime(binary))}"
     except OSError:
         stamp = "?"
-    return f"genomes={args.genomes} seed={args.seed} cpu_sample={args.cpu_sample} thr={THR!r} cores={cores} binary={stamp}"
+    return (f"genomes={args.genomes} seed={args.seed} cpu_sample={args.cpu_sample} steps={args.steps} thr={THR!r} cores={cores} "
+            f"binary={stamp}")
 
 
 def run_reference_arm(args):
@@ -230,13 +232,17 @@ def run_reference_arm(args):
     try:
         if not full:
             passes = 1
-        ph, wall = cpu_arm_step(tmp, binary, cores, passes)          # ONE run: a second one would only repeat ~minutes of CPU work
-        per = (ph.get("index_ms", 0) + ph.get("matrix_ms", 0) + ph.get("greedy_ms", 0)) / 1e3 if ph else wall
+        # --steps timed runs (each minutes of CPU at full size), no warm-up; the phase timers are averaged over the runs
+        runs = [cpu_arm_step(tmp, binary, cores, passes) for _ in range(args.steps)]
+        ph = {k: sum(r[0].get(k, 0) for r in runs) / len(runs) for k in runs[-1][0]}
+        wall = sum(r[1] for r in runs) / len(runs)
+        per =(ph.get("index_ms", 0) + ph.get("matrix_ms", 0) + ph.get("greedy_ms", 0)) / 1e3 if ph else wall
         pairs = n_s * (n_s - 1)
         val = pairs / per if per > 0 else 0.0
         cfg = workload_config(args, db)
         sample = (f"{'ALL' if full else 'first'} {n_s} of {n} genomes (file order), all-vs-all, {os.path.basename(binary)} -t {cores} -p {passes}, "
-                  f"one run (steps_run = 1, no warm-up: a run is minutes of CPU); time = its own index+matrix+greedy phase timers "
+                  f"{args.steps} run(s) (steps_run = {args.steps}, no warm-up: a run is minutes of CPU); time = the mean of its own "
+                  f"index+matrix+greedy phase timers "
                   f"(JSON read phase {ph.get('read_ms', 0)} ms excluded: the GPU arm's e2e also starts from parsed arrays)")
         if not full:
             # not the same configuration: say so where the driver looks (config.genomes) and never publish a ratio from it
@@ -244,7 +250,7 @@ def run_reference_arm(args):
                        workload=cfg["workload"] + f" -- REFERENCE ARM RAN ONLY THE FIRST {n_s} GENOMES "
                                                     f"(host memory available {avail / 1e9:.0f} GB < {need / 1e9:.0f} GB needed)")
         line = {"impl": "reference", "metric": "ref-pair containments/s (yacht train hot path)", "value": val, "unit": "pairs/s",
-                "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "steps_run": 1, "warmup_run": 0,
+                "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "steps_run": len(runs), "warmup_run": 0,
                 "ms_per_step": per * 1e3,
                 "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "u64/int32 (+f64 threshold)",
                 "data": "synthetic", "config": cfg,
@@ -307,6 +313,26 @@ def check_digest(args, n, F, lines=None, pairs=None, sizes=None, selected=None):
            "n_selected": None if selected is None else int(len(selected))}
     out["parity_digest_ok"] = bool(out["F_ok"] and out["pairs_sha256_ok"] and out["selected_sha256_ok"] is not False)
     return out
+
+
+DUMP_BYTES = 64 * 1024 * 1024
+
+
+def dump_outputs(out_dir: str, stats: dict, pairs: np.ndarray) -> None:
+    """What a caller of the train step receives, as float64 .npy files (every value is an integer below 2**53, so exact):
+    index_stats = [n_distinct, n_singleton, n_index, flagged pairs]; pairs_i / pairs_j / pairs_count = the flagged ordered
+    pairs in the library's (i, j) order.  A pair list over DUMP_BYTES is cut to a fixed, seeded sample of its rows, in order,
+    so that two builds that flag the same pairs dump the same rows."""
+    os.makedirs(out_dir, exist_ok=True)
+    cols = ("i", "j", "count")
+    max_rows = (DUMP_BYTES - 4096) // (8 * len(cols))
+    rows = slice(None)
+    if len(pairs) > max_rows:
+        rows = np.sort(np.random.default_rng(0).choice(len(pairs), size=max_rows, replace=False))
+    np.save(os.path.join(out_dir, "index_stats.npy"),
+            np.array([stats["n_distinct"], stats["n_singleton"], stats["n_index"], len(pairs)], dtype=np.float64))
+    for c in cols:
+        np.save(os.path.join(out_dir, f"pairs_{c}.npy"), pairs[c][rows].astype(np.float64))
 
 
 def workload_config(args, db):
@@ -470,6 +496,12 @@ def run_b200_arm(args):
         return float(t.item()) / args.steps, tm, clocks, res, wall / args.steps
 
     ms_res, tm_res, clocks, n_flagged, wall_res = timed(step_resident, True)
+    if args.dump_outputs:
+        # the last resident step's results, read back outside the timed region; after the sharded step every rank holds the
+        # whole list, so every rank reads it (as step_e2e does) and rank 0 writes it
+        pairs_last = ctx.pairs_host(n_flagged)
+        if rank == 0:
+            dump_outputs(args.dump_outputs, index_stats, pairs_last)
     ms_e2e, tm_e2e, clocks_e2e, pairs_host, wall_e2e = timed(step_e2e, False)
 
     if rank == 0:
@@ -695,7 +727,13 @@ def main():
                     help="--impl reference: measure again even if this box already holds a measurement of the same configuration")
     ap.add_argument("--residency", default="hashes", choices=["hashes", "genomes"],
                     help="N > 1: what a rank holds -- its hash range of every sketch (default) or the sketches of its genome range")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the flagged pairs and index statistics of the last resident step to DIR/*.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference_arm(args)

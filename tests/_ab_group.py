@@ -1,6 +1,6 @@
 """A/B of the grouping kernel's occupancy variants at full size (run manually on the GPU box)."""
-import sys, time, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, time, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from yacht_b200 import _lib, synth
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 85205
 db = synth.make_reference_db(n, 3)

@@ -1,5 +1,5 @@
-import sys, time, numpy as np
-sys.path.insert(0,'/root/repo')
+import os, sys, time, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from yacht_b200 import _lib, synth
 from oracle import train_oracle as to
 ctx=_lib.GpuContext(0)

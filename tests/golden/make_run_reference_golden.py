@@ -27,7 +27,9 @@ per database, and single_hyp_test for every (n_exclusive, n_match) pair that cam
 (ksize, significance, ani, min_coverage).
 Part B (6 databases): the whole hypothesis_recovery(...) call, one frame per min_coverage.
 
-Output: tests/golden/run_reference_golden.npz (inputs and outputs; the tests never need /root/reference).
+Output: tests/golden/run_reference_golden.npz (the tests never need /root/reference).  It holds what the reference
+returned; the inputs it was given -- the seeded databases and samples of make_case(), the single_hyp_test arguments -- are
+made again from their seeds by load(), which checks them against checksums stored beside the outputs (pack()).
 """
 import gzip
 import hashlib
@@ -207,6 +209,73 @@ def make_case(seed):
     return sketches, sample
 
 
+def case_b_inputs(c):
+    """Part B database c: hypothesis_recovery keys files by md5, so exact duplicates are dropped and manifest rows and
+    files are one to one."""
+    sketches, sample = make_case(100 + c)
+    seen, uniq = set(), []
+    for s in sketches:
+        key = s.tobytes()
+        if key not in seen:
+            seen.add(key)
+            uniq.append(s)
+    return uniq, sample
+
+
+def _csr(sketches):
+    offsets = np.zeros(len(sketches) + 1, np.int64)
+    np.cumsum([len(s) for s in sketches], out=offsets[1:])
+    return np.concatenate(sketches).astype(np.uint64), offsets
+
+
+def _checksum(hashes, sample):
+    return [int(len(hashes)), int(np.bitwise_xor.reduce(hashes)), int(len(sample)), int(np.bitwise_xor.reduce(sample))]
+
+
+def _hyp_in(pairs, meta):
+    """single_hyp_test arguments in the generator's order: for each (n_exclusive, n_match), each grid point, each coverage."""
+    return np.array([(ne, nm, k, sig, ani, cov) for ne, nm in pairs for k, sig, ani in meta["hyp_grid"] for cov in meta["covs"]],
+                    dtype=np.float64)
+
+
+def pack(out, meta):
+    """The committed layout: the reference's outputs, and checksums of the seeded inputs instead of the inputs."""
+    keep = {}
+    for case in meta["cases_a"]:
+        c = case["id"]
+        case["inputs"] = _checksum(out[f"a{c}_hashes"], out[f"a{c}_sample"])
+        keep[f"a{c}_overlap"] = out[f"a{c}_overlap"]
+        for v in range(case["variants"]):
+            keep[f"a{c}_mask{v}"], keep[f"a{c}_info{v}"] = out[f"a{c}_mask{v}"], out[f"a{c}_info{v}"]
+    for case in meta["cases_b"]:
+        case["inputs"] = _checksum(out[f"b{case['id']}_hashes"], out[f"b{case['id']}_sample"])
+    pairs = np.array(sorted({(int(a), int(b)) for a, b in out["hyp_in"][:, :2]}), dtype=np.int64)
+    assert np.array_equal(_hyp_in(pairs, meta), out["hyp_in"])
+    keep["hyp_pairs"] = pairs
+    keep["hyp_out_t"] = np.ascontiguousarray(out["hyp_out"].T)      # column by column: compresses to half
+    keep["meta"] = np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8)
+    return keep
+
+
+def load(path=OUT):
+    """(arrays, meta) with every input and output array main() produced, the inputs made again from their seeds."""
+    with np.load(path) as f:
+        z = dict(f)
+    meta = json.loads(bytes(z.pop("meta")).decode())
+    for part, cases, make in (("a", meta["cases_a"], make_case), ("b", meta["cases_b"], case_b_inputs)):
+        for case in cases:
+            c = case["id"]
+            sketches, sample = make(c)
+            hashes, offsets = _csr(sketches)
+            sample = sample.astype(np.uint64)
+            assert _checksum(hashes, sample) == case["inputs"], \
+                f"make_case no longer reproduces the inputs of case {part}{c} the reference was run on"
+            z[f"{part}{c}_hashes"], z[f"{part}{c}_offsets"], z[f"{part}{c}_sample"] = hashes, offsets, sample
+    z["hyp_in"] = _hyp_in(z.pop("hyp_pairs"), meta)
+    z["hyp_out"] = np.ascontiguousarray(z.pop("hyp_out_t").T)
+    return z, meta
+
+
 def write_db(root, sketches, ksize, extra_ksize=None, seed=0):
     """root/signatures/<md5>.sig per genome (the layout `yacht train` leaves); returns the manifest frame."""
     os.makedirs(os.path.join(root, "signatures"))
@@ -298,15 +367,7 @@ def main():
         os.chmod(cli, os.stat(cli).st_mode | stat.S_IXUSR | stat.S_IXGRP | stat.S_IXOTH)
         os.environ["PATH"] = bindir + os.pathsep + os.environ["PATH"]
         for c in range(N_CASES_B):
-            sketches, sample = make_case(100 + c)
-            # hypothesis_recovery keys files by md5: drop exact duplicates so that manifest rows and files are one to one
-            seen, uniq = set(), []
-            for s in sketches:
-                key = s.tobytes()
-                if key not in seen:
-                    seen.add(key)
-                    uniq.append(s)
-            sketches = uniq
+            sketches, sample = case_b_inputs(c)
             ksize, sig, ani = HYP_GRID[c % len(HYP_GRID)]
             root = os.path.join(tmp, f"b{c}")
             manifest = write_db(root, sketches, ksize, extra_ksize=(21 if ksize != 21 else 31) if c % 2 == 1 else None, seed=100 + c)
@@ -332,9 +393,8 @@ def main():
             })
     finally:
         shutil.rmtree(tmp, ignore_errors=True)
-    out["meta"] = np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8)
     buf = io.BytesIO()
-    np.savez_compressed(buf, **out)
+    np.savez_compressed(buf, **pack(out, meta))
     with open(OUT, "wb") as f:
         f.write(buf.getvalue())
     print(f"wrote {OUT}: {len(buf.getvalue())} bytes, {N_CASES_A} databases / {sum(c['variants'] for c in meta['cases_a'])} "

@@ -1,5 +1,6 @@
 """N > 1 host logic on CPU: world_size-2 gloo run of the row sharding + pair-list gather
 (the same code path bench.py and multi-GPU callers use with NCCL on device tensors)."""
+import multiprocessing
 import os
 import socket
 
@@ -44,8 +45,9 @@ def _worker(rank, world, port, q):
 
 
 def test_two_rank_gather_matches_single_rank():
-    import torch.multiprocessing as mp
-    ctx = mp.get_context("spawn")
+    # torch is imported in the spawned workers only: after the library's multi-GPU calls this process holds the NCCL the
+    # loader found first, which need not be the one torch was built against
+    ctx = multiprocessing.get_context("spawn")
     q = ctx.Queue()
     port = _free_port()
     procs = [ctx.Process(target=_worker, args=(r, 2, port, q)) for r in range(2)]
@@ -155,8 +157,7 @@ def _plan_worker(rank, world, port, q):
 
 
 def test_exchange_plan_two_ranks():
-    import torch.multiprocessing as mp
-    ctx = mp.get_context("spawn")
+    ctx = multiprocessing.get_context("spawn")           # torch only in the workers, as above
     q = ctx.Queue()
     port = _free_port()
     procs = [ctx.Process(target=_plan_worker, args=(r, 2, port, q)) for r in range(2)]
