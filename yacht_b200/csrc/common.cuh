@@ -53,7 +53,7 @@ struct ygpu_ctx {
     uint32_t* d_msd_aux = nullptr;  // histograms / bases / cursors
     uint32_t* d_units = nullptr;    // level-2 tile descriptors (uint2 per tile)
     uint32_t* d_tile_g0 = nullptr;  // genome holding the first hash slot of every level-1 tile
-    int group_ctas = 4;             // test hook: CTAs per SM the grouping kernel k2_group2 is compiled for (4 or 5; measured: 4.48 ms vs 4.96 ms at 85k genomes)
+    int group_ctas = 4;             // test hook: CTAs per SM the grouping kernel k2_group2 is compiled for (4 or 5; measured at 85k genomes on 1 x B200: 3.72 ms vs 4.21 ms, profiles/r03b_ab_group.txt)
     int group_kernel = 0;           // test hook: 1 = always the general grouping kernel k2_group (0: k2_group2 where it applies)
     // final buckets too large for shared memory (k2_big_*): their list, compact starts, gathered / sorted words
     uint32_t* d_big_list = nullptr;

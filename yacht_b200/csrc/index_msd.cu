@@ -726,8 +726,13 @@ __global__ void __launch_bounds__(GK_THREADS, 4) k2_group(const GroupArgs a) {
 // Buckets of <= G2_MAXM words whose remaining hash bits (below the sub-bucket digit) fit 32 bits -- every bucket of a
 // database without extreme skew.  Same idea as k2_group (sub-bucket counting filter, dense candidate scan), rebuilt
 // around the instruction count, which is what bounds this step (not HBM):
-//   * the bucket's words arrive by ONE bulk asynchronous copy (cp.async.bulk + mbarrier) issued by one thread while
-//     the previous bucket is still being grouped; every thread then picks its four words with two 16-byte loads;
+//   * the bucket's words arrive by ONE bulk asynchronous copy (cp.async.bulk + mbarrier) into a ring of two stage
+//     buffers, requested two buckets ahead; every thread then picks its four words with two 16-byte loads;
+//   * the candidate-array room of a sub-bucket is claimed by its first word (warp scan + one shared atomic per warp),
+//     so a bucket costs four CTA barriers and no pass over the 2 048 sub-bucket counters.  The order of the sub-buckets
+//     inside a region is therefore the order in which the warps' atomics land, and it varies from run to run; so do
+//     the positions of a bucket's postings and the posting offsets inside indirect items.  Nothing depends on them:
+//     items are order-free, k2_group allocates its group slots with atomics too, and the flagged pairs are sorted;
 //   * a candidate is one 64-bit word (remaining hash << 32 | genome id) plus the extent of its sub-bucket, so the scan
 //     of a sub-bucket is one load and three compares per word, branch-free and fixed-length (4) for sub-buckets of
 //     <= 4 words (all but a few per bucket);
@@ -742,17 +747,18 @@ constexpr uint32_t IG_MAXL = 16;                  // sharded build: groups up to
 constexpr uint64_t IG_ROW_MUL = (IG_MAXL - 1 + 2) / 3;   // ... so one shared hash is worth at most this many items of a query row
 
 struct __align__(16) G2Smem {
-    uint64_t stage[G2_WIN];                       // the bucket's words (bulk copy target)
+    uint64_t stage[2][G2_WIN];                    // ring of two bucket windows (bulk copy targets): the CTA's i-th bucket lands in stage[i & 1]
     uint64_t cand[G2_WIN + 4];                    // candidates, sub-bucket by sub-bucket: remaining hash << 32 | genome id
-    uint32_t cnt[G2_NSUB];                        // sub-bucket sizes; after phase B: candidate-array start | size << 16 (zero between buckets)
+    uint32_t cnt[G2_NSUB];                        // sub-bucket sizes; after phase B: start in its region | size << 16 (zero between buckets)
     uint32_t ext[G2_WIN];                         // per candidate of a sub-bucket of >= 3 words: start of its sub-bucket | size << 16
     uint32_t stg_g[G2_WIN + 4];                   // ordered groups: genome id
     unsigned short stg_r[G2_WIN];                 // ordered groups: members that follow | 0x8000 posting wanted | 0x4000 hole
     uint32_t wsum[G2_THREADS / 32];
-    uint32_t next[2][2];                          // [parity]{first word, words} of the bucket after this one (words = 0: none)
+    uint32_t next[2][2];                          // {first word, words} of the CTA's i-th bucket in next[i & 1] (words = 0: none)
+    uint32_t cur;                                 // phase B cursor: words claimed in the pair region | in the larger region << 16
     uint32_t dcnt[YG_MAX_RANKS];                  // STREAM: items of this bucket per destination rank
     uint32_t dbase[YG_MAX_RANKS];                 // STREAM: ... and where they start in that rank's inbox
-    uint64_t mbar;
+    uint64_t mbar[2];                             // "full" barrier of each stage buffer
 };
 
 template <bool STREAM, int MIN_CTAS>
@@ -764,17 +770,20 @@ __global__ void __launch_bounds__(G2_THREADS, MIN_CTAS) k2_group2(const GroupArg
     const uint32_t kmask = (uint32_t)a.rest_mask;
     const bool can_inline = a.gb <= YG_ITEM_INLINE_BITS;
 
-    // thread 0: the next bucket this CTA takes at or after `b` (stride gridDim.x) that is non-empty and fits; its
-    // extent goes to sm.next[par] and its words are requested from the copy engine
+    // The scheduler is the last thread: its warp has the least phase-D work (candidates are dealt out from thread 0 up).
+    // It picks the CTA's buckets (stride gridDim.x, skipping empty ones and those over G2_MAXM words) two ahead: while
+    // bucket i is grouped, the words of bucket i + 1 are already in flight and those of bucket i + 2 are requested in
+    // phase D of bucket i, into the stage buffer bucket i's phase A has released.  Unless it has to skip buckets, the
+    // barrier after phase D never waits on its loads.
+    constexpr uint32_t SCHED = G2_THREADS - 1;
     const uint32_t b_end = a.range ? (uint32_t)a.range[1] : a.b_hi;
-    uint32_t b_next = (a.range ? (uint32_t)a.range[0] : a.b_lo) + blockIdx.x;       // thread 0 only
-    // the extent of bucket b_next is fetched one phase before it is needed, so that the two dependent loads never sit between
-    // two barriers of the whole CTA
+    uint32_t b_next = (a.range ? (uint32_t)a.range[0] : a.b_lo) + blockIdx.x;       // scheduler only
+    // the extent of bucket b_next is fetched one bucket before it is needed, so that its two dependent loads are not waited for
     uint32_t pre_lo = 0, pre_hi = 0;
     auto preload = [&]() {
         if (b_next < b_end) { pre_lo = a.base[b_next]; pre_hi = a.base[b_next + 1]; }
     };
-    auto advance = [&](uint32_t par) {
+    auto advance = [&](uint32_t slot) {
         uint32_t bb = 0, m = 0;
         while (b_next < b_end) {
             bb = pre_lo;
@@ -784,37 +793,39 @@ __global__ void __launch_bounds__(G2_THREADS, MIN_CTAS) k2_group2(const GroupArg
             m = 0;
             preload();
         }
-        sm.next[par][0] = bb;
-        sm.next[par][1] = m;
+        sm.next[slot][0] = bb;
+        sm.next[slot][1] = m;
         if (m) {
             const uint32_t w0 = bb & ~1u, w1 = (bb + m + 1u) & ~1u;
-            bulk_load(sm.stage, a.ent + w0, (w1 - w0) * 8u, &sm.mbar);
+            bulk_load(sm.stage[slot], a.ent + w0, (w1 - w0) * 8u, &sm.mbar[slot]);
         }
-        preload();          // the extent of the bucket after that one: in flight during phases B..F, consumed after the next phase A
+        preload();
     };
     for (uint32_t i = tid; i < G2_NSUB; i += G2_THREADS) sm.cnt[i] = 0;
-    if (tid == 0) {
-        mbar_init(&sm.mbar, 1);
+    if (tid == SCHED) {
+        mbar_init(&sm.mbar[0], 1);
+        mbar_init(&sm.mbar[1], 1);
         mbar_init_fence();
+        sm.cur = 0;
         preload();
         advance(0);
+        advance(1);
     }
     __syncthreads();
 
     uint32_t n_heads = 0, n_single = 0, n_dups = 0;
     unsigned long long n_w = 0;
     GroupPending pd{0ull, 0u, 0u, false}, pd2{0ull, 0u, 0u, false};   // two appends in flight: the atomic's answer is consumed two items later
-    uint32_t par = 0, phase = 0;
-    for (;;) {
+    for (uint32_t it = 0;; it++) {
+        const uint32_t par = it & 1u;
         const uint32_t bb = sm.next[par][0], m = sm.next[par][1];
         if (!m) break;
-        mbar_wait(&sm.mbar, phase);
-        phase ^= 1u;
+        mbar_wait(&sm.mbar[par], (it >> 1) & 1u);
         // ---- A: four words per thread, sub-bucket rank -----------------------------------------------------------
         const uint32_t wlo = bb & 1u, whi = wlo + m;                 // the bucket inside the copied window
         uint64_t e[4];
         {
-            const uint4* s4 = reinterpret_cast<const uint4*>(sm.stage);
+            const uint4* s4 = reinterpret_cast<const uint4*>(sm.stage[par]);
             const uint4 v0 = s4[tid], v1 = s4[G2_THREADS + tid];
             e[0] = (uint64_t)v0.x | ((uint64_t)v0.y << 32); e[1] = (uint64_t)v0.z | ((uint64_t)v0.w << 32);
             e[2] = (uint64_t)v1.x | ((uint64_t)v1.y << 32); e[3] = (uint64_t)v1.z | ((uint64_t)v1.w << 32);
@@ -829,60 +840,59 @@ __global__ void __launch_bounds__(G2_THREADS, MIN_CTAS) k2_group2(const GroupArg
                 sr[k] = s | (atomicAdd(&sm.cnt[s], 1u) << 16);
             }
         }
-        __syncthreads();                                             // stage is free: request the next bucket
-        if (tid == 0) advance(par ^ 1u);
-        // ---- B: candidate-array starts of the sub-buckets with >= 2 words, in TWO regions: sub-buckets of exactly two words
+        __syncthreads();                                             // stage[par] is free (refilled in phase D)
+        // ---- B: candidate-array place of every sub-bucket with >= 2 words, in TWO regions: sub-buckets of exactly two words
         //      (most of them: two genomes sharing a hash, or two hashes that merely share 11 bits) come first, as aligned
-        //      pairs; phase D settles those with one compare.  Larger sub-buckets follow.  One packed scan serves both
-        //      regions (16 bits each); the counter of a sub-bucket is replaced by start | size << 16 (0: no candidates).
-        uint32_t nx, ncand;
+        //      pairs; phase D settles those with one compare.  Larger sub-buckets follow.  The word of rank 0 claims its
+        //      sub-bucket's room: one warp scan and one shared-memory atomic per warp on a cursor that packs both regions
+        //      (16 bits each).  Only the ~824 words of the bucket are visited, not the 2 048 counters; the order of the
+        //      sub-buckets inside a region is the order of the claims.  The counter of a claimed sub-bucket becomes
+        //      start in its region | size << 16 (an unclaimed one keeps its size, 1).
         {
-            uint4* c4 = reinterpret_cast<uint4*>(&sm.cnt[8 * tid]);
-            const uint4 c0 = c4[0], c1 = c4[1];
-            uint32_t c[8] = {c0.x, c0.y, c0.z, c0.w, c1.x, c1.y, c1.z, c1.w};
-            uint32_t sum = 0;                                        // words of pair sub-buckets | words of larger ones << 16
+            uint32_t cl[4];                                          // size of the sub-bucket this word claims (0: none)
+            uint32_t own = 0;                                        // words claimed in the pair region | in the larger region << 16
 #pragma unroll
-            for (int i = 0; i < 8; i++) sum += c[i] == 2 ? 2u : (c[i] >= 3 ? (c[i] << 16) : 0u);
-            uint32_t inc = sum;
+            for (int k = 0; k < 4; k++) {
+                const uint32_t c = sr[k] < 0x10000u ? sm.cnt[sr[k]] : 0u;     // rank 0 of a word of the bucket
+                cl[k] = c >= 2 ? c : 0u;
+                own += c == 2 ? 2u : (c >= 3 ? (c << 16) : 0u);
+            }
+            uint32_t inc = own;
 #pragma unroll
             for (int o = 1; o < 32; o <<= 1) {
                 const uint32_t v = __shfl_up_sync(0xffffffffu, inc, o);
                 if ((int)lane >= o) inc += v;
             }
-            if (lane == 31) sm.wsum[warp] = inc;
-            __syncthreads();
-            const uint4 wa = *reinterpret_cast<const uint4*>(&sm.wsum[0]), wb = *reinterpret_cast<const uint4*>(&sm.wsum[4]);
-            const uint32_t wp = (warp > 0 ? wa.x : 0u) + (warp > 1 ? wa.y : 0u) + (warp > 2 ? wa.z : 0u) + (warp > 3 ? wa.w : 0u) +
-                                (warp > 4 ? wb.x : 0u) + (warp > 5 ? wb.y : 0u) + (warp > 6 ? wb.z : 0u);
-            const uint32_t tot = wa.x + wa.y + wa.z + wa.w + wb.x + wb.y + wb.z + wb.w;
-            nx = tot & 0xffffu;
-            ncand = nx + (tot >> 16);
-            const uint32_t ex = wp + inc - sum;
-            uint32_t px = ex & 0xffffu, py = nx + (ex >> 16);
+            uint32_t wbase = 0;
+            if (lane == 31 && inc) wbase = atomicAdd(&sm.cur, inc);
+            const uint32_t ex = __shfl_sync(0xffffffffu, wbase, 31) + inc - own;
+            uint32_t px = ex & 0xffffu, py = ex >> 16;
 #pragma unroll
-            for (int i = 0; i < 8; i++) {                            // branch-free: the lanes of a warp see every mix of sizes
-                const bool two = c[i] == 2, more = c[i] >= 3;
-                const uint32_t v = two ? (px | (2u << 16)) : (more ? (py | (c[i] << 16)) : 0u);
-                px += two ? 2u : 0u;
-                py += more ? c[i] : 0u;
-                c[i] = v;
+            for (int k = 0; k < 4; k++) {
+                if (cl[k]) {
+                    const bool two = cl[k] == 2;
+                    sm.cnt[sr[k]] = (two ? px : py) | (cl[k] << 16);
+                    px += two ? 2u : 0u;
+                    py += two ? 0u : cl[k];
+                }
             }
-            c4[0] = make_uint4(c[0], c[1], c[2], c[3]);
-            c4[1] = make_uint4(c[4], c[5], c[6], c[7]);
         }
         __syncthreads();
+        const uint32_t cur = sm.cur;
+        const uint32_t nx = cur & 0xffffu, ncand = nx + (cur >> 16);
         // ---- C: candidates -> dense array, sub-bucket by sub-bucket; a word alone in its sub-bucket is a singleton ----
         uint32_t solo = 0;
 #pragma unroll
         for (int k = 0; k < 4; k++) {
             if (sr[k] != 0xFFFFFFFFu) {
                 const uint32_t v = sm.cnt[sr[k] & 0xffffu];
-                if (v) {
-                    const uint32_t pos = (v & 0xffffu) + (sr[k] >> 16);
+                if (v >= (2u << 16)) {
+                    const uint32_t start = v >= (3u << 16) ? v + nx : v;   // larger region: after the nx pair words
+                    const uint32_t pos = (start & 0xffffu) + (sr[k] >> 16);
                     const uint32_t K = (uint32_t)(e[k] >> a.gb) & kmask;
                     const uint32_t G = (uint32_t)e[k] & gmask;
                     sm.cand[pos] = ((uint64_t)K << 32) | (uint64_t)G;
-                    if (v >= (3u << 16)) sm.ext[pos] = v;
+                    if (v >= (3u << 16)) sm.ext[pos] = start;
                 } else {
                     solo++;
                 }
@@ -891,11 +901,11 @@ __global__ void __launch_bounds__(G2_THREADS, MIN_CTAS) k2_group2(const GroupArg
         n_heads += solo;
         n_single += solo;
         __syncthreads();
-        {   // the counters are free again: zero for the next bucket
-            uint4* c4 = reinterpret_cast<uint4*>(&sm.cnt[8 * tid]);
-            c4[0] = make_uint4(0u, 0u, 0u, 0u);
-            c4[1] = make_uint4(0u, 0u, 0u, 0u);
-        }
+        // the counters and the cursor are free again: zero for the next bucket (its phase A is behind the barrier after D)
+#pragma unroll
+        for (int k = 0; k < 4; k++)
+            if (sr[k] != 0xFFFFFFFFu) sm.cnt[sr[k] & 0xffffu] = 0u;
+        if (tid == SCHED) sm.cur = 0;
         // ---- D: group size, rank in the group (by genome id), slot in the (hash, genome) order of the sub-bucket ------------
         // pairs: the partner is the other word of the aligned pair
         for (uint32_t q = tid; q < nx; q += G2_THREADS) {
@@ -943,6 +953,7 @@ __global__ void __launch_bounds__(G2_THREADS, MIN_CTAS) k2_group2(const GroupArg
             n_dups += dup;
             if (L >= 2 && rank == 0) n_w += (unsigned long long)L * L;
         }
+        if (tid == SCHED) advance(par);                              // bucket i + 2 -> stage[par]
         __syncthreads();
         if (STREAM) {
             // ---- F' (sharded build): the groups leave this rank --------------------------------------------------------------
@@ -1022,7 +1033,6 @@ __global__ void __launch_bounds__(G2_THREADS, MIN_CTAS) k2_group2(const GroupArg
                     for (uint32_t i = tid; i < np; i += G2_THREADS) { dg[i] = cg[i]; dr[i] = cr[i]; }
                 }
             }
-            par ^= 1u;
             continue;          // (the next bucket's first barrier separates its phases from this one)
         }
         // ---- F: postings + work items, one thread per ordered slot ------------------------------------------------------
@@ -1048,7 +1058,6 @@ __global__ void __launch_bounds__(G2_THREADS, MIN_CTAS) k2_group2(const GroupArg
                 pd2.item = item; pd2.dst = dst; pd2.slot = slot; pd2.has = true;
             }
         }
-        par ^= 1u;
         // (the next bucket's phase A only touches stage / cnt; its barriers order everything else against this phase F)
     }
     if (pd.has) a.row_items[(uint64_t)pd.dst + pd.slot] = pd.item;
@@ -1545,7 +1554,7 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
         g.m_lo = 0;
         if (fast2 && nbk) {
             const size_t smem2 = sizeof(G2Smem);
-            // 4 CTAs per SM (64 registers) against 5 (48 registers, spills 88 bytes: measured slower): test hook "group_ctas"
+            // 4 CTAs per SM (61 registers) against 5 (48 registers, spills 24 bytes; measured slower): test hook "group_ctas"
             auto kern2 = ctx->group_ctas == 5 ? k2_group2<false, 5> : k2_group2<false, 4>;
             YG_CUDA(ctx, cudaFuncSetAttribute(kern2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
             int occ2 = 1;
