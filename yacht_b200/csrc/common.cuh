@@ -38,7 +38,8 @@ struct ygpu_ctx {
     uint8_t* d_flag = nullptr;      // [T]   1 if the sorted slot belongs to a run of length >= 2
     uint32_t* d_cpos = nullptr;     // [T]   exclusive scan of d_flag (slot in the compacted postings)
     uint64_t P = 0;                 // postings kept
-    uint32_t* d_post = nullptr;     // [P]   compacted posting array (genome ids), runs contiguous
+    uint32_t* d_post = nullptr;     // [P]   compacted posting array (genome ids), runs contiguous (partition path: indexed by
+                                    //       position in the final buffer, + the words of oversized buckets behind it)
     uint32_t* d_rem = nullptr;      // [P]   postings that follow slot c inside its run
     uint64_t n_items = 0;
     uint64_t* d_row_ptr = nullptr;  // [n+1] CSR over row_items (general path)
@@ -48,8 +49,8 @@ struct ygpu_ctx {
     bool row_work_valid = false;
     unsigned long long* d_row_cnt = nullptr;  // [n+1] build scratch
     // MSD-partition build (index_msd.cu)
-    uint64_t* d_ent1 = nullptr;     // [T] packed (hash low bits | genome id) words, level-1 buckets
-    uint64_t* d_ent2 = nullptr;     // [T] same, final buckets
+    uint64_t* d_ent1 = nullptr;     // [max(T, slots x capacity)] packed (hash low bits | genome id) words, level-1 buckets
+    uint64_t* d_ent2 = nullptr;     // [max(T, slots x capacity)] same, final buckets ([T] on the exact layout)
     uint32_t* d_msd_aux = nullptr;  // histograms / bases / cursors
     uint32_t* d_units = nullptr;    // level-2 tile descriptors (uint2 per tile)
     uint32_t* d_tile_g0 = nullptr;  // genome holding the first hash slot of every level-1 tile

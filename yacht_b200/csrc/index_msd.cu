@@ -16,8 +16,9 @@
 //      not take: a counting filter over the next 11 hash bits drops the words that are alone in their sub-bucket,
 //      the rest are scanned densely; no ordering of singleton hashes is ever computed), orders only the members of
 //      shared groups by genome id, and emits compact postings + per-genome work items.
-// Algorithmic HBM traffic: 8T (histogram) + 8T + 8T (scatter 1) + 8T (histogram 2) + 16T (scatter 2)
-// + 8T (bucket read) + O(P) outputs ~= 56 bytes per hash, against ~176 for the 7-pass pair sort.
+// Algorithmic HBM traffic: 8T + 8T (scatter 1) + 16T (scatter 2) + 8T (bucket read) + O(P) outputs ~= 40 bytes per hash,
+// against ~176 for the 7-pass pair sort.  The buckets live in fixed-capacity slots sized from the plan (msd_build); only a
+// database that overflows one pays the two histogram passes (8T each) of the exact layout.
 //
 // Skew: a final bucket that does not fit shared memory (a hash held by thousands of genomes) leaves this path
 // alone -- its words are sorted device-wide (in chunks of buckets) and grouped by neighbour comparison (k2_big_*).
@@ -46,7 +47,8 @@ constexpr int SC_BND = 16;          // level 1: genome boundaries per tile resol
 constexpr int NB_MAX = 2048;        // digits per partition level
 constexpr uint32_t A_TARGET = 900;  // average elements per used final bucket (k2_group2 takes buckets of <= 1022)
 
-enum { SCM_PCUR = 8, SCM_ICUR = 9, SCM_MAXB = 10, SCM_STREAM = 12 };   // extra slots of ctx->d_scalars (SCM_MAXB uses two)
+// extra slots of ctx->d_scalars (SCM_MAXB uses two; SCM_OVF1 / SCM_OVF2: a slot of that partition level overflowed)
+enum { SCM_PCUR = 8, SCM_ICUR = 9, SCM_MAXB = 10, SCM_STREAM = 12, SCM_OVF1 = 13, SCM_OVF2 = 14 };
 // sharded step: the first REP_WORDS slots of d_scalars are one rank's report to the others (statistics, largest bucket, posting-
 // stream length, and from REP_ICUR the number of work items it sent to every rank); ONE all-gather after the grouping carries it
 enum { REP_ICUR = 16, REP_WORDS = 32 };
@@ -133,17 +135,21 @@ __global__ void __launch_bounds__(256) k2_hist1(const uint64_t* __restrict__ has
         if (sh[k]) atomicAdd(&hist[k], sh[k]);
 }
 
-// one CTA: bucket bases, tile prefix (for level-2 work units) and cursors from the level-1 histogram
-__global__ void __launch_bounds__(1024) k2_prep1(const uint32_t* __restrict__ hist, uint32_t nb, uint32_t* __restrict__ base,
-                                                  uint32_t* __restrict__ tile_start, uint32_t* __restrict__ cursor,
-                                                  unsigned long long* __restrict__ scal) {
+// one CTA: tile prefix (for level-2 work units) and largest bucket from the level-1 bucket sizes, plus either
+//   end == NULL (exact layout, before the scatter): cnt is the histogram; begin = its exclusive scan, begin[nb] = total, and
+//               the scatter's cursors start there;
+//   end != NULL (slotted layout, after the scatter): cnt are the scatter's counters, clamped to cap (a slot that overflowed is
+//               cut; the host redoes the partition on the exact layout); end = begin + size.
+__global__ void __launch_bounds__(1024) k2_prep1(const uint32_t* __restrict__ cnt, const uint32_t* __restrict__ cap, uint32_t nb,
+                                                  uint32_t* __restrict__ begin, uint32_t* __restrict__ end, uint32_t* __restrict__ cursor,
+                                                  uint32_t* __restrict__ tile_start, unsigned long long* __restrict__ scal) {
     typedef cub::BlockScan<uint32_t, 1024> Scan;
     __shared__ typename Scan::TempStorage ts1, ts2;
     const int per = (NB_MAX + 1023) / 1024;
     uint32_t h[per], t[per], hs = 0, tsum = 0, mx = 0;
     for (int k = 0; k < per; k++) {
         const uint32_t i = threadIdx.x * per + k;
-        h[k] = i < nb ? hist[i] : 0u;
+        h[k] = i < nb ? (end ? min(cnt[i], cap[i]) : cnt[i]) : 0u;
         t[k] = (h[k] + SC_TILE - 1) / SC_TILE;
         hs += h[k]; tsum += t[k]; mx = max(mx, h[k]);
     }
@@ -152,11 +158,40 @@ __global__ void __launch_bounds__(1024) k2_prep1(const uint32_t* __restrict__ hi
     Scan(ts2).ExclusiveSum(tsum, toff, ttot);
     for (int k = 0; k < per; k++) {
         const uint32_t i = threadIdx.x * per + k;
-        if (i < nb) { base[i] = hoff; cursor[i] = hoff; tile_start[i] = toff; }
+        if (i < nb) {
+            if (end) end[i] = begin[i] + h[k];
+            else { begin[i] = hoff; cursor[i] = hoff; }
+            tile_start[i] = toff;
+        }
         hoff += h[k]; toff += t[k];
     }
-    if (threadIdx.x == 0) { base[nb] = htot; tile_start[nb] = ttot; }
+    if (threadIdx.x == 0) {
+        if (!end) begin[nb] = htot;
+        tile_start[nb] = ttot;
+    }
     if (mx) atomicMax(&scal[SCM_MAXB], (unsigned long long)mx);
+}
+
+// slotted layout: bucket b owns words [b * c, (b + 1) * c) of the level's buffer
+__global__ void __launch_bounds__(256) k2_slots(uint32_t nb, uint32_t c, uint32_t* __restrict__ begin, uint32_t* __restrict__ cap) {
+    for (uint32_t b = blockIdx.x * blockDim.x + threadIdx.x; b <= nb; b += gridDim.x * blockDim.x) {
+        begin[b] = b * c;
+        cap[b] = c;
+    }
+}
+
+// slotted layout, level 2: bucket extents from the scatter's counters (clamped to the slot) and the largest bucket
+__global__ void __launch_bounds__(256) k2_ends(const uint32_t* __restrict__ cnt, const uint32_t* __restrict__ cap,
+                                               const uint32_t* __restrict__ begin, uint32_t nb, uint32_t* __restrict__ end,
+                                               unsigned long long* __restrict__ maxb) {
+    uint32_t mx = 0;
+    for (uint32_t b = blockIdx.x * blockDim.x + threadIdx.x; b < nb; b += gridDim.x * blockDim.x) {
+        const uint32_t m = min(cnt[b], cap[b]);
+        end[b] = begin[b] + m;
+        mx = max(mx, m);
+    }
+    mx = __reduce_max_sync(0xffffffffu, mx);
+    if ((threadIdx.x & 31) == 0 && mx) atomicMax(maxb, (unsigned long long)mx);
 }
 
 // ---- scatter (level 1: raw hashes -> packed words by leading digit; level 2: words -> final buckets)
@@ -167,9 +202,14 @@ struct ScatterArgs {
     uint32_t n;
     const uint64_t* in_ent;      // level 2 input
     uint64_t* out_ent;
-    const uint32_t* base1;       // level 2: level-1 bucket bases
     const uint32_t* tile_start;  // level 2: prefix of tiles per level-1 bucket ([nb1] = number of units)
-    uint32_t* cursor;            // per output bucket
+    // Slotted layout (slot != 0): bucket b's words go to out_ent[b * slot + rank], rank counted from zero in cursor[b], so an
+    // overshoot cannot wrap 32 bits; words of rank >= slot are dropped and raise *ovf.  Exact layout (slot == 0, sized by a
+    // histogram, cannot overflow): cursor[b] starts at the bucket's first position (sharded step: where this rank's words go).
+    // Neither needs a load per (tile, digit) run beside the cursor atomic.
+    uint32_t slot;
+    uint32_t* cursor;
+    unsigned long long* ovf;
     uint32_t* hist2;             // hist2 kernel only
     const uint2* units;          // level 2: per tile {first word, words | level-1 bucket << 16} (k2_units)
     // sharded build across GPUs (level 1, PEER): a word goes to the rank that owns its leading digit, stored straight into
@@ -196,9 +236,9 @@ __device__ __forceinline__ bool unit_range(const ScatterArgs& a, const MsdPlan& 
     return true;
 }
 
-// one thread per level-2 tile: which level-1 bucket it belongs to and which words it covers
-__global__ void __launch_bounds__(256) k2_units(const uint32_t* __restrict__ tile_start, const uint32_t* __restrict__ base1, uint32_t nb1,
-                                                uint2* __restrict__ units) {
+// one thread per level-2 tile: which level-1 bucket it belongs to and which words it covers (bucket b: [begin1[b], end1[b]))
+__global__ void __launch_bounds__(256) k2_units(const uint32_t* __restrict__ tile_start, const uint32_t* __restrict__ begin1,
+                                                const uint32_t* __restrict__ end1, uint32_t nb1, uint2* __restrict__ units) {
     const uint32_t n_units = tile_start[nb1];
     for (uint32_t unit = blockIdx.x * blockDim.x + threadIdx.x; unit < n_units; unit += gridDim.x * blockDim.x) {
         uint32_t lo = 0, hi = nb1;          // last bucket b with tile_start[b] <= unit
@@ -207,8 +247,8 @@ __global__ void __launch_bounds__(256) k2_units(const uint32_t* __restrict__ til
             if (tile_start[mid] <= unit) lo = mid; else hi = mid;
         }
         const uint32_t k = unit - tile_start[lo];
-        const uint64_t begin = (uint64_t)base1[lo] + (uint64_t)k * SC_TILE;
-        const uint32_t m = (uint32_t)min((uint64_t)SC_TILE, (uint64_t)base1[lo + 1] - begin);
+        const uint64_t begin = (uint64_t)begin1[lo] + (uint64_t)k * SC_TILE;
+        const uint32_t m = (uint32_t)min((uint64_t)SC_TILE, (uint64_t)end1[lo] - begin);
         units[unit] = make_uint2((uint32_t)begin, m | (lo << 16));
     }
 }
@@ -290,10 +330,12 @@ __global__ void __launch_bounds__(SC_THREADS, 2) k2_scatter(const ScatterArgs a,
     uint64_t* buf0 = (uint64_t*)smem_raw;                          // [2][SC_BUF]
     const uint32_t nd = LEVEL == 1 ? p.nb1 : (1u << p.d2);
     uint64_t** gptr = (uint64_t**)(buf0 + 2 * SC_BUF);             // [nd] PEER only: where this tile's run of digit d goes
-    uint32_t* cnt = (uint32_t*)(gptr + (PEER ? nd : 0));           // [nd]
+    // [nd] {gbase, glim}: slot q of digit d's run goes to gbase + q if q < glim (beyond: past its bucket's cap) -- one 8-byte
+    // shared load per word
+    uint2* gdst = (uint2*)(gptr + (PEER ? nd : 0));
+    uint32_t* cnt = (uint32_t*)(gdst + nd);                        // [nd]
     uint32_t* lbase = cnt + nd;                                    // [nd]
-    uint32_t* gbase = lbase + nd;                                  // [nd]
-    uint16_t* sdig = (uint16_t*)(gbase + nd);                      // [SC_TILE]
+    uint16_t* sdig = (uint16_t*)(lbase + nd);                      // [SC_TILE]
     typedef cub::BlockScan<uint32_t, SC_THREADS> Scan;
     __shared__ typename Scan::TempStorage scan_ts;
     __shared__ __align__(8) uint64_t mbar[2];
@@ -373,10 +415,10 @@ __global__ void __launch_bounds__(SC_THREADS, 2) k2_scatter(const ScatterArgs a,
             if (dg[k] != SKIP) rk[k] = (uint16_t)atomicAdd(&cnt[dg[k]], 1u);
         __syncthreads();                   // every word of the tile is in registers: the buffer becomes the staging area
         uint32_t mv = 0;     // words of this tile that are kept
-        // exclusive scan of cnt -> lbase; reserve global space per digit (the cursor atomics' answers are only needed for the
+        // exclusive scan of cnt -> lbase; reserve room per digit in its bucket (the cursor atomics' answers are only needed for the
         // write-out: they travel while the tile is being reordered); counters back to zero
         constexpr uint32_t PER_MAX = (NB_MAX + SC_THREADS - 1) / SC_THREADS;
-        uint32_t gb0[PER_MAX], lb0[PER_MAX];
+        uint32_t gb0[PER_MAX], has = 0;
         const uint32_t per = (nd + SC_THREADS - 1) / SC_THREADS;
         const uint32_t d0 = tid * per;
         {
@@ -387,14 +429,14 @@ __global__ void __launch_bounds__(SC_THREADS, 2) k2_scatter(const ScatterArgs a,
 #pragma unroll
             for (uint32_t k = 0; k < PER_MAX; k++) {
                 const uint32_t d = d0 + k;
-                gb0[k] = 0; lb0[k] = 0xFFFFFFFFu;
+                gb0[k] = 0;
                 if (k < per && d < nd) {
                     const uint32_t c = cnt[d];
                     lbase[d] = off;
                     if (c) {
                         const uint64_t ci = LEVEL == 1 ? (uint64_t)d : (((uint64_t)b1 << p.d2) + d);
                         gb0[k] = atomicAdd(&a.cursor[ci], c);
-                        lb0[k] = off;
+                        has |= 1u << k;
                         cnt[d] = 0;
                     }
                     off += c;
@@ -410,13 +452,18 @@ __global__ void __launch_bounds__(SC_THREADS, 2) k2_scatter(const ScatterArgs a,
                 sdig[q] = dg[k];
             }
         }
-        // where the run of digit d goes: slot q of the reordered tile lands at gbase[d] + q (PEER: in the owner's buffer)
+        // where the run of digit d goes: slot q of the reordered tile lands at gbase + q (PEER: in the owner's buffer), for
+        // q < glim (the rest of the run is beyond the bucket's cap)
 #pragma unroll
         for (uint32_t k = 0; k < PER_MAX; k++) {
-            if (lb0[k] != 0xFFFFFFFFu) {
+            if (has & (1u << k)) {
                 const uint32_t d = d0 + k;
-                if (PEER) gptr[d] = a.peer_ent[a.owner[d]] + gb0[k] - lb0[k];
-                else gbase[d] = gb0[k] - lb0[k];
+                const uint32_t ci = LEVEL == 1 ? d : (b1 << p.d2) + d;
+                const uint32_t bg = ci * a.slot;              // 0 on the exact layout: the cursor is a position there
+                const uint32_t lb = lbase[d];
+                if (PEER) gptr[d] = a.peer_ent[a.owner[d]] + bg + gb0[k] - lb;
+                gdst[d] = make_uint2(bg + gb0[k] - lb,
+                                     !a.slot ? (uint32_t)SC_TILE : lb + (gb0[k] < a.slot ? min(a.slot - gb0[k], (uint32_t)SC_TILE) : 0u));
             }
         }
         __syncthreads();
@@ -425,8 +472,10 @@ __global__ void __launch_bounds__(SC_THREADS, 2) k2_scatter(const ScatterArgs a,
             const uint32_t q = k * SC_THREADS + tid;
             if (q < mv) {
                 const uint32_t d = sdig[q];
-                if (PEER) gptr[d][q] = buf[q];                               // a store over NVLink when the owner is a peer
-                else a.out_ent[(uint64_t)(uint32_t)(gbase[d] + q)] = buf[q];
+                const uint2 g = gdst[d];
+                if (q >= g.y) *a.ovf = 1ull;                                 // the bucket's slot is full: the host re-partitions
+                else if (PEER) gptr[d][q] = buf[q];                          // a store over NVLink when the owner is a peer
+                else a.out_ent[(uint64_t)(uint32_t)(g.x + q)] = buf[q];
             }
         }
         fetch_bnd(unit + gridDim.x, slot ^ 1u);
@@ -467,7 +516,8 @@ constexpr int GK_SLOW = BK_CAP / GK_THREADS;        // 12
 
 struct GroupArgs {
     const uint64_t* ent;
-    const uint32_t* base;        // [nb + 1]
+    const uint32_t* begin;       // bucket b: words [begin[b], end[b]) of ent (exact layout: end = begin + 1)
+    const uint32_t* end;
     uint32_t nb;
     uint32_t b_lo, b_hi;         // final buckets this launch covers (all, or one rank's hash range)
     uint32_t m_lo;               // k2_group: only buckets of more than m_lo words (the smaller ones went to k2_group2)
@@ -692,13 +742,13 @@ __global__ void __launch_bounds__(GK_THREADS, 4) k2_group(const GroupArgs a) {
     uint32_t par = 0;
     uint32_t b = a.b_lo + blockIdx.x;
     uint32_t bb = 0, m = 0;
-    if (b < a.b_hi) { bb = a.base[b]; m = a.base[b + 1] - bb; }
+    if (b < a.b_hi) { bb = a.begin[b]; m = a.end[b] - bb; }
     bool staged = false;
     while (b < a.b_hi) {
         // the next bucket's extent is fetched now and used in phase E, where its words are prefetched
         const uint32_t bn = b + gridDim.x;
         uint32_t bbn = 0, mn = 0;
-        if (bn < a.b_hi) { bbn = a.base[bn]; mn = a.base[bn + 1] - bbn; }
+        if (bn < a.b_hi) { bbn = a.begin[bn]; mn = a.end[bn] - bbn; }
         if (m > a.m_lo && m <= BK_CAP) {    // uniform per CTA (larger buckets: k2_big_*, below)
             if (m <= GK_FAST * GK_THREADS) group_bucket<GK_FAST>(a, bb, m, sm, &s_pcur[par], &s_gpos[par], st, pd, staged, bbn, mn);
             else group_bucket<GK_SLOW>(a, bb, m, sm, &s_pcur[par], &s_gpos[par], st, pd, false, bbn, mn);
@@ -781,7 +831,7 @@ __global__ void __launch_bounds__(G2_THREADS, MIN_CTAS) k2_group2(const GroupArg
     // the extent of bucket b_next is fetched one bucket before it is needed, so that its two dependent loads are not waited for
     uint32_t pre_lo = 0, pre_hi = 0;
     auto preload = [&]() {
-        if (b_next < b_end) { pre_lo = a.base[b_next]; pre_hi = a.base[b_next + 1]; }
+        if (b_next < b_end) { pre_lo = a.begin[b_next]; pre_hi = a.end[b_next]; }
     };
     auto advance = [&](uint32_t slot) {
         uint32_t bb = 0, m = 0;
@@ -1080,10 +1130,11 @@ __global__ void __launch_bounds__(G2_THREADS, MIN_CTAS) k2_group2(const GroupArg
 // neighbour comparison -- same outputs as k2_group (postings, work items appended to the genome lists, the
 // statistics), postings stored behind the T regular slots of d_post.  Everything else stays on the fast path.
 
-__global__ void __launch_bounds__(256) k2_big_list(const uint32_t* __restrict__ base, uint32_t b_lo, uint32_t b_hi,
-                                                   uint32_t* __restrict__ list, uint32_t list_cap, unsigned long long* __restrict__ scal) {
+__global__ void __launch_bounds__(256) k2_big_list(const uint32_t* __restrict__ begin, const uint32_t* __restrict__ end, uint32_t b_lo,
+                                                   uint32_t b_hi, uint32_t* __restrict__ list, uint32_t list_cap,
+                                                   unsigned long long* __restrict__ scal) {
     for (uint32_t b = b_lo + blockIdx.x * blockDim.x + threadIdx.x; b < b_hi; b += gridDim.x * blockDim.x) {
-        const uint32_t m = base[b + 1] - base[b];
+        const uint32_t m = end[b] - begin[b];
         if (m > BK_CAP) {
             const unsigned long long k = atomicAdd(&scal[SCM_STREAM], 1ull);       // (slot unused outside stream mode)
             if (k < list_cap) list[k] = b;
@@ -1091,13 +1142,13 @@ __global__ void __launch_bounds__(256) k2_big_list(const uint32_t* __restrict__ 
     }
 }
 
-__global__ void __launch_bounds__(256) k2_big_gather(const uint64_t* __restrict__ ent, const uint32_t* __restrict__ base,
-                                                     const uint32_t* __restrict__ list, const uint64_t* __restrict__ cstart, uint32_t n_big,
+__global__ void __launch_bounds__(256) k2_big_gather(const uint64_t* __restrict__ ent, const uint32_t* __restrict__ begin,
+                                                     const uint32_t* __restrict__ end, const uint32_t* __restrict__ list, const uint64_t* __restrict__ cstart, uint32_t n_big,
                                                      int low_bits, uint64_t* __restrict__ out) {
     const uint64_t lowmask = low_bits >= 64 ? ~0ull : ((1ull << low_bits) - 1ull);
     for (uint32_t j = blockIdx.x; j < n_big; j += gridDim.x) {
         const uint32_t b = list[j];
-        const uint64_t bb = base[b], m = base[b + 1] - base[b], dst = cstart[j];
+        const uint64_t bb = begin[b], m = end[b] - begin[b], dst = cstart[j];
         const uint64_t tag = low_bits >= 64 ? 0ull : ((uint64_t)j << low_bits);
         for (uint64_t i = threadIdx.x; i < m; i += blockDim.x) out[dst + i] = tag | (ent[bb + i] & lowmask);
     }
@@ -1334,12 +1385,27 @@ __global__ void __launch_bounds__(1024) k2s_range(const uint32_t* __restrict__ h
     }
 }
 
+// Views of ctx->d_msd_aux.  Per level and bucket b: begin, cap (exact layout: the histogram), the scatter's cursor (slotted:
+// counts from zero; exact: a position, starting at begin) and, slotted layout only, end = begin + words.  Exact layout: bucket b
+// spans [begin[b], begin[b + 1]), so its consumers take end = begin + 1.
+struct MsdAux {
+    uint32_t *begin1, *cap1, *cur1, *end1, *tile_start;            // [NB_MAX + 2] each
+    uint32_t *begin2, *cap2, *cur2, *end2;                         // [nfb + 2] each (cap2 and cur2 adjacent: one memset)
+    static uint64_t words(uint32_t nfb) { return 5ull * (NB_MAX + 2) + 4ull * ((uint64_t)nfb + 2); }
+    MsdAux(uint32_t* x, uint32_t nfb) {
+        const uint64_t s1 = NB_MAX + 2, s2 = (uint64_t)nfb + 2;
+        begin1 = x; cap1 = begin1 + s1; cur1 = cap1 + s1; end1 = cur1 + s1; tile_start = end1 + s1;
+        begin2 = tile_start + s1; cap2 = begin2 + s2; cur2 = cap2 + s2; end2 = cur2 + s2;
+    }
+};
+
 // What the partition leaves behind (kept per context: `yacht run` probes many samples against one partitioned reference)
 struct MsdPartState {
     MsdPlan p;
     int sbits = 0, rest_bits = 0;
     const uint64_t* final_ent = nullptr;
-    const uint32_t* final_base = nullptr;
+    const uint32_t* final_begin = nullptr;     // final bucket b: words [final_begin[b], final_end[b]) of final_ent
+    const uint32_t* final_end = nullptr;
     uint32_t nbuckets = 0;
     uint64_t largest = 0;
 };
@@ -1350,8 +1416,25 @@ int bitlen(uint64_t v) {
     return b;
 }
 
+// Slot capacity of a bucket of the leading `bits` hash bits.  Sketch hashes are FracMinHash values, uniform in [0, maxkey], so a
+// full bucket expects mean = T * 2^(hb - bits) / (maxkey + 1) words; the capacity is f * mean + add, rounded up to 16 words
+// (every slot starts 16-byte aligned, as the bulk copies need).
+uint64_t slot_capacity(uint64_t T, uint64_t maxkey, int hb, int bits, double f, double add) {
+    const double mean = (double)T * std::ldexp(1.0, hb - bits) / ((double)maxkey + 1.0);
+    const double c = std::ceil(f * mean + add);
+    if (!(c < 4294967296.0)) return 1ull << 32;
+    return ((uint64_t)c + 15ull) & ~15ull;
+}
+
 // Partition + grouping of the resident sketches on one GPU.  partition_only: stop after the partition (the run path probes
 // it, run_buckets.cuh).  *used = 0 when the input does not qualify for this path.
+//
+// Bucket layout.  Slotted (the rule): bucket b of a level owns a fixed slot of C words at b * C, C from the plan alone
+// (slot_capacity), so the scatters need no histogram; a (tile, digit) run that would pass its slot's end is cut and raises that
+// level's overflow flag, which the host reads at the one synchronisation after the partition.  Exact (the fallback): a
+// histogram pass sizes every bucket.  A level-2 overflow repeats level 2 on the exact layout; a level-1 overflow repeats the
+// whole partition on it (level 2 ran on cut buckets).  Slot positions must fit 32 bits (work items address postings by
+// position), otherwise the exact layout is taken from the start.
 int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only = false) {
     *used = 0;
     ctx->part_valid = false;
@@ -1387,106 +1470,176 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
     const int sbits = std::max(0, std::min(GK_SUBBITS, key_bits));
     const int rest_bits = key_bits - sbits;                // compared inside a sub-bucket (32 low bits + the rest beside the genome id)
     if (!partition_only && rest_bits > 32 && rest_bits - 32 + p.gb > 32) return 0;     // does not fit the candidate arrays: general path
+    // Slot capacities.  Level 1: 2 % over the mean plus one scatter tile -- at 85 205 genomes a full bucket averages 822 516 words
+    // and the largest holds 827 327 (+0.6 %).  Level 2: 25 % over the mean plus 64 -- at 85 205 genomes the buckets average
+    // 804 words with a standard deviation of 35.5 (Poisson: 28.4; clusters of related genomes widen it) and the largest holds
+    // 984, against C2 = 1 072, 7.5 deviations over the mean.  A database that fills a slot anyway is re-partitioned exactly.
+    const uint64_t C1 = slot_capacity(T, maxkey, p.hb, d1, 1.02, (double)SC_TILE);
+    const uint64_t C2 = slot_capacity(T, maxkey, p.hb, d1 + d2, 1.25, 64.0);
+    // Positions in a level's buffer, and behind the final one the postings of oversized buckets (at most T words), must fit 32
+    // bits: slot space + T < 2^32.  (400 000 genomes, T = 2.1e9: the exact layout from the start.)
+    const bool slots_fit = C1 * p.nb1 + T < (1ull << 32) && (!d2 || C2 * p.nfb + T < (1ull << 32));
 
     // ---- buffers ----------------------------------------------------------------------------------
-    YG_CHECK(dev_alloc(ctx, &ctx->d_ent1, T));
-    if (d2) YG_CHECK(dev_alloc(ctx, &ctx->d_ent2, T));
-    const uint64_t aux_words = 3ull * (NB_MAX + 2) + 3ull * ((uint64_t)p.nfb + 2);
+    const uint64_t aux_words = MsdAux::words(p.nfb);
     YG_CHECK(dev_alloc(ctx, &ctx->d_msd_aux, aux_words));
-    uint32_t* hist1 = ctx->d_msd_aux;
-    uint32_t* base1 = hist1 + (NB_MAX + 2);
-    uint32_t* tile_start = base1 + (NB_MAX + 2);
-    uint32_t* hist2 = tile_start + (NB_MAX + 2);
-    uint32_t* base2 = hist2 + ((uint64_t)p.nfb + 2);
-    uint32_t* cursor = base2 + ((uint64_t)p.nfb + 2);      // level-1 cursors first, then reused for level 2
-    YG_CUDA(ctx, cudaMemsetAsync(ctx->d_msd_aux, 0, aux_words * sizeof(uint32_t), st));
-    YG_CUDA(ctx, cudaMemsetAsync(&ctx->d_scalars[SCM_PCUR], 0, 5 * sizeof(unsigned long long), st));
-
-    YG_CUDA(ctx, cudaEventRecord(ctx->ev[0], st));
-    // ---- level 1 ----------------------------------------------------------------------------------
-    YG_CUDA(ctx, cudaEventRecord(ctx->evp[0], st));
-    k2_hist1<<<ctx->num_sms * 8, 256, p.nb1 * sizeof(uint32_t), st>>>(ctx->d_hashes, p, hist1);
-    YG_CUDA(ctx, cudaGetLastError());
-    YG_CUDA(ctx, cudaEventRecord(ctx->evp[1], st));
-    k2_prep1<<<1, 1024, 0, st>>>(hist1, p.nb1, base1, tile_start, cursor, ctx->d_scalars);
-    YG_CUDA(ctx, cudaGetLastError());
+    const MsdAux x(ctx->d_msd_aux, p.nfb);
+    const uint32_t units1 = (uint32_t)((T + SC_TILE - 1) / SC_TILE);
+    const uint64_t max_units = T / SC_TILE + p.nb1 + 1;
+    YG_CHECK(dev_alloc(ctx, &ctx->d_tile_g0, (uint64_t)units1 + 1));
+    if (d2) YG_CHECK(dev_alloc(ctx, &ctx->d_units, 2 * max_units));
     const uint64_t T_mine = T;
     ScatterArgs a{};
-    a.hashes = ctx->d_hashes; a.offsets = ctx->d_offsets; a.n = n; a.out_ent = ctx->d_ent1; a.cursor = cursor;
-    a.base1 = base1; a.tile_start = tile_start; a.hist2 = hist2;
-    const uint32_t units1 = (uint32_t)((T + SC_TILE - 1) / SC_TILE);
+    a.hashes = ctx->d_hashes; a.offsets = ctx->d_offsets; a.n = n; a.tile_g0 = ctx->d_tile_g0;
+    a.tile_start = x.tile_start; a.hist2 = x.cap2; a.units = (const uint2*)ctx->d_units;
+    const size_t smem1 = (size_t)2 * SC_BUF * 8 + (size_t)p.nb1 * 16 + (size_t)SC_TILE * 2;
+    const size_t smem2 = (size_t)2 * SC_BUF * 8 + (size_t)(1u << d2) * 16 + (size_t)SC_TILE * 2;
+    int grid1 = 1, grid2 = 1;
     {
-        // genome of the first hash slot of every level-1 tile (the scatter derives genome ids from the CSR offsets)
-        YG_CHECK(dev_alloc(ctx, &ctx->d_tile_g0, (uint64_t)units1 + 1));
-        k2_tile_g0<<<grid_for(ctx, (uint64_t)units1 + 1, 256, 8), 256, 0, st>>>(ctx->d_offsets, n, T, units1, ctx->d_tile_g0);
-        YG_CUDA(ctx, cudaGetLastError());
-        a.tile_g0 = ctx->d_tile_g0;
-        const size_t smem = (size_t)2 * SC_BUF * 8 + (size_t)p.nb1 * 12 + (size_t)SC_TILE * 2;
-        YG_CUDA(ctx, cudaFuncSetAttribute(k2_scatter<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int occ = 1;
-        YG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k2_scatter<1, false>, SC_THREADS, smem));
-        const int grid = (int)std::min<uint64_t>(units1, (uint64_t)ctx->num_sms * std::max(occ, 1));
+        YG_CUDA(ctx, cudaFuncSetAttribute(k2_scatter<1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem1));
+        YG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k2_scatter<1, false>, SC_THREADS, smem1));
+        grid1 = (int)std::min<uint64_t>(units1, (uint64_t)ctx->num_sms * std::max(occ, 1));
+        if (d2) {
+            YG_CUDA(ctx, cudaFuncSetAttribute(k2_scatter<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
+            YG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k2_scatter<2, false>, SC_THREADS, smem2));
+            grid2 = ctx->num_sms * std::max(occ, 1);
+        }
+    }
+    bool ran_hist1 = false, ran_hist2 = false;
+
+    // level 1: raw hashes -> packed words in d_ent1, by leading digit
+    auto level1 = [&](bool exact) -> int {
+        YG_CUDA(ctx, cudaMemsetAsync(ctx->d_msd_aux, 0, aux_words * sizeof(uint32_t), st));
+        YG_CUDA(ctx, cudaMemsetAsync(&ctx->d_scalars[SCM_PCUR], 0, (SCM_OVF2 + 1 - SCM_PCUR) * sizeof(unsigned long long), st));
+        YG_CHECK(dev_alloc(ctx, &ctx->d_ent1, exact ? T : std::max<uint64_t>(T, C1 * p.nb1)));
+        a.out_ent = ctx->d_ent1; a.cursor = x.cur1; a.ovf = &ctx->d_scalars[SCM_OVF1];
+        a.slot = exact ? 0u : (uint32_t)C1;
+        if (exact) {
+            YG_CUDA(ctx, cudaEventRecord(ctx->evp[0], st));
+            k2_hist1<<<ctx->num_sms * 8, 256, p.nb1 * sizeof(uint32_t), st>>>(ctx->d_hashes, p, x.cap1);
+            YG_CUDA(ctx, cudaGetLastError());
+            YG_CUDA(ctx, cudaEventRecord(ctx->evp[1], st));
+            k2_prep1<<<1, 1024, 0, st>>>(x.cap1, nullptr, p.nb1, x.begin1, nullptr, x.cur1, x.tile_start, ctx->d_scalars);
+            ran_hist1 = true;
+        } else {
+            k2_slots<<<grid_for(ctx, (uint64_t)p.nb1 + 1, 256, 8), 256, 0, st>>>(p.nb1, (uint32_t)C1, x.begin1, x.cap1);
+        }
+        YG_CUDA(ctx, cudaGetLastError());
         YG_CUDA(ctx, cudaEventRecord(ctx->evp[2], st));
-        k2_scatter<1, false><<<grid, SC_THREADS, smem, st>>>(a, p, 0u, units1);
+        k2_scatter<1, false><<<grid1, SC_THREADS, smem1, st>>>(a, p, 0u, units1);
         YG_CUDA(ctx, cudaGetLastError());
         YG_CUDA(ctx, cudaEventRecord(ctx->evp[3], st));
-    }
-    ctx->tm.n_kernel_launches += 4;
-    const uint64_t* final_ent = ctx->d_ent1;
-    const uint32_t* final_base = base1;
-    // ---- level 2 ----------------------------------------------------------------------------------
-    if (d2) {
+        if (!exact) {
+            k2_prep1<<<1, 1024, 0, st>>>(x.cur1, x.cap1, p.nb1, x.begin1, x.end1, nullptr, x.tile_start, ctx->d_scalars);
+            YG_CUDA(ctx, cudaGetLastError());
+        }
+        ctx->tm.n_kernel_launches += 3;
+        return 0;
+    };
+    // level 2: words -> final buckets in d_ent2, by the next d2 bits (the level-1 units are laid out once per level-1 pass)
+    auto level2 = [&](bool exact, bool units) -> int {
+        YG_CHECK(dev_alloc(ctx, &ctx->d_ent2, exact ? T : std::max<uint64_t>(T, C2 * p.nfb)));
         a.in_ent = ctx->d_ent1; a.out_ent = ctx->d_ent2;
-        const uint64_t max_units = T / SC_TILE + p.nb1 + 1;
-        YG_CHECK(dev_alloc(ctx, &ctx->d_units, 2 * max_units));
-        k2_units<<<grid_for(ctx, max_units, 256, 8), 256, 0, st>>>(tile_start, base1, p.nb1, (uint2*)ctx->d_units);
-        YG_CUDA(ctx, cudaGetLastError());
-        ctx->tm.n_kernel_launches += 1;
-        a.units = (const uint2*)ctx->d_units;
-        const int grid_h = ctx->num_sms * 8;
-        k2_hist2<<<grid_h, 256, (size_t)(1u << d2) * sizeof(uint32_t), st>>>(a, p, p.unit_hi);
-        YG_CUDA(ctx, cudaGetLastError());
-        YG_CUDA(ctx, cudaEventRecord(ctx->evp[4], st));
-        // final-bucket bases: a rank's own buckets are contiguous, foreign ones are empty -> positions are local
-        size_t tb = 0;
-        YG_CUDA(ctx, cub::DeviceScan::ExclusiveSum(nullptr, tb, hist2, base2, (int64_t)p.nfb + 1, st));
-        size_t tb2 = 0;
-        YG_CUDA(ctx, cub::DeviceReduce::Max(nullptr, tb2, hist2, (uint32_t*)&ctx->d_scalars[SCM_MAXB + 1], (int64_t)p.nfb, st));
-        YG_CHECK(ygpu_temp_reserve(ctx, std::max(tb, tb2)));
-        tb = ctx->temp_bytes;
-        YG_CUDA(ctx, cub::DeviceScan::ExclusiveSum(ctx->d_temp, tb, hist2, base2, (int64_t)p.nfb + 1, st));
-        tb = ctx->temp_bytes;
-        YG_CUDA(ctx, cub::DeviceReduce::Max(ctx->d_temp, tb, hist2, (uint32_t*)&ctx->d_scalars[SCM_MAXB + 1], (int64_t)p.nfb, st));
-        ctx->tm.n_library_launches += 4;
-        YG_CUDA(ctx, cudaMemcpyAsync(cursor, base2, ((uint64_t)p.nfb + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
-        a.cursor = cursor;
-        const size_t smem = (size_t)2 * SC_BUF * 8 + (size_t)(1u << d2) * 12 + (size_t)SC_TILE * 2;
-        YG_CUDA(ctx, cudaFuncSetAttribute(k2_scatter<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int occ = 1;
-        YG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k2_scatter<2, false>, SC_THREADS, smem));
-        const int grid = ctx->num_sms * std::max(occ, 1);
+        a.cursor = x.cur2; a.ovf = &ctx->d_scalars[SCM_OVF2];
+        a.slot = exact ? 0u : (uint32_t)C2;
+        if (units) {
+            k2_units<<<grid_for(ctx, max_units, 256, 8), 256, 0, st>>>(x.tile_start, x.begin1, ran_hist1 ? x.begin1 + 1 : x.end1, p.nb1,
+                                                                       (uint2*)ctx->d_units);
+            YG_CUDA(ctx, cudaGetLastError());
+            ctx->tm.n_kernel_launches += 1;
+        }
+        if (exact) {
+            YG_CUDA(ctx, cudaEventRecord(ctx->evp[12], st));
+            k2_hist2<<<ctx->num_sms * 8, 256, (size_t)(1u << d2) * sizeof(uint32_t), st>>>(a, p, p.unit_hi);
+            YG_CUDA(ctx, cudaGetLastError());
+            YG_CUDA(ctx, cudaEventRecord(ctx->evp[4], st));
+            // final-bucket bases and the largest bucket
+            size_t tb = 0, tb2 = 0;
+            YG_CUDA(ctx, cub::DeviceScan::ExclusiveSum(nullptr, tb, x.cap2, x.begin2, (int64_t)p.nfb + 1, st));
+            YG_CUDA(ctx, cub::DeviceReduce::Max(nullptr, tb2, x.cap2, (uint32_t*)&ctx->d_scalars[SCM_MAXB + 1], (int64_t)p.nfb, st));
+            YG_CHECK(ygpu_temp_reserve(ctx, std::max(tb, tb2)));
+            tb = ctx->temp_bytes;
+            YG_CUDA(ctx, cub::DeviceScan::ExclusiveSum(ctx->d_temp, tb, x.cap2, x.begin2, (int64_t)p.nfb + 1, st));
+            tb = ctx->temp_bytes;
+            YG_CUDA(ctx, cub::DeviceReduce::Max(ctx->d_temp, tb, x.cap2, (uint32_t*)&ctx->d_scalars[SCM_MAXB + 1], (int64_t)p.nfb, st));
+            ctx->tm.n_library_launches += 4;
+            ctx->tm.n_kernel_launches += 1;
+            YG_CUDA(ctx, cudaMemcpyAsync(x.cur2, x.begin2, (uint64_t)p.nfb * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+            ran_hist2 = true;
+        } else {
+            k2_slots<<<grid_for(ctx, (uint64_t)p.nfb + 1, 256, 8), 256, 0, st>>>(p.nfb, (uint32_t)C2, x.begin2, x.cap2);
+            YG_CUDA(ctx, cudaGetLastError());
+            ctx->tm.n_kernel_launches += 1;
+        }
         YG_CUDA(ctx, cudaEventRecord(ctx->evp[5], st));
-        k2_scatter<2, false><<<grid, SC_THREADS, smem, st>>>(a, p, p.unit_lo, p.unit_hi);
+        k2_scatter<2, false><<<grid2, SC_THREADS, smem2, st>>>(a, p, p.unit_lo, p.unit_hi);
         YG_CUDA(ctx, cudaGetLastError());
         YG_CUDA(ctx, cudaEventRecord(ctx->evp[6], st));
-        ctx->tm.n_kernel_launches += 2;
-        final_ent = ctx->d_ent2;
-        final_base = base2;
+        ctx->tm.n_kernel_launches += 1;
+        if (!exact) {
+            k2_ends<<<grid_for(ctx, p.nfb, 256, 8), 256, 0, st>>>(x.cur2, x.cap2, x.begin2, p.nfb, x.end2, &ctx->d_scalars[SCM_MAXB + 1]);
+            YG_CUDA(ctx, cudaGetLastError());
+            ctx->tm.n_kernel_launches += 1;
+        }
+        return 0;
+    };
+    // largest buckets of both levels and the overflow flags, at the one synchronisation after the partition
+    unsigned long long rb[SCM_OVF2 + 1 - SCM_MAXB] = {};
+    auto read_back = [&]() -> int {
+        YG_CUDA(ctx, cudaMemcpyAsync(rb, &ctx->d_scalars[SCM_MAXB], sizeof rb, cudaMemcpyDeviceToHost, st));
+        YG_CUDA(ctx, cudaEventRecord(ctx->ev[1], st));
+        YG_CUDA(ctx, cudaStreamSynchronize(st));
+        return 0;
+    };
+
+    YG_CUDA(ctx, cudaEventRecord(ctx->ev[0], st));
+    // genome of the first hash slot of every level-1 tile (the scatter derives genome ids from the CSR offsets)
+    k2_tile_g0<<<grid_for(ctx, (uint64_t)units1 + 1, 256, 8), 256, 0, st>>>(ctx->d_offsets, n, T, units1, ctx->d_tile_g0);
+    YG_CUDA(ctx, cudaGetLastError());
+    ctx->tm.n_kernel_launches += 1;
+    bool exact1 = !slots_fit;
+    YG_CHECK(level1(exact1));
+    if (d2) YG_CHECK(level2(exact1, true));
+    YG_CHECK(read_back());
+    if (!exact1 && rb[SCM_OVF1 - SCM_MAXB]) {
+        // a level-1 slot overflowed: everything after it ran on cut buckets -- the whole partition again, exactly
+        exact1 = true;
+        YG_CHECK(level1(true));
+        if (d2) YG_CHECK(level2(true, true));
+        YG_CHECK(read_back());
+    } else if (d2 && !exact1 && rb[SCM_OVF2 - SCM_MAXB]) {
+        YG_CUDA(ctx, cudaMemsetAsync(x.cap2, 0, 2 * ((uint64_t)p.nfb + 2) * sizeof(uint32_t), st));      // histogram + cursors
+        YG_CUDA(ctx, cudaMemsetAsync(&ctx->d_scalars[SCM_MAXB + 1], 0, sizeof(unsigned long long), st));
+        YG_CHECK(level2(true, false));
+        YG_CHECK(read_back());
     }
+    const uint64_t* final_ent = d2 ? ctx->d_ent2 : ctx->d_ent1;
+    const uint32_t* final_begin = d2 ? x.begin2 : x.begin1;
+    const uint32_t* final_end = d2 ? (ran_hist2 ? x.begin2 + 1 : x.end2) : (ran_hist1 ? x.begin1 + 1 : x.end1);
+    // positions in the final buffer: the slot space, or T (exact layout)
+    const uint64_t final_words = d2 ? (ran_hist2 ? T : std::max<uint64_t>(T, C2 * p.nfb)) : (ran_hist1 ? T : std::max<uint64_t>(T, C1 * p.nb1));
     // largest final bucket decides whether the shared-memory grouping applies
-    unsigned long long maxb[2] = {0, 0};
-    YG_CUDA(ctx, cudaMemcpyAsync(maxb, &ctx->d_scalars[SCM_MAXB], sizeof maxb, cudaMemcpyDeviceToHost, st));
-    YG_CUDA(ctx, cudaEventRecord(ctx->ev[1], st));
-    YG_CUDA(ctx, cudaStreamSynchronize(st));
-    const uint64_t largest = d2 ? (uint64_t)(uint32_t)maxb[1] : (uint64_t)maxb[0];   // (level-1 maximum: over all digits, a safe bound)
+    const uint64_t largest = d2 ? (uint64_t)(uint32_t)rb[1] : (uint64_t)rb[0];   // (level-1 maximum: over all digits, a safe bound)
     const uint32_t nbuckets = d2 ? p.nfb : p.nb1;
     {
         if (!ctx->part_state) ctx->part_state = new MsdPartState();
         MsdPartState* ps = (MsdPartState*)ctx->part_state;
-        ps->p = p; ps->sbits = sbits; ps->rest_bits = rest_bits; ps->final_ent = final_ent; ps->final_base = final_base;
+        ps->p = p; ps->sbits = sbits; ps->rest_bits = rest_bits; ps->final_ent = final_ent;
+        ps->final_begin = final_begin; ps->final_end = final_end;
         ps->nbuckets = nbuckets; ps->largest = largest;
         ctx->part_valid = true;
     }
+    auto record_phases = [&]() {
+        auto el = [&](int x0, int y0) { float ms = 0.f; cudaEventElapsedTime(&ms, ctx->evp[x0], ctx->evp[y0]); return (double)ms; };
+        // phase times of the partition that was kept (a discarded slotted attempt shows in ms_sort only)
+        if (ran_hist1) ctx->tm.ms_hist1 += el(0, 1);
+        ctx->tm.ms_scatter1 += el(2, 3);
+        if (d2) {
+            if (ran_hist2) ctx->tm.ms_hist2 += el(12, 4);
+            ctx->tm.ms_scatter2 += el(5, 6);
+        }
+    };
     if (partition_only) {
         ctx->tm.ms_sort += elapsed(ctx, 0, 1);
         *used = 1;
@@ -1504,7 +1657,8 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
         if (ok) {
             YG_CHECK(dev_alloc(ctx, &ctx->d_big_list, (uint64_t)nbuckets));
             YG_CUDA(ctx, cudaMemsetAsync(&ctx->d_scalars[SCM_STREAM], 0, sizeof(unsigned long long), st));
-            k2_big_list<<<grid_for(ctx, nbuckets, 256, 8), 256, 0, st>>>(final_base, 0, nbuckets, ctx->d_big_list, nbuckets, ctx->d_scalars);
+            k2_big_list<<<grid_for(ctx, nbuckets, 256, 8), 256, 0, st>>>(final_begin, final_end, 0, nbuckets, ctx->d_big_list, nbuckets,
+                                                                        ctx->d_scalars);
             YG_CUDA(ctx, cudaGetLastError());
             unsigned long long nb = 0;
             YG_CUDA(ctx, cudaMemcpyAsync(&nb, &ctx->d_scalars[SCM_STREAM], sizeof nb, cudaMemcpyDeviceToHost, st));
@@ -1515,12 +1669,13 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
                 big_list.resize(n_big);
                 YG_CUDA(ctx, cudaMemcpy(big_list.data(), ctx->d_big_list, (size_t)n_big * sizeof(uint32_t), cudaMemcpyDeviceToHost));
                 std::sort(big_list.begin(), big_list.end());          // deterministic ordinals
-                std::vector<uint32_t> hb(nbuckets + 1);
-                YG_CUDA(ctx, cudaMemcpy(hb.data(), final_base, ((size_t)nbuckets + 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+                std::vector<uint32_t> hb(nbuckets), he(nbuckets);
+                YG_CUDA(ctx, cudaMemcpy(hb.data(), final_begin, (size_t)nbuckets * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+                YG_CUDA(ctx, cudaMemcpy(he.data(), final_end, (size_t)nbuckets * sizeof(uint32_t), cudaMemcpyDeviceToHost));
                 big_cstart.assign((size_t)n_big + 1, 0);
-                for (uint32_t j = 0; j < n_big; j++) big_cstart[j + 1] = big_cstart[j] + (hb[big_list[j] + 1] - hb[big_list[j]]);
+                for (uint32_t j = 0; j < n_big; j++) big_cstart[j + 1] = big_cstart[j] + (he[big_list[j]] - hb[big_list[j]]);
                 N_big = big_cstart[n_big];
-                ok = T + N_big + 4 < (1ull << 32);
+                ok = final_words + N_big + 4 < (1ull << 32);
             }
             YG_CUDA(ctx, cudaMemsetAsync(&ctx->d_scalars[SCM_STREAM], 0, sizeof(unsigned long long), st));
         }
@@ -1531,13 +1686,13 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
     }
 
     // ---- buckets -> postings + per-genome work lists (or the group stream) ------------------------------
-    YG_CHECK(dev_alloc(ctx, &ctx->d_post, T + N_big));
+    YG_CHECK(dev_alloc(ctx, &ctx->d_post, final_words + N_big));      // postings of oversized buckets: behind the final buffer's positions
     YG_CHECK(dev_alloc(ctx, &ctx->d_row_items, T));
     YG_CHECK(dev_alloc(ctx, &ctx->d_row_cnt, (uint64_t)n + 1));
     YG_CUDA(ctx, cudaMemsetAsync(ctx->d_row_cnt, 0, ((uint64_t)n + 1) * sizeof(unsigned long long), st));
     {
         GroupArgs g{};
-        g.ent = final_ent; g.base = final_base; g.gb = p.gb;
+        g.ent = final_ent; g.begin = final_begin; g.end = final_end; g.gb = p.gb;
         g.nb = d2 ? p.nfb : p.nb1;
         g.b_lo = d2 ? (p.dlo << d2) : p.dlo;
         g.b_hi = d2 ? (p.dhi << d2) : p.dhi;
@@ -1603,7 +1758,7 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
             const uint64_t words = big_cstart[c1] - big_cstart[c0];
             for (uint32_t j = 0; j <= nc; j++) rel[j] = big_cstart[c0 + j] - big_cstart[c0];
             YG_CUDA(ctx, cudaMemcpyAsync(ctx->d_big_cstart, rel.data(), ((size_t)nc + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
-            k2_big_gather<<<(unsigned)std::min<uint32_t>(nc, (uint32_t)ctx->num_sms * 8), 256, 0, st>>>(final_ent, final_base, ctx->d_big_list + c0, ctx->d_big_cstart,
+            k2_big_gather<<<(unsigned)std::min<uint32_t>(nc, (uint32_t)ctx->num_sms * 8), 256, 0, st>>>(final_ent, final_begin, final_end, ctx->d_big_list + c0, ctx->d_big_cstart,
                                                                                                      nc, low_bits, ctx->d_big_a);
             YG_CUDA(ctx, cudaGetLastError());
             const int end_bit = std::min(64, low_bits + bitlen((uint64_t)nc - 1));
@@ -1613,7 +1768,7 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
             tb = ctx->temp_bytes;
             YG_CUDA(ctx, cub::DeviceRadixSort::SortKeys(ctx->d_temp, tb, ctx->d_big_a, ctx->d_big_b, (int64_t)words, 0, std::max(end_bit, 1), st));
             ctx->tm.n_library_launches += 2 + (std::max(end_bit, 1) + 7) / 8;
-            k2_big_groups<<<grid_for(ctx, words, 256, 8), 256, 0, st>>>(ctx->d_big_b, words, p.gb, T + big_cstart[c0], p.gb <= YG_ITEM_INLINE_BITS ? 1 : 0, ctx->d_post,
+            k2_big_groups<<<grid_for(ctx, words, 256, 8), 256, 0, st>>>(ctx->d_big_b, words, p.gb, final_words + big_cstart[c0], p.gb <= YG_ITEM_INLINE_BITS ? 1 : 0, ctx->d_post,
                                                                         ctx->d_offsets, ctx->d_row_cnt, ctx->d_row_items, ctx->d_scalars);
             YG_CUDA(ctx, cudaGetLastError());
             ctx->tm.n_kernel_launches += 2;
@@ -1632,12 +1787,11 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
     const uint64_t I = P - (sc[SC_HEADS] - sc[SC_SINGLE]);
     ctx->tm.ms_sort += elapsed(ctx, 0, 1);
     ctx->tm.ms_index += elapsed(ctx, 1, 2);
+    record_phases();
     {
-        auto el = [&](int x, int y) { float ms = 0.f; cudaEventElapsedTime(&ms, ctx->evp[x], ctx->evp[y]); return (double)ms; };
-        ctx->tm.ms_hist1 += el(0, 1);
-        ctx->tm.ms_scatter1 += el(2, 3);
-        if (d2) { ctx->tm.ms_hist2 += el(3, 4); ctx->tm.ms_scatter2 += el(5, 6); }
-        ctx->tm.ms_group += el(7, 8);
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, ctx->evp[7], ctx->evp[8]);
+        ctx->tm.ms_group += ms;
     }
     ctx->P = P;
     ctx->n_items = I;
@@ -1755,7 +1909,7 @@ int ygpu_run_counts_buckets(ygpu_ctx* ctx, const uint64_t* d_sample, uint64_t n_
         ctx->tm.n_kernel_launches += 2;
     }
     RunBucketArgs a{};
-    a.ent = ps.final_ent; a.base = ps.final_base; a.nb = nb; a.gb = p.gb;
+    a.ent = ps.final_ent; a.begin = ps.final_begin; a.end = ps.final_end; a.nb = nb; a.gb = p.gb;
     a.sub_shift = p.gb + ps.rest_bits; a.sub_mask = (1u << ps.sbits) - 1u; a.rest_bits = ps.rest_bits;
     a.key_mask = key_mask; a.skeys = r->d_skeys; a.sbase = sbase; a.ntbits = r->d_ntbits; a.counts = d_counts;
     const size_t smem = sizeof(RunSmem);
@@ -2108,7 +2262,7 @@ extern "C" int ygpu_train_step_sharded(ygpu_ctx* ctx, double threshold, ygpu_ind
     YG_CHECK(dev_alloc(ctx, &ctx->d_sh_hist_all, (uint64_t)(N + 1) * NB_MAX));
     YG_CHECK(dev_alloc(ctx, &ctx->d_sh_owner, (uint64_t)NB_MAX));
     YG_CHECK(dev_alloc(ctx, &ctx->d_sh_info, (uint64_t)SHI_WORDS));
-    const uint64_t aux_words = 3ull * (NB_MAX + 2) + 3ull * ((uint64_t)p.nfb + 2);
+    const uint64_t aux_words = MsdAux::words(p.nfb);
     YG_CHECK(dev_alloc(ctx, &ctx->d_msd_aux, aux_words));
     const uint32_t units1 = (uint32_t)((T + SC_TILE - 1) / SC_TILE);
     YG_CHECK(dev_alloc(ctx, &ctx->d_tile_g0, (uint64_t)units1 + 2));
@@ -2134,12 +2288,8 @@ extern "C" int ygpu_train_step_sharded(ygpu_ctx* ctx, double threshold, ygpu_ind
             ctx->sh_shared_item = ctx->d_inbox_item; ctx->sh_shared_row = ctx->d_inbox_row;
         }
     }
-    uint32_t* hist1 = ctx->d_msd_aux;
-    uint32_t* base1 = hist1 + (NB_MAX + 2);
-    uint32_t* tile_start = base1 + (NB_MAX + 2);
-    uint32_t* hist2 = tile_start + (NB_MAX + 2);
-    uint32_t* base2 = hist2 + ((uint64_t)p.nfb + 2);
-    uint32_t* cursor = base2 + ((uint64_t)p.nfb + 2);
+    // exact layout (every rank's histograms are exchanged anyway): bucket b spans [begin[b], begin[b + 1]); the histograms are the caps
+    const MsdAux x(ctx->d_msd_aux, p.nfb);
     YG_CUDA(ctx, cudaEventRecord(ctx->ev[0], st));
     YG_CUDA(ctx, cudaMemsetAsync(ctx->d_msd_aux, 0, aux_words * sizeof(uint32_t), st));
     YG_CUDA(ctx, cudaMemsetAsync(ctx->d_scalars, 0, REP_WORDS * sizeof(unsigned long long), st));
@@ -2149,21 +2299,23 @@ extern "C" int ygpu_train_step_sharded(ygpu_ctx* ctx, double threshold, ygpu_ind
     //         Hash-range residency: purely local -- this rank already holds exactly the hashes of its range. ---------------------
     YG_CUDA(ctx, cudaEventRecord(ctx->evp[0], st));
     if (T) {
-        k2_hist1<<<ctx->num_sms * 8, 256, p.nb1 * sizeof(uint32_t), st>>>(ctx->d_hashes, p, hist1);
+        k2_hist1<<<ctx->num_sms * 8, 256, p.nb1 * sizeof(uint32_t), st>>>(ctx->d_hashes, p, x.cap1);
         YG_CUDA(ctx, cudaGetLastError());
     }
     YG_CUDA(ctx, cudaEventRecord(ctx->evp[1], st));
     ScatterArgs a{};
-    a.hashes = ctx->d_hashes; a.out_ent = ctx->d_ent1; a.cursor = cursor; a.base1 = base1; a.tile_start = tile_start; a.hist2 = hist2;
+    a.hashes = ctx->d_hashes; a.out_ent = ctx->d_ent1; a.tile_start = x.tile_start; a.hist2 = x.cap2;
+    a.cursor = x.cur1; a.ovf = &ctx->d_scalars[SCM_OVF1];
     if (hr) {
-        k2_prep1<<<1, 1024, 0, st>>>(hist1, p.nb1, base1, tile_start, cursor, ctx->d_scalars);
+        k2_prep1<<<1, 1024, 0, st>>>(x.cap1, nullptr, p.nb1, x.begin1, nullptr, x.cur1, x.tile_start, ctx->d_scalars);
         YG_CUDA(ctx, cudaGetLastError());
-        k2s_range<<<1, 1024, 0, st>>>(hist1, p.nb1, d2, (unsigned long long)T, ctx->d_sh_info);
+        k2s_range<<<1, 1024, 0, st>>>(x.cap1, p.nb1, d2, (unsigned long long)T, ctx->d_sh_info);
         YG_CUDA(ctx, cudaGetLastError());
         a.offsets = ctx->d_offsets; a.n = n; a.gid_base = 0;           // the resident CSR spans all genomes
     } else {
-        YG_CHECK(ygpu_comm_allgather(ctx, hist1, ctx->d_sh_hist_all, (size_t)NB_MAX * sizeof(uint32_t)));
-        k2s_prep<<<1, 1024, 0, st>>>(ctx->d_sh_hist_all, p.nb1, N, rank, d2, ctx->d_sh_owner, cursor, base1, tile_start, ctx->d_sh_info, ctx->d_scalars);
+        YG_CHECK(ygpu_comm_allgather(ctx, x.cap1, ctx->d_sh_hist_all, (size_t)NB_MAX * sizeof(uint32_t)));
+        k2s_prep<<<1, 1024, 0, st>>>(ctx->d_sh_hist_all, p.nb1, N, rank, d2, ctx->d_sh_owner, x.cur1, x.begin1, x.tile_start, ctx->d_sh_info,
+                                     ctx->d_scalars);
         YG_CUDA(ctx, cudaGetLastError());
         // the plan is the same on every rank, so every rank sees whether some rank would own more words than the exchange
         // buffers hold (a hash distribution far from uniform) and all of them stop here, before a single word is stored
@@ -2180,7 +2332,7 @@ extern "C" int ygpu_train_step_sharded(ygpu_ctx* ctx, double threshold, ygpu_ind
         k2_tile_g0<<<grid_for(ctx, (uint64_t)units1 + 1, 256, 8), 256, 0, st>>>(a.offsets, a.n, T, units1, ctx->d_tile_g0);
         YG_CUDA(ctx, cudaGetLastError());
         a.tile_g0 = ctx->d_tile_g0;
-        const size_t smem = (size_t)2 * SC_BUF * 8 + (size_t)p.nb1 * (hr ? 12 : 20) + (size_t)SC_TILE * 2;
+        const size_t smem = (size_t)2 * SC_BUF * 8 + (size_t)p.nb1 * (hr ? 16 : 24) + (size_t)SC_TILE * 2;
         auto kern = hr ? k2_scatter<1, false> : k2_scatter<1, true>;
         YG_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int occ = 1;
@@ -2200,27 +2352,27 @@ extern "C" int ygpu_train_step_sharded(ygpu_ctx* ctx, double threshold, ygpu_ind
 
     // ---- 2. level 2 + grouping on this rank's share of the hash space; groups stored into every rank's stream ---------
     const uint64_t* final_ent = ctx->d_ent1;
-    const uint32_t* final_base = base1;
+    const uint32_t* final_begin = x.begin1;
     if (d2) {
         a.in_ent = ctx->d_ent1; a.out_ent = ctx->d_ent2;
-        k2_units<<<grid_for(ctx, max_units, 256, 8), 256, 0, st>>>(tile_start, base1, p.nb1, (uint2*)ctx->d_units);
+        k2_units<<<grid_for(ctx, max_units, 256, 8), 256, 0, st>>>(x.tile_start, x.begin1, x.begin1 + 1, p.nb1, (uint2*)ctx->d_units);
         YG_CUDA(ctx, cudaGetLastError());
         a.units = (const uint2*)ctx->d_units;
         k2_hist2<<<ctx->num_sms * 8, 256, (size_t)(1u << d2) * sizeof(uint32_t), st>>>(a, p, 0xFFFFFFFFu);
         YG_CUDA(ctx, cudaGetLastError());
         YG_CUDA(ctx, cudaEventRecord(ctx->evp[4], st));
         size_t tb = 0, tb2 = 0;
-        YG_CUDA(ctx, cub::DeviceScan::ExclusiveSum(nullptr, tb, hist2, base2, (int64_t)p.nfb + 1, st));
-        YG_CUDA(ctx, cub::DeviceReduce::Max(nullptr, tb2, hist2, (uint32_t*)&ctx->d_scalars[SCM_MAXB + 1], (int64_t)p.nfb, st));
+        YG_CUDA(ctx, cub::DeviceScan::ExclusiveSum(nullptr, tb, x.cap2, x.begin2, (int64_t)p.nfb + 1, st));
+        YG_CUDA(ctx, cub::DeviceReduce::Max(nullptr, tb2, x.cap2, (uint32_t*)&ctx->d_scalars[SCM_MAXB + 1], (int64_t)p.nfb, st));
         YG_CHECK(ygpu_temp_reserve(ctx, std::max(tb, tb2)));
         tb = ctx->temp_bytes;
-        YG_CUDA(ctx, cub::DeviceScan::ExclusiveSum(ctx->d_temp, tb, hist2, base2, (int64_t)p.nfb + 1, st));
+        YG_CUDA(ctx, cub::DeviceScan::ExclusiveSum(ctx->d_temp, tb, x.cap2, x.begin2, (int64_t)p.nfb + 1, st));
         tb = ctx->temp_bytes;
-        YG_CUDA(ctx, cub::DeviceReduce::Max(ctx->d_temp, tb, hist2, (uint32_t*)&ctx->d_scalars[SCM_MAXB + 1], (int64_t)p.nfb, st));
+        YG_CUDA(ctx, cub::DeviceReduce::Max(ctx->d_temp, tb, x.cap2, (uint32_t*)&ctx->d_scalars[SCM_MAXB + 1], (int64_t)p.nfb, st));
         ctx->tm.n_library_launches += 4;
-        YG_CUDA(ctx, cudaMemcpyAsync(cursor, base2, ((uint64_t)p.nfb + 1) * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
-        a.cursor = cursor;
-        const size_t smem = (size_t)2 * SC_BUF * 8 + (size_t)(1u << d2) * 12 + (size_t)SC_TILE * 2;
+        YG_CUDA(ctx, cudaMemcpyAsync(x.cur2, x.begin2, (uint64_t)p.nfb * sizeof(uint32_t), cudaMemcpyDeviceToDevice, st));
+        a.cursor = x.cur2; a.ovf = &ctx->d_scalars[SCM_OVF2];
+        const size_t smem = (size_t)2 * SC_BUF * 8 + (size_t)(1u << d2) * 16 + (size_t)SC_TILE * 2;
         YG_CUDA(ctx, cudaFuncSetAttribute(k2_scatter<2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         int occ = 1;
         YG_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k2_scatter<2, false>, SC_THREADS, smem));
@@ -2230,12 +2382,12 @@ extern "C" int ygpu_train_step_sharded(ygpu_ctx* ctx, double threshold, ygpu_ind
         YG_CUDA(ctx, cudaEventRecord(ctx->evp[6], st));
         ctx->tm.n_kernel_launches += 3;
         final_ent = ctx->d_ent2;
-        final_base = base2;
+        final_begin = x.begin2;
     }
     YG_CUDA(ctx, cudaEventRecord(ctx->ev[1], st));
     {
         GroupArgs g{};
-        g.ent = final_ent; g.base = final_base; g.gb = p.gb;
+        g.ent = final_ent; g.begin = final_begin; g.end = final_begin + 1; g.gb = p.gb;
         g.nb = d2 ? p.nfb : p.nb1;
         g.b_lo = 0; g.b_hi = g.nb; g.m_lo = 0;
         g.range = d2 ? &ctx->d_sh_info[SHI_BLO] : &ctx->d_sh_info[SHI_DLO];

@@ -18,7 +18,8 @@
 // Each pass streams the packed words once (8 bytes per hash slot) through bulk asynchronous copies.
 struct RunBucketArgs {
     const uint64_t* ent;            // partitioned reference words (remaining hash bits << gb | genome id)
-    const uint32_t* base;           // [nb + 1] final-bucket bases
+    const uint32_t* begin;          // final bucket b: words [begin[b], end[b]) of ent
+    const uint32_t* end;
     uint32_t nb;
     int gb;
     int sub_shift;                  // sub-bucket digit = (word >> sub_shift) & sub_mask
@@ -63,7 +64,7 @@ __global__ void __launch_bounds__(G2_THREADS, 4) k5_bucket(const RunBucketArgs a
     uint32_t b_next = blockIdx.x;                 // thread 0 only
     uint32_t pre_lo = 0, pre_hi = 0;
     auto preload = [&]() {
-        if (b_next < a.nb) { pre_lo = a.base[b_next]; pre_hi = a.base[b_next + 1]; }
+        if (b_next < a.nb) { pre_lo = a.begin[b_next]; pre_hi = a.end[b_next]; }
     };
     auto advance = [&](uint32_t par) {
         uint32_t bb = 0, m = 0, b = 0;
