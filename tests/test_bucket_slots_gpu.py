@@ -85,16 +85,16 @@ def test_run_path_after_slotted_build(gpu_ctx):
         assert np.array_equal(counts[k], exp[k]), k
 
 
-def level2_db(extra, seed):
-    """2 048 final buckets (hb 40, d1 6, d2 5) of 850 words, except bucket 700: C2 words, and bucket 1 500: C2 + extra.
+def level2_db(extra, seed, base=850):
+    """2 048 final buckets (hb 40, d1 6, d2 5) of `base` words, except bucket 700: C2 words, and bucket 1 500: C2 + extra.
     C2 depends on the word count, which depends on C2: iterate to the fixed point."""
     hb, D = 40, 11
-    sizes = [850] * (1 << D)
+    sizes = [base] * (1 << D)
     for _ in range(8):
         h, o = bucket_db(hb, D, sizes, seed)
         _, d1, d2, c1, c2 = plan(h, len(o) - 1)
         if sizes[700] == c2 and sizes[1500] == c2 + extra:
-            assert (d1, d2) == (6, 5) and 30 * 850 + 2 * c2 + extra <= c1
+            assert (d1, d2) == (6, 5) and 30 * base + 2 * c2 + extra <= c1
             return h, o, c2
         sizes[700], sizes[1500] = c2, c2 + extra
     raise AssertionError("slot capacity did not settle")

@@ -84,19 +84,35 @@ def test_alt_mut_rate_reference_kats_on_gpu(gpu_ctx):
         assert np.isclose(float(row["alt_confidence_mut_rate_with_coverage"]), exp)
 
 
-def _check_counts(ctx, db, sample, mask=None):
-    ctx.load_sketches(db.hashes, db.offsets)
-    got = ctx.exclusive_hashes(sample, mask)
+COUNT_FIELDS = ("n_overlap", "nontrivial", "n_exclusive", "n_match")
+
+
+def _check_counts(ctx, db, sample, mask=None, *, probe):
+    """Both run paths against the set oracle: run_path 1 (the bucket probe of run_buckets.cuh, when the input qualifies) and
+    run_path 0 (the general sort path).  `probe`: whether run_path 1 is expected to take the probe.  Which path answered is
+    read from the timers: ms_sample_kernels grows only when the probe ran."""
     exp = ro.exclusive_counts(db.hashes, db.offsets, sample, mask)
-    for f in ("n_overlap", "nontrivial", "n_exclusive", "n_match"):
-        assert np.array_equal(got[f], exp[f]), f
-    return got
+    ctx.load_sketches(db.hashes, db.offsets)
+    res = {}
+    for path in (1, 0):
+        ctx.set_option("run_path", path)
+        try:
+            ctx.reset_timers()
+            got = ctx.exclusive_hashes(sample, mask)
+            took_probe = ctx.timings()["ms_sample_kernels"] > 0.0
+        finally:
+            ctx.set_option("run_path", 1)
+        assert took_probe == (probe and path == 1), f"run_path {path}: probe expected {probe and path == 1}, taken {took_probe}"
+        for f in COUNT_FIELDS:
+            assert np.array_equal(got[f], exp[f]), f"run_path {path}: {f}"
+        res[path] = got
+    return res[1]
 
 
 def test_fixture20_known_answer(gpu_ctx):
     z = np.load(os.path.join(GOLD, "fixture20.npz"))
     db = synth.SketchDB(hashes=z["hashes"], offsets=z["offsets"], cluster=np.full(20, -1))
-    got = _check_counts(gpu_ctx, db, z["sample_hashes"])
+    got = _check_counts(gpu_ctx, db, z["sample_hashes"], probe=True)
     nt = np.flatnonzero(got["nontrivial"])
     assert len(nt) == 1 and str(z["names"][nt[0]]).startswith("CP032507.1")
     assert (int(got["n_exclusive"][nt[0]]), int(got["n_match"][nt[0]])) == (3741, 2)
@@ -106,7 +122,16 @@ def test_fixture20_known_answer(gpu_ctx):
 def test_exclusive_counts_synthetic(gpu_ctx, n, seed):
     db = synth.make_reference_db(n, seed, mean_size=400, sd_size=100)
     sample, present, cov = synth.make_sample(db, seed + 100, n_present=n // 5, total_hashes=60000)
-    _check_counts(gpu_ctx, db, sample)
+    got = _check_counts(gpu_ctx, db, sample, probe=True)
+    # the sample shuffled, with every tenth hash three times: membership is a set question
+    rng = np.random.default_rng(seed + 200)
+    _check_counts(gpu_ctx, db, rng.permutation(np.concatenate([sample, np.repeat(sample[::10], 2)])), probe=True)
+    # masks: nothing nontrivial, everything nontrivial, and only genomes that share no hash with the sample
+    _check_counts(gpu_ctx, db, sample, mask=np.zeros(n, np.uint8), probe=True)
+    _check_counts(gpu_ctx, db, sample, mask=np.ones(n, np.uint8), probe=True)
+    none = (got["n_overlap"] == 0).astype(np.uint8)
+    assert 0 < none.sum() < n
+    _check_counts(gpu_ctx, db, sample, mask=none, probe=True)
     # also after the index has been built on the same context (shared sorted array)
     gpu_ctx.build_index()
     got = gpu_ctx.exclusive_hashes(sample)
@@ -118,8 +143,29 @@ def test_exclusive_counts_edge_cases(gpu_ctx):
     parts = [np.array([1, 2, 3, 4], np.uint64), np.array([3, 4, 5, 5, 5], np.uint64), np.zeros(0, np.uint64),
              np.array([2**64 - 1, 7, 7], np.uint64), np.array([100, 200], np.uint64)]
     db = synth.from_sketches(parts)
-    _check_counts(gpu_ctx, db, np.array([5, 7, 2**64 - 1, 3, 3, 999], dtype=np.uint64))
-    _check_counts(gpu_ctx, db, np.zeros(0, dtype=np.uint64))                       # empty sample: nothing nontrivial
-    _check_counts(gpu_ctx, db, np.array([424242], dtype=np.uint64))                # no overlap at all
-    _check_counts(gpu_ctx, db, np.array([1], dtype=np.uint64), mask=np.array([1, 1, 1, 0, 1], np.uint8))  # explicit mask
-    _check_counts(gpu_ctx, db, np.array([0, 1, 2**63], dtype=np.uint64), mask=np.ones(5, np.uint8))
+    _check_counts(gpu_ctx, db, np.array([5, 7, 2**64 - 1, 3, 3, 999], dtype=np.uint64), probe=True)
+    _check_counts(gpu_ctx, db, np.zeros(0, dtype=np.uint64), probe=True)                       # empty sample: nothing nontrivial
+    _check_counts(gpu_ctx, db, np.array([424242], dtype=np.uint64), probe=True)                # no overlap at all
+    _check_counts(gpu_ctx, db, np.array([1], dtype=np.uint64), mask=np.array([1, 1, 1, 0, 1], np.uint8), probe=True)  # explicit mask
+    _check_counts(gpu_ctx, db, np.array([0, 1, 2**63], dtype=np.uint64), mask=np.ones(5, np.uint8), probe=True)
+    _check_counts(gpu_ctx, db, np.array([7, 3, 100], dtype=np.uint64), mask=np.zeros(5, np.uint8), probe=True)   # nothing nontrivial
+    # mask marking only genomes without overlap (0, 2, 4 share nothing with {7}): their hashes count as exclusive, no match
+    _check_counts(gpu_ctx, db, np.array([7], dtype=np.uint64), mask=np.array([1, 0, 1, 0, 1], np.uint8), probe=True)
+
+
+def test_exclusive_counts_small_edges(gpu_ctx):
+    # one genome: the probe needs two (the partition packs genome ids beside the hash), so the sort path answers
+    one = synth.from_sketches([np.array([1, 2, 3, 3, 9], np.uint64)])
+    _check_counts(gpu_ctx, one, np.array([3, 9, 9, 11], dtype=np.uint64), probe=False)
+    _check_counts(gpu_ctx, one, np.array([3], dtype=np.uint64), mask=np.zeros(1, np.uint8), probe=False)
+    # every sketch empty (T = 0): no hash to hold, the mask alone decides what is nontrivial
+    empty = synth.from_sketches([np.zeros(0, np.uint64)] * 3)
+    _check_counts(gpu_ctx, empty, np.array([1, 2], dtype=np.uint64), probe=False)
+    _check_counts(gpu_ctx, empty, np.array([1, 2], dtype=np.uint64), mask=np.ones(3, np.uint8), probe=False)
+    # a 10-bit reference (largest hash 1000): 1010 and 1023 are above the largest hash but inside the hash width, 1024 and
+    # 2^63 beyond it; the sample is shuffled and repeats hashes
+    narrow = synth.from_sketches([np.array([1, 5, 900, 1000], np.uint64), np.array([5, 7, 7, 1000], np.uint64), np.zeros(0, np.uint64),
+                                  np.array([3, 900, 950], np.uint64)])
+    for sample in ([1010, 1023, 1024, 2**63, 5000], [7, 1010, 5, 7, 1024, 5, 3, 1023], [1000, 1000, 2**64 - 1]):
+        _check_counts(gpu_ctx, narrow, np.array(sample, dtype=np.uint64), probe=True)
+    _check_counts(gpu_ctx, narrow, np.array([1023, 1], dtype=np.uint64), mask=np.array([0, 1, 1, 1], np.uint8), probe=True)

@@ -1642,6 +1642,7 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
     };
     if (partition_only) {
         ctx->tm.ms_sort += elapsed(ctx, 0, 1);
+        record_phases();            // the run path's own partition reports its phases (and a retry) like the index build's
         *used = 1;
         return 0;
     }
