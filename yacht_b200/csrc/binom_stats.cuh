@@ -13,7 +13,8 @@
 //   * cdf as a one-sided sum of pmf ratios started at the boundary term and running AWAY from the
 //     mode (every ratio < 1, geometric convergence, no cancellation); the side that is < 1/2 is
 //     summed, the other is its complement -- the same choice an incomplete-beta evaluation makes;
-//   * ppf as "the smallest k with cdf(k) >= q" (SURVEY.md appendix B: equals scipy's binom.ppf);
+//   * ppf as "the smallest k with cdf(k) >= q" (SURVEY.md appendix B: equals scipy's binom.ppf),
+//     exact ties cdf(k) == q settled as >= (see cdf_ge_tie);
 //   * betaincinv(n-k, k+1, y) through the identity I_x(n-k, k+1) = P[Bin(n, 1-x) <= k], solved
 //     for w = 1-x by safeguarded Newton iterations on the log of the small tail.
 // Target: integers exact, floats within 1e-9 relative of scipy (tests/test_run_parity_gpu.py).
@@ -158,6 +159,50 @@ YS_HD double norm_ppf_guess(double p) {
            (((((b[0] * r + b[1]) * r + b[2]) * r + b[3]) * r + b[4]) * r + 1.0);
 }
 
+// ---- exact ties cdf(k) == q --------------------------------------------------------------------
+// cdf(k) can equal a double q exactly only when p has few significant bits (p = a / 2^m, so the cdf is a
+// dyadic rational) and n is small -- or, for p = 1/2 and any odd n, at k = (n - 1) / 2 where it is 1/2 by
+// symmetry.  The fp64 cdf above is good to ~1e-15 relative and rounds such a tie to either side, so
+// binom_ppf re-decides the comparison that fixed its answer with the sum below, in double-double.
+struct DD { double hi, lo; };
+YS_HD DD dd_two_sum(double a, double b) { const double s = a + b, bb = s - a; return {s, (a - (s - bb)) + (b - bb)}; }
+YS_HD DD dd_add(DD a, DD b) { DD s = dd_two_sum(a.hi, b.hi); s.lo += a.lo + b.lo; return dd_two_sum(s.hi, s.lo); }
+YS_HD DD dd_mul(DD a, double b) { const double h = a.hi * b; return dd_two_sum(h, fma(a.hi, b, -h) + a.lo * b); }
+YS_HD DD dd_div(DD a, double b) {
+    const double q1 = a.hi / b, h = q1 * b;
+    const double r = ((a.hi - h) - fma(q1, b, -h)) + a.lo;   // a - q1 b, exactly up to a.lo's rounding
+    return dd_two_sum(q1, r / b);
+}
+
+constexpr double TIE_NMAX = 4096.0;
+
+// whether cdf(k; n, p) == q is possible for a double q: p a multiple of 2^-32, and n small (or p = 1/2)
+YS_HD bool tie_possible(double n, double p) {
+    const double s = p * 4294967296.0;
+    return s == floor(s) && (n <= TIE_NMAX || p == 0.5);
+}
+
+// P[Bin(n, p) <= k] >= q, settled to ~1e-27 and counting a cdf within that of q as equal (ties -> true).
+// For tie_possible(n, p) with n <= TIE_NMAX only: (n - i + 1) p and i (1 - p) are then exact doubles.
+YS_HD bool cdf_ge_tie(double k, double n, double p, double q) {
+    // t_i = C(n, i) (p/q)^i relative to t_0; S = sum_{i<=k} t_i, T = sum_{i<=n} t_i, both rescaled by 2^-600
+    // together whenever a term grows past 2^600 (a power of two: exact)
+    const double pq = 1.0 - p;
+    DD t = {1.0, 0.0}, S = {1.0, 0.0}, T = {1.0, 0.0};
+    for (double i = 1.0; i <= n; i += 1.0) {
+        t = dd_div(dd_mul(t, (n - i + 1.0) * p), i * pq);
+        T = dd_add(T, t);
+        if (i <= k) S = T;
+        if (t.hi > 0x1p600) {
+            const double sc = 0x1p-600;
+            t = {t.hi * sc, t.lo * sc}; S = {S.hi * sc, S.lo * sc}; T = {T.hi * sc, T.lo * sc};
+        }
+    }
+    const DD qT = dd_mul(T, -q);
+    const DD d = dd_add(S, qT);                               // S - q T: cdf >= q  <=>  d >= 0
+    return d.hi + d.lo >= -1e-27 * T.hi;
+}
+
 // smallest integer k in [0, n] with P[Bin(n,p) <= k] >= q   (== scipy.stats.binom.ppf(q, n, p))
 YS_HD double binom_ppf(double q, double n, double p) {
     if (isnan(q) || isnan(p) || q < 0.0 || q > 1.0 || p < 0.0 || p > 1.0) return NAN;
@@ -186,6 +231,16 @@ YS_HD double binom_ppf(double q, double n, double p) {
     while (hi - lo > 1.0) {
         const double mid = floor(0.5 * (lo + hi));
         if (binom_cdf(mid, n, p) >= q) hi = mid; else lo = mid;
+    }
+    // cdf(lo) < q decided the answer; if that cdf may be an exact tie within fp64's reach of q, settle it
+    if (lo >= 0.0 && tie_possible(n, p)) {
+        if (n > TIE_NMAX) {
+            if (2.0 * lo + 1.0 == n && 0.5 >= q) hi = lo;   // p = 1/2: only cdf((n-1)/2) = 1/2 can tie
+        } else {
+            const double c = binom_cdf(lo, n, p);
+            const double tol = 4.0 * 0x1p-53 * fmax(q, 1.0 - q) + 1e-13 * fmin(q, 1.0 - q);
+            if (q - c <= tol && cdf_ge_tie(lo, n, p, q)) hi = lo;
+        }
     }
     return hi;
 }
