@@ -155,7 +155,8 @@ int ygpu_elapsed_ms(ygpu_ctx* ctx, int slot_a, int slot_b, double* ms);
  * "run_path" = 0 forces the general sort-based run path (default 1: probe the partitioned reference);
  * "count_thresholds" = 0 evaluates the containment expression per pair in fp64 inside the count kernel (default 1: the
  * smallest passing count per genome is found with that expression once, the kernel compares integers);
- * "sketch_kernel" = 2 forces the byte-wise sketching kernel for every k-mer size (default 0: k <= 64 uses packed words).  */
+ * "sketch_kernel" = 2 forces the byte-wise sketching kernel for every k-mer size (default 0: k <= 64 uses packed words);
+ * "stream_chunk_bytes" = raw bytes per device chunk of ygpu_stream_* (default 64 MiB, at most 1 GiB).                */
 int ygpu_set_option(ygpu_ctx* ctx, const char* name, int64_t value);
 
 /* ---- ingest (host side of the path) ------------------------------------------------------------ */
@@ -291,6 +292,43 @@ typedef struct {
 int ygpu_sketch_sequences(ygpu_ctx* ctx, const uint8_t* bases, uint64_t n_bases, const uint64_t* sketch_offsets,
                           uint32_t n_sketches, int ksize, uint64_t max_hash, uint32_t seed, ygpu_sketch_result* out);
 void ygpu_sketch_result_free(ygpu_sketch_result* r);
+
+/* Streamed sketching of FASTA / FASTQ text of any size.  The raw (decompressed) text goes to the device in chunks of
+ * "stream_chunk_bytes" (ygpu_set_option; default 64 MiB); the device parses it, hashes it with the kernels of
+ * ygpu_sketch_sequences and adds the result to a sketch kept on the device.  Host memory stays at a few chunks plus
+ * the output.  The parse follows the records of a whole-file read exactly: '\r' is dropped everywhere, leading
+ * whitespace of a file is skipped and the next byte chooses FASTA ('>') or FASTQ ('@'); a FASTA record's inner line
+ * ends vanish; a FASTQ record is four lines, '@' name, sequence, '+', quality.
+ *   ygpu_stream_begin(ctx, ksize, max_hash, seed, mode)   mode YGPU_STREAM_WHOLE: one sketch of everything fed;
+ *                                                         YGPU_STREAM_PER_RECORD: one sketch per record, with names
+ *   ygpu_stream_feed(ctx, bytes, n)      the next bytes of the current file, split anywhere.  HOST pointer, free to
+ *                                        reuse when the call returns (page-locked memory from ygpu_host_alloc copies
+ *                                        fastest); reading the next piece on another thread overlaps the device work
+ *   ygpu_stream_end_file(ctx)            end of the current file and its checks; the next feed starts a new file
+ *   ygpu_stream_finish(ctx, &result, &stats, &names, &name_offsets, &n_names)
+ * Malformed input fails with YGPU_ERR_ARG and one of "neither FASTA ('>') nor FASTQ ('@')", "malformed FASTQ record at
+ * line N", "FASTQ with N lines (not a multiple of 4)" (lines counted from the first byte after the leading whitespace);
+ * the stream must then be begun again.  Names (the header line without its first byte and without '\r') are kept for
+ * every record in per-record mode and for FASTA records in whole mode; names[name_offsets[i] .. name_offsets[i + 1])
+ * is name i; both arrays are library-owned, release them with ygpu_free (NULL when there are none).               */
+#define YGPU_STREAM_WHOLE 0
+#define YGPU_STREAM_PER_RECORD 1
+typedef struct {
+    uint64_t n_bytes;       /* bytes fed, leading whitespace of the files excluded                  */
+    uint64_t n_bases;       /* bytes handed to the hashing kernels (sequence + one separator per record + carried bases) */
+    uint64_t n_records;
+    uint64_t n_kmers;       /* valid windows hashed                                                 */
+    uint64_t n_chunks;      /* device chunks parsed                                                 */
+    double ms_h2d;          /* host -> device copies of the raw text                                */
+    double ms_parse;        /* line scan, classification, compaction                                */
+    double ms_hash;         /* the K7 hashing kernel                                                */
+    double ms_merge;        /* sort + reduce of each chunk's kept hashes into the resident sketch   */
+} ygpu_stream_stats;
+int ygpu_stream_begin(ygpu_ctx* ctx, int ksize, uint64_t max_hash, uint32_t seed, int mode);
+int ygpu_stream_feed(ygpu_ctx* ctx, const uint8_t* bytes, uint64_t n);
+int ygpu_stream_end_file(ygpu_ctx* ctx);
+int ygpu_stream_finish(ygpu_ctx* ctx, ygpu_sketch_result* out, ygpu_stream_stats* stats /* may be NULL */,
+                       char** names, uint64_t** name_offsets, uint64_t* n_names);
 
 #ifdef __cplusplus
 }

@@ -25,7 +25,9 @@ ABI_SYMBOLS = [
     "ygpu_comm_get_unique_id", "ygpu_comm_init", "ygpu_comm_destroy", "ygpu_load_sketches_sharded", "ygpu_load_sketches_sharded_device",
     "ygpu_train_step_sharded", "ygpu_upload_finish_sharded", "ygpu_load_sketches_hashrange", "ygpu_load_sketches_hashrange_device",
     "ygpu_train_step_replicated", "ygpu_sketch_sequences", "ygpu_sketch_result_free",
+    "ygpu_stream_begin", "ygpu_stream_feed", "ygpu_stream_end_file", "ygpu_stream_finish",
 ]
+STREAM_WHOLE, STREAM_PER_RECORD = 0, 1
 COMM_ID_BYTES = 128
 
 
@@ -61,6 +63,15 @@ class SketchResult(ctypes.Structure):
     _fields_ = [("hashes", ctypes.POINTER(ctypes.c_uint64)), ("abundances", ctypes.POINTER(ctypes.c_uint32)),
                 ("offsets", ctypes.POINTER(ctypes.c_uint64)), ("n_sketches", ctypes.c_uint32), ("_pad", ctypes.c_uint32),
                 ("n_kmers", ctypes.c_uint64)]
+
+
+class StreamStats(ctypes.Structure):
+    _fields_ = [("n_bytes", ctypes.c_uint64), ("n_bases", ctypes.c_uint64), ("n_records", ctypes.c_uint64),
+                ("n_kmers", ctypes.c_uint64), ("n_chunks", ctypes.c_uint64), ("ms_h2d", ctypes.c_double),
+                ("ms_parse", ctypes.c_double), ("ms_hash", ctypes.c_double), ("ms_merge", ctypes.c_double)]
+
+    def as_dict(self) -> dict:
+        return {k: (float(getattr(self, k)) if t is ctypes.c_double else int(getattr(self, k))) for k, t in self._fields_}
 
 
 class SketchSet(ctypes.Structure):
@@ -143,6 +154,11 @@ def load_library() -> ctypes.CDLL:
     lib.ygpu_sketch_sequences.argtypes = [vp, vp, u64, vp, u32, ctypes.c_int, u64, u32, ctypes.POINTER(SketchResult)]
     lib.ygpu_sketch_result_free.argtypes = [ctypes.POINTER(SketchResult)]
     lib.ygpu_sketch_result_free.restype = None
+    lib.ygpu_stream_begin.argtypes = [vp, ctypes.c_int, u64, u32, ctypes.c_int]
+    lib.ygpu_stream_feed.argtypes = [vp, vp, u64]
+    lib.ygpu_stream_end_file.argtypes = [vp]
+    lib.ygpu_stream_finish.argtypes = [vp, ctypes.POINTER(SketchResult), ctypes.POINTER(StreamStats), ctypes.POINTER(vp),
+                                       ctypes.POINTER(vp), ctypes.POINTER(u64)]
     for name in ABI_SYMBOLS:
         getattr(lib, name)  # AttributeError here means the .so does not match include/yacht_gpu.h
     _lib = lib
@@ -352,6 +368,62 @@ class GpuContext:
             return hashes, abund, offsets, int(res.n_kmers)
         finally:
             self.lib.ygpu_sketch_result_free(ctypes.byref(res))
+
+    # -- streamed sketching (ygpu_stream_*) ------------------------------------------------------
+    def _stream_error(self, rc: int, what: str, path: Optional[str]) -> None:
+        if rc == 0:
+            return
+        msg = self.lib.ygpu_last_error(self.h)
+        text = msg.decode(errors="replace") if msg else ""
+        if rc == -3 and path is not None:           # YGPU_ERR_ARG: the input is not a FASTA / FASTQ file the reader accepts
+            raise ValueError(f"{path}: {text}")
+        raise YgpuError(f"{what} failed ({rc}): {text}")
+
+    def host_buffer(self, nbytes: int):
+        """A page-locked host buffer (ygpu_host_alloc) -> (writable memoryview, address, release function)."""
+        ptr = self.lib.ygpu_host_alloc(int(nbytes))
+        if not ptr:
+            raise YgpuError(f"ygpu_host_alloc({nbytes}) failed")
+        mv = memoryview((ctypes.c_uint8 * int(nbytes)).from_address(ptr)).cast("B")
+        return mv, int(ptr), lambda: self.lib.ygpu_host_free(ctypes.c_void_p(ptr))
+
+    def stream_begin(self, ksize: int, max_hash: int, seed: int = 42, per_record: bool = False) -> None:
+        self._check(self.lib.ygpu_stream_begin(self.h, int(ksize), int(max_hash), int(seed),
+                                               STREAM_PER_RECORD if per_record else STREAM_WHOLE), "ygpu_stream_begin")
+
+    def stream_feed(self, ptr: int, n: int, path: Optional[str] = None) -> None:
+        """The next n bytes of the current file at host address ptr (free to reuse when this returns)."""
+        self._stream_error(self.lib.ygpu_stream_feed(self.h, ctypes.c_void_p(ptr), int(n)), "ygpu_stream_feed", path)
+
+    def stream_end_file(self, path: Optional[str] = None) -> None:
+        self._stream_error(self.lib.ygpu_stream_end_file(self.h), "ygpu_stream_end_file", path)
+
+    def stream_finish(self, path: Optional[str] = None):
+        """-> (hashes, abundances, offsets, names or None, stats dict); names are bytes, one per record that kept its name."""
+        res, st = SketchResult(), StreamStats()
+        names, name_off, n_names = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
+        self._stream_error(self.lib.ygpu_stream_finish(self.h, ctypes.byref(res), ctypes.byref(st), ctypes.byref(names),
+                                                       ctypes.byref(name_off), ctypes.byref(n_names)), "ygpu_stream_finish", path)
+        try:
+            ns = int(res.n_sketches)
+            offsets = np.ctypeslib.as_array(res.offsets, shape=(ns + 1,)).copy()
+            total = int(offsets[-1])
+            if total:
+                hashes = np.ctypeslib.as_array(res.hashes, shape=(total,)).copy()
+                abund = np.ctypeslib.as_array(res.abundances, shape=(total,)).copy()
+            else:
+                hashes, abund = np.zeros(0, np.uint64), np.zeros(0, np.uint32)
+            out_names = None
+            nn = int(n_names.value)
+            if nn:
+                off = np.ctypeslib.as_array(ctypes.cast(name_off, ctypes.POINTER(ctypes.c_uint64)), shape=(nn + 1,)).copy()
+                blob = ctypes.string_at(names, int(off[-1])) if int(off[-1]) else b""
+                out_names = [blob[int(off[i]):int(off[i + 1])] for i in range(nn)]
+            return hashes, abund, offsets, out_names, st.as_dict()
+        finally:
+            self.lib.ygpu_sketch_result_free(ctypes.byref(res))
+            self.lib.ygpu_free(names)
+            self.lib.ygpu_free(name_off)
 
     # -- run path -----------------------------------------------------------------------------
     def exclusive_hashes(self, sample: np.ndarray, mask: Optional[np.ndarray] = None) -> np.ndarray:

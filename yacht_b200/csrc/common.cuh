@@ -134,6 +134,8 @@ struct ygpu_ctx {
     void* upload = nullptr;         // streaming ingest state (yacht_gpu.cu: ygpu_upload_*)
     void* sketch_scratch = nullptr; // sketching buffers (sketch.cu)
     int sketch_kernel = 0;          // 0 = by k-mer size (packed words up to k = 64), 2 = always the byte-wise kernel (test hook)
+    void* seq_stream = nullptr;     // streamed FASTA / FASTQ sketching (seq_stream.cu)
+    uint64_t stream_chunk_bytes = 64ull << 20;   // raw bytes the stream parses per device chunk
 
     ygpu_timings tm = {};
 };
@@ -233,4 +235,11 @@ void ygpu_part_release(ygpu_ctx* ctx);
 void ygpu_run_release(ygpu_ctx* ctx);
 // sketching (sketch.cu)
 void ygpu_sketch_release(ygpu_ctx* ctx);
+void ygpu_stream_release(ygpu_ctx* ctx);
+// K7 on a device buffer (d_bases zero-padded by YG_SKETCH_PAD bytes behind n_bases); survivors stay in the sketch scratch
+constexpr uint64_t YG_SKETCH_PAD = 4096 + 256 + 16;
+constexpr uint64_t YG_STREAM_CHUNK_MAX = 1ull << 30;
+int ygpu_sketch_hash_device(ygpu_ctx* ctx, const uint8_t* d_bases, uint64_t n_bases, const uint64_t* d_off, uint32_t n_sketches,
+                            int ksize, uint64_t max_hash, uint32_t seed, cudaEvent_t ev_done, uint64_t* m, uint64_t* n_kmers);
+void ygpu_sketch_survivors(ygpu_ctx* ctx, uint64_t** d_key, uint32_t** d_sid);
 void ygpu_upload_release(ygpu_ctx* ctx);

@@ -31,6 +31,7 @@ constexpr int SK_TILE = SK_NT * SK_PER;         // 4096
 constexpr int SK_KMAX = 256;                    // largest supported k-mer size
 static_assert(SK_PER == 16 && SK_NT == 256, "the packed kernel's span layout (sketch_hash.cuh) assumes 16 windows per thread");
 constexpr int SK_PAD = SK_TILE + SK_KMAX + 16;  // zero bytes behind the bases: the last tile is loaded without bounds checks
+static_assert(SK_PAD == YG_SKETCH_PAD, "the stream pads its hashing buffer by YG_SKETCH_PAD");
 
 struct SketchScratch {
     uint8_t* d_bases = nullptr;
@@ -225,6 +226,56 @@ __global__ void __launch_bounds__(SK_NT) k_sketch_hash_packed2(const uint8_t* __
     if ((tid & 31) == 0 && valid_kmers) atomicAdd(&cnt[1], valid_kmers);
 }
 
+}  // namespace
+
+// K7 on a device buffer: d_bases[0, n_bases) followed by SK_PAD zero bytes (16-byte aligned), d_off[0 .. n_sketches] on the
+// device.  Leaves the m survivors in the context's scratch (sketch_survivors) and the valid windows in *n_kmers; records
+// ev_done behind the hashing kernel.  ygpu_sketch_sequences and the stream (seq_stream.cu) both hash through here.
+int ygpu_sketch_hash_device(ygpu_ctx* ctx, const uint8_t* d_bases, uint64_t n_bases, const uint64_t* d_off, uint32_t n_sketches,
+                            int ksize, uint64_t max_hash, uint32_t seed, cudaEvent_t ev_done, uint64_t* m, uint64_t* n_kmers) {
+    SketchScratch* S = sk_scratch(ctx);
+    cudaStream_t st = ctx->stream;
+    YG_CHECK(dev_alloc(ctx, &S->d_cnt, 2));
+    // Expected survivors: windows x (max_hash + 1) / 2^64.  Twice that plus slack; a second pass with the exact count
+    // follows in the (never observed) case that it does not suffice.
+    const double frac = ((double)max_hash + 1.0) / 18446744073709551616.0;
+    uint64_t cap = (uint64_t)std::min<double>((double)n_bases, (double)n_bases * frac * 2.0 + 65536.0);
+    unsigned long long h_cnt[2] = {0, 0};
+    const uint64_t n_tiles = (n_bases + SK_TILE - 1) / SK_TILE;
+    const int grid = (int)std::min<uint64_t>(n_tiles, (uint64_t)ctx->num_sms * 8);
+    for (int attempt = 0; attempt < 2; attempt++) {
+        if (cap >= (1ull << 31)) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: more than 2^31 kept hashes in one call; split the batch");
+        YG_CHECK(dev_alloc(ctx, &S->d_key, cap));
+        YG_CHECK(dev_alloc(ctx, &S->d_sid, cap));
+        YG_CUDA(ctx, cudaMemsetAsync(S->d_cnt, 0, 2 * sizeof(unsigned long long), st));
+        if (ksize <= 32 && ctx->sketch_kernel != 2)
+            k_sketch_hash_packed<<<grid, SK_NT, 0, st>>>(d_bases, n_bases, d_off, n_sketches, ksize, seed, max_hash, S->d_key, S->d_sid, cap, S->d_cnt);
+        else if (ksize <= 64 && ctx->sketch_kernel != 2)
+            k_sketch_hash_packed2<<<grid, SK_NT, 0, st>>>(d_bases, n_bases, d_off, n_sketches, ksize, seed, max_hash, S->d_key, S->d_sid, cap, S->d_cnt);
+        else
+            k_sketch_hash<<<grid, SK_NT, 0, st>>>(d_bases, n_bases, d_off, n_sketches, ksize, seed, max_hash, S->d_key, S->d_sid, cap, S->d_cnt);
+        YG_CUDA(ctx, cudaGetLastError());
+        ctx->tm.n_kernel_launches++;
+        YG_CUDA(ctx, cudaEventRecord(ev_done, st));
+        YG_CUDA(ctx, cudaMemcpyAsync(h_cnt, S->d_cnt, sizeof h_cnt, cudaMemcpyDeviceToHost, st));
+        YG_CUDA(ctx, cudaStreamSynchronize(st));
+        if (h_cnt[0] <= cap) break;
+        if (attempt == 1) return ygpu_fail(ctx, YGPU_ERR_STATE, "ygpu_sketch_sequences: survivor count changed between passes");
+        cap = h_cnt[0];
+    }
+    *m = h_cnt[0];
+    *n_kmers = h_cnt[1];
+    return 0;
+}
+
+void ygpu_sketch_survivors(ygpu_ctx* ctx, uint64_t** d_key, uint32_t** d_sid) {
+    SketchScratch* S = sk_scratch(ctx);
+    *d_key = S->d_key;
+    *d_sid = S->d_sid;
+}
+
+namespace {
+
 __global__ void __launch_bounds__(256) k_sketch_heads(const uint64_t* __restrict__ key, const uint32_t* __restrict__ sid, uint64_t m,
                                                        uint32_t* __restrict__ flag) {
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (uint64_t)gridDim.x * blockDim.x)
@@ -287,37 +338,11 @@ extern "C" int ygpu_sketch_sequences(ygpu_ctx* ctx, const uint8_t* bases, uint64
     YG_CUDA(ctx, cudaMemcpyAsync(S->d_off, sketch_offsets, ((size_t)n_sketches + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
     YG_CUDA(ctx, cudaEventRecord(ctx->ev[1], st));
 
-    // Expected survivors: windows x (max_hash + 1) / 2^64.  Twice that plus slack; a second pass with the exact count
-    // follows in the (never observed) case that it does not suffice.
-    const double frac = ((double)max_hash + 1.0) / 18446744073709551616.0;
-    uint64_t cap = (uint64_t)std::min<double>((double)n_bases, (double)n_bases * frac * 2.0 + 65536.0);
-    unsigned long long h_cnt[2] = {0, 0};
-    const uint64_t n_tiles = (n_bases + SK_TILE - 1) / SK_TILE;
-    const int grid = (int)std::min<uint64_t>(n_tiles, (uint64_t)ctx->num_sms * 8);
-    for (int attempt = 0; attempt < 2; attempt++) {
-        if (cap >= (1ull << 31)) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: more than 2^31 kept hashes in one call; split the batch");
-        YG_CHECK(dev_alloc(ctx, &S->d_key, cap));
-        YG_CHECK(dev_alloc(ctx, &S->d_sid, cap));
-        YG_CUDA(ctx, cudaMemsetAsync(S->d_cnt, 0, 2 * sizeof(unsigned long long), st));
-        if (ksize <= 32 && ctx->sketch_kernel != 2)
-            k_sketch_hash_packed<<<grid, SK_NT, 0, st>>>(S->d_bases, n_bases, S->d_off, n_sketches, ksize, seed, max_hash, S->d_key, S->d_sid, cap, S->d_cnt);
-        else if (ksize <= 64 && ctx->sketch_kernel != 2)
-            k_sketch_hash_packed2<<<grid, SK_NT, 0, st>>>(S->d_bases, n_bases, S->d_off, n_sketches, ksize, seed, max_hash, S->d_key, S->d_sid, cap, S->d_cnt);
-        else
-            k_sketch_hash<<<grid, SK_NT, 0, st>>>(S->d_bases, n_bases, S->d_off, n_sketches, ksize, seed, max_hash, S->d_key, S->d_sid, cap, S->d_cnt);
-        YG_CUDA(ctx, cudaGetLastError());
-        ctx->tm.n_kernel_launches++;
-        YG_CUDA(ctx, cudaEventRecord(ctx->ev[2], st));
-        YG_CUDA(ctx, cudaMemcpyAsync(h_cnt, S->d_cnt, sizeof h_cnt, cudaMemcpyDeviceToHost, st));
-        YG_CUDA(ctx, cudaStreamSynchronize(st));
-        if (h_cnt[0] <= cap) break;
-        if (attempt == 1) return ygpu_fail(ctx, YGPU_ERR_STATE, "ygpu_sketch_sequences: survivor count changed between passes");
-        cap = h_cnt[0];
-    }
+    uint64_t m = 0, n_kmers = 0;
+    YG_CHECK(ygpu_sketch_hash_device(ctx, S->d_bases, n_bases, S->d_off, n_sketches, ksize, max_hash, seed, ctx->ev[2], &m, &n_kmers));
     ctx->tm.ms_h2d = elapsed(ctx, 0, 1);
     ctx->tm.ms_sketch = elapsed(ctx, 1, 2);
-    out->n_kmers = h_cnt[1];
-    const uint64_t m = h_cnt[0];
+    out->n_kmers = n_kmers;
     if (m == 0) return 0;
 
     // order by (sketch id, hash): LSD radix sort by hash, then -- stable -- by sketch id

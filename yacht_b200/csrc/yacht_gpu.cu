@@ -143,6 +143,7 @@ extern "C" void ygpu_ctx_destroy(ygpu_ctx* ctx) {
     ygpu_run_release(ctx);
     ygpu_part_release(ctx);
     ygpu_sketch_release(ctx);
+    ygpu_stream_release(ctx);
     ygpu_upload_release(ctx);
     ygpu_comm_destroy(ctx);
     if (ctx->d_pairs_local) cudaFree(ctx->d_pairs_local);
@@ -1407,6 +1408,11 @@ extern "C" int ygpu_set_option(ygpu_ctx* ctx, const char* name, int64_t value) {
     if (!strcmp(name, "group_kernel")) { ctx->group_kernel = (int)value; return 0; }
     if (!strcmp(name, "run_path")) { ctx->run_path = (int)value; return 0; }
     if (!strcmp(name, "sketch_kernel")) { ctx->sketch_kernel = (int)value; return 0; }
+    if (!strcmp(name, "stream_chunk_bytes")) {
+        if (value < 1 || value > (int64_t)YG_STREAM_CHUNK_MAX) return ygpu_fail(ctx, YGPU_ERR_ARG, "stream_chunk_bytes must lie in [1, %llu]", (unsigned long long)YG_STREAM_CHUNK_MAX);
+        ctx->stream_chunk_bytes = (uint64_t)value;
+        return 0;
+    }
     if (!strcmp(name, "group_ctas")) { ctx->group_ctas = (int)value; return 0; }
     if (!strcmp(name, "count_thresholds")) { ctx->count_thresholds = (int)value; return 0; }
     return ygpu_fail(ctx, YGPU_ERR_ARG, "unknown option %s", name);

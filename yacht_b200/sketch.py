@@ -9,6 +9,8 @@ from __future__ import annotations
 
 import gzip
 import os
+import queue
+import threading
 from typing import Iterable, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -18,6 +20,9 @@ from . import _lib, sigio
 SEED = 42                       # "seed": 42 in every sourmash DNA signature
 BATCH_BASES = 1 << 31           # bases per device call (2 GiB of sequence + separators)
 CHUNK_FILE_BYTES = 1 << 29      # on-disk bytes of sequence files read ahead of the device (gzip expands ~3.5x)
+STREAM_FILE_BYTES = 1 << 30     # a file larger than this on disk is streamed: its text is parsed on the device chunk by chunk
+STREAM_READ_BYTES = 64 << 20    # bytes per read into one page-locked buffer (one device chunk at the library's default)
+STREAM_BUFFERS = 3              # page-locked read buffers: the reader fills one while the device works on another
 _ctx = None
 
 
@@ -75,6 +80,86 @@ def read_records(path: str) -> List[Tuple[str, bytes]]:
     else:
         raise ValueError(f"{path}: neither FASTA ('>') nor FASTQ ('@')")
     return records
+
+
+def is_streamed(path: str) -> bool:
+    """Whether `path` takes the streamed route (decided by its size on disk only)."""
+    return os.path.getsize(path) > STREAM_FILE_BYTES
+
+
+def _open_text(path: str):
+    """The file's decompressed bytes as a stream: gzip (every member) when it starts with the gzip magic, else plain."""
+    f = open(path, "rb")
+    if f.read(2) == b"\x1f\x8b":
+        f.seek(0)
+        return gzip.GzipFile(fileobj=f, mode="rb"), f
+    f.seek(0)
+    return f, f
+
+
+def _reader(path: str, bufs, free: "queue.Queue", full: "queue.Queue") -> None:
+    """Reader thread: fills free buffers with the file's next bytes, hands them over as (index, n); (None, 0) at the end,
+    (None, exception) on a read error.  A None taken from `free` asks it to stop."""
+    try:
+        text, raw = _open_text(path)
+        try:
+            while True:
+                i = free.get()
+                if i is None:
+                    return
+                n = text.readinto(bufs[i][0])
+                if not n:
+                    full.put((None, 0))
+                    return
+                full.put((i, n))
+        finally:
+            text.close()
+            raw.close()
+    except BaseException as e:          # handed to the feeding thread, which raises it
+        full.put((None, e))
+
+
+def sketch_stream(paths: Sequence[str], ksize: int, scaled: int, per_record: bool = False, seed: int = SEED,
+                  stats: Optional[dict] = None):
+    """Sketch the files one after another through the device stream (ygpu_stream_*): the text is read and gunzipped on a
+    reader thread into STREAM_BUFFERS page-locked buffers and parsed, hashed and accumulated on the device, so host memory
+    stays at a few buffers plus the sketch whatever the size of the input.
+    Returns ([(mins, abundances)], names): one sketch of all records, or with `per_record` one per record with its name.
+    `stats`, when given, receives the stream's counters and device times (ygpu_stream_stats)."""
+    ctx = _context()
+    ctx.stream_begin(ksize, max_hash_for_scaled(scaled), seed, per_record)
+    bufs = [ctx.host_buffer(STREAM_READ_BYTES) for _ in range(STREAM_BUFFERS)]
+    try:
+        for path in paths:
+            free: queue.Queue = queue.Queue()
+            full: queue.Queue = queue.Queue()
+            for i in range(len(bufs)):
+                free.put(i)
+            th = threading.Thread(target=_reader, args=(path, bufs, free, full), daemon=True)
+            th.start()
+            try:
+                while True:
+                    i, n = full.get()
+                    if i is None:
+                        if isinstance(n, BaseException):
+                            raise n
+                        break
+                    ctx.stream_feed(bufs[i][1], n, path)
+                    free.put(i)
+            finally:
+                free.put(None)
+                th.join()
+            ctx.stream_end_file(path)
+        hashes, abund, offsets, names, st = ctx.stream_finish(paths[-1] if paths else None)
+        if stats is not None:
+            stats.update(st)
+    finally:
+        for _, _, release in bufs:
+            release()
+    # names come back as bytes; decoding them raises on invalid UTF-8 as the record path's reader does
+    names = [b.decode() for b in names] if names else []
+    sketches = [(hashes[int(offsets[s]):int(offsets[s + 1])], abund[int(offsets[s]):int(offsets[s + 1])]) for s in range(len(offsets) - 1)]
+    return sketches, names
 
 
 def sketch_record_groups(groups: Sequence[Sequence[bytes]], ksize: int, scaled: int, seed: int = SEED):
@@ -144,8 +229,18 @@ def sketch_files(paths: Sequence[str], ksize: int, scaled: int, singleton: bool 
     out: List[dict] = []
     i = 0
     while i < len(paths):
+        if is_streamed(paths[i]):       # a large file: parsed on the device, never held in host memory
+            sketches, rec_names = sketch_stream([paths[i]], ksize, scaled, per_record=singleton)
+            if singleton:
+                out.extend({"name": name, "filename": paths[i], "mins": mins, "abundances": ab}
+                           for name, (mins, ab) in zip(rec_names, sketches))
+            else:
+                [(mins, ab)] = sketches
+                out.append({"name": names[i] if names is not None else "", "filename": paths[i], "mins": mins, "abundances": ab})
+            i += 1
+            continue
         j, size = i, 0
-        while j < len(paths) and (j == i or size + os.path.getsize(paths[j]) <= CHUNK_FILE_BYTES):
+        while j < len(paths) and (j == i or (size + os.path.getsize(paths[j]) <= CHUNK_FILE_BYTES and not is_streamed(paths[j]))):
             size += os.path.getsize(paths[j])
             j += 1
         chunk = list(paths[i:j])

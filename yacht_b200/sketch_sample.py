@@ -16,9 +16,14 @@ def add_arguments(parser):
 
 
 def sketch_reads(infiles, kmer, scaled, outfile):
-    """All records of `infiles` -> one sketch (name empty, filename = the first file, like `sourmash sketch dna`)."""
-    reads = [seq for path in infiles for _, seq in sketch.read_records(path)]
-    [(mins, abundances)] = sketch.sketch_record_groups([reads], kmer, scaled)
+    """All records of `infiles` -> one sketch (name empty, filename = the first file, like `sourmash sketch dna`).
+    When one of the files is larger than sketch.STREAM_FILE_BYTES, all of them are streamed through the device parser,
+    file after file, into the one sketch; otherwise the records are read whole and batched."""
+    if any(sketch.is_streamed(path) for path in infiles):
+        [(mins, abundances)], _ = sketch.sketch_stream(list(infiles), kmer, scaled)
+    else:
+        reads = [seq for path in infiles for _, seq in sketch.read_records(path)]
+        [(mins, abundances)] = sketch.sketch_record_groups([reads], kmer, scaled)
     sketch.write_sketches(outfile, [dict(name="", filename=infiles[0], mins=mins, abundances=abundances)], kmer, scaled)
 
 
