@@ -158,6 +158,11 @@ int ygpu_elapsed_ms(ygpu_ctx* ctx, int slot_a, int slot_b, double* ms);
  * "sketch_kernel" = 2 forces the byte-wise sketching kernel for every k-mer size (default 0: k <= 64 uses packed words);
  * "stream_chunk_bytes" = raw bytes per device chunk of ygpu_stream_* (default 64 MiB, at most 1 GiB).                */
 int ygpu_set_option(ygpu_ctx* ctx, const char* name, int64_t value);
+/* Read-only state of the last count call (ygpu_pairwise_flag / _device): "last_count_kernel" (1 = dense row accumulator,
+ * 2 = warp per row), "last_count_overflow_rows" (rows the warp kernel deferred to the dense kernel), and the dense kernel's
+ * accumulator geometry "last_count_tile_w" (columns per tile), "last_count_n_tiles" and "last_count_u16" (1 = packed 16-bit
+ * counters).  An unknown name fails with YGPU_ERR_ARG.                                                                    */
+int ygpu_get_option(ygpu_ctx* ctx, const char* name, int64_t* out);
 
 /* ---- ingest (host side of the path) ------------------------------------------------------------ */
 /* Parse n sourmash signature files (uncompressed JSON) on `threads` host threads: sketch i =

@@ -78,6 +78,34 @@ def exclusive_counts(hashes: np.ndarray, offsets: np.ndarray, sample: np.ndarray
     return out
 
 
+def exclusive_counts_np(hashes: np.ndarray, offsets: np.ndarray, sample: np.ndarray, mask: np.ndarray = None) -> np.ndarray:
+    """exclusive_counts with whole-array numpy operations, for databases of millions of genomes (the set restatement
+    loops in Python per genome).  tests/test_sparse_oracle.py checks that both agree."""
+    n = offsets.shape[0] - 1
+    out = np.zeros(n, dtype=COUNTS_DTYPE)
+    gid = np.repeat(np.arange(n, dtype=np.int64), np.diff(np.asarray(offsets, dtype=np.int64)))
+    h = np.asarray(hashes, dtype=np.uint64)
+    order = np.lexsort((gid, h))                                   # by hash, then genome
+    h, gid = h[order], gid[order]
+    first = np.ones(h.shape[0], dtype=bool)                       # one entry per distinct (hash, genome): sketches are sets
+    first[1:] = (h[1:] != h[:-1]) | (gid[1:] != gid[:-1])
+    h, gid = h[first], gid[first]
+    in_sample = np.isin(h, np.unique(np.asarray(sample, dtype=np.uint64)))
+    out["n_overlap"] = np.bincount(gid[in_sample], minlength=n)
+    nontrivial = (out["n_overlap"] > 0) if mask is None else (np.asarray(mask) != 0)
+    out["nontrivial"] = nontrivial
+    keep = nontrivial[gid]
+    h, gid, in_sample = h[keep], gid[keep], in_sample[keep]
+    head = np.ones(h.shape[0] + 1, dtype=bool)                    # runs of equal hashes among the nontrivial genomes
+    head[1:-1] = h[1:] != h[:-1]
+    starts = np.flatnonzero(head)
+    run_len = np.diff(starts)
+    excl = np.repeat(run_len == 1, run_len)
+    out["n_exclusive"] = np.bincount(gid[excl], minlength=n)
+    out["n_match"] = np.bincount(gid[excl & in_sample], minlength=n)
+    return out
+
+
 def get_alt_mut_rate(nu: int, thresh: int, ksize: int, significance: float = 0.99) -> float:
     """hypothesis_recovery_src.py:209-230."""
     from scipy.special import betaincinv

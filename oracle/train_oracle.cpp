@@ -31,6 +31,10 @@
 //
 // The index here is a sort-grouped posting array instead of the reference's
 // unordered_map; the counts it yields are identical (same multiset of (hash, id)).
+//
+// yo_train_sparse shares the index and greedy stages with yo_train and accumulates each row over
+// the columns its postings touch instead of a dense row of n counters; tests/test_oracle_pinned.py
+// checks it against yo_train field for field.
 // =====================================================================================
 #include <algorithm>
 #include <cstdint>
@@ -72,13 +76,17 @@ void yo_free_result(yo_result* r) {
     r->selected = nullptr;
 }
 
-// hashes: concatenated sketches (any order inside a sketch, duplicates allowed);
-// offsets: n+1 prefix offsets into hashes.
-int yo_train(const uint64_t* hashes, const uint64_t* offsets, uint32_t n, double thr, yo_result* out) {
-    memset(out, 0, sizeof(*out));
-    const uint64_t T = offsets[n];
+}  // extern "C"
 
-    // ---- inverted index (main.cpp:215-246) -------------------------------------------------
+// The inverted index of main.cpp:215-246 and its statistics.
+struct yo_index {
+    std::vector<uint64_t> key;       // kept hashes (posting length >= 2), ascending
+    std::vector<uint64_t> post_off;  // CSR offsets into post
+    std::vector<int32_t> post;
+};
+
+static void build_index(const uint64_t* hashes, const uint64_t* offsets, uint32_t n, yo_index& ix, yo_result* out) {
+    const uint64_t T = offsets[n];
     // entries are generated in ascending (genome, position) order; a stable sort by hash keeps
     // each posting list in ascending genome order with one entry per occurrence.
     std::vector<std::pair<uint64_t, int32_t>> ent;
@@ -88,18 +96,15 @@ int yo_train(const uint64_t* hashes, const uint64_t* offsets, uint32_t n, double
     std::stable_sort(ent.begin(), ent.end(),
                      [](const std::pair<uint64_t, int32_t>& a, const std::pair<uint64_t, int32_t>& b) { return a.first < b.first; });
 
-    std::vector<uint64_t> key;       // kept hashes (posting length >= 2), ascending
-    std::vector<uint64_t> post_off;  // CSR offsets into post
-    std::vector<int32_t> post;
-    post_off.push_back(0);
+    ix.post_off.push_back(0);
     for (uint64_t s = 0; s < T;) {
         uint64_t e = s;
         while (e < T && ent[e].first == ent[s].first) e++;
         out->n_distinct++;
         if (e - s >= 2) {
-            key.push_back(ent[s].first);
-            for (uint64_t q = s; q < e; q++) post.push_back(ent[q].second);
-            post_off.push_back(post.size());
+            ix.key.push_back(ent[s].first);
+            for (uint64_t q = s; q < e; q++) ix.post.push_back(ent[q].second);
+            ix.post_off.push_back(ix.post.size());
             out->n_postings += e - s;
             out->n_increments += (e - s) * (e - s);
         } else {
@@ -107,46 +112,47 @@ int yo_train(const uint64_t* hashes, const uint64_t* offsets, uint32_t n, double
         }
         s = e;
     }
-    out->n_index = key.size();
-    std::vector<std::pair<uint64_t, int32_t>>().swap(ent);
+    out->n_index = ix.key.size();
+}
 
-    // ---- counts + threshold (main.cpp:252-308) ---------------------------------------------
-    std::vector<yo_pair> pairs;
-    std::vector<std::vector<int32_t>> similars(n);
-    std::vector<int32_t> row(n, 0);
-    for (uint32_t i = 0; i < n; i++) {
-        std::fill(row.begin(), row.end(), 0);
-        for (uint64_t p = offsets[i]; p < offsets[i + 1]; p++) {
-            auto it = std::lower_bound(key.begin(), key.end(), hashes[p]);
-            if (it == key.end() || *it != hashes[p]) continue;
-            size_t r = it - key.begin();
-            for (uint64_t q = post_off[r]; q < post_off[r + 1]; q++) row[post[q]]++;
-        }
-        const uint64_t ni = offsets[i + 1] - offsets[i];
-        for (uint32_t j = 0; j < n; j++) {
-            if (i == j) continue;
-            const int32_t m = row[j];
-            if (m == 0) continue;
-            const uint64_t nj = offsets[j + 1] - offsets[j];
-            if (ni == 0 || nj == 0) continue;
-            // the reference evaluates size_t + size_t - int, i.e. modulo 2^64 (main.cpp:292,296)
-            const uint64_t uni = ni + nj - (uint64_t)(int64_t)m;
-            if (uni == 0) continue;
-            const double jac = 1.0 * m / uni;
-            const double cij = 1.0 * m / ni;
-            const double cji = 1.0 * m / nj;
-            if (cij < thr) continue;
-            yo_pair pr;
-            pr.i = (int32_t)i; pr.j = (int32_t)j; pr.count = m; pr._pad = 0;
-            pr.jaccard = jac; pr.c_ij = cij; pr.c_ji = cji;
-            pairs.push_back(pr);
-            similars[i].push_back((int32_t)j);
-        }
+// M[i][g] += 1 for every query hash of row i and every posting g of that hash (main.cpp:252-262)
+template <class F>
+static void for_each_posting(const uint64_t* hashes, const uint64_t* offsets, const yo_index& ix, uint32_t i, F&& f) {
+    for (uint64_t p = offsets[i]; p < offsets[i + 1]; p++) {
+        auto it = std::lower_bound(ix.key.begin(), ix.key.end(), hashes[p]);
+        if (it == ix.key.end() || *it != hashes[p]) continue;
+        const size_t r = it - ix.key.begin();
+        for (uint64_t q = ix.post_off[r]; q < ix.post_off[r + 1]; q++) f(ix.post[q]);
     }
+}
 
-    // ---- greedy selection (main.cpp:371-420) -----------------------------------------------
-    // same container type, same initial order (file-list order), same comparator, same
-    // std::sort => the same permutation of equal-size genomes as the reference build.
+// the reference's test of one ordered pair (main.cpp:274-308); appends it when it is kept
+static void test_pair(const uint64_t* offsets, uint32_t i, uint32_t j, int32_t m, double thr, std::vector<yo_pair>& pairs) {
+    if (i == j) return;
+    if (m == 0) return;
+    const uint64_t ni = offsets[i + 1] - offsets[i];
+    const uint64_t nj = offsets[j + 1] - offsets[j];
+    if (ni == 0 || nj == 0) return;
+    // the reference evaluates size_t + size_t - int, i.e. modulo 2^64 (main.cpp:292,296)
+    const uint64_t uni = ni + nj - (uint64_t)(int64_t)m;
+    if (uni == 0) return;
+    const double jac = 1.0 * m / uni;
+    const double cij = 1.0 * m / ni;
+    const double cji = 1.0 * m / nj;
+    if (cij < thr) return;
+    yo_pair pr;
+    pr.i = (int32_t)i; pr.j = (int32_t)j; pr.count = m; pr._pad = 0;
+    pr.jaccard = jac; pr.c_ij = cij; pr.c_ji = cji;
+    pairs.push_back(pr);
+}
+
+// greedy selection (main.cpp:371-420) over the kept pairs (row-major: each genome's similars in ascending j).
+// Same container type, same initial order (file-list order), same comparator, same std::sort => the same
+// permutation of equal-size genomes as the reference build.
+static void greedy(const uint64_t* offsets, uint32_t n, const std::vector<yo_pair>& pairs, yo_result* out) {
+    std::vector<uint64_t> sim_off(n + 1, 0);
+    for (const yo_pair& pr : pairs) sim_off[pr.i + 1]++;
+    for (uint32_t g = 0; g < n; g++) sim_off[g + 1] += sim_off[g];
     std::vector<std::pair<int, int>> id_size(n);
     for (uint32_t g = 0; g < n; g++) id_size[g] = {(int)g, (int)(offsets[g + 1] - offsets[g])};
     std::sort(id_size.begin(), id_size.end(),
@@ -157,7 +163,8 @@ int yo_train(const uint64_t* hashes, const uint64_t* offsets, uint32_t n, double
         const int g = id_size[v].first;
         const int sz = id_size[v].second;
         bool keep = true;
-        for (int32_t o : similars[g]) {
+        for (uint64_t k = sim_off[g]; k < sim_off[g + 1]; k++) {
+            const int32_t o = pairs[k].j;
             if (dropped[o]) continue;
             const int so = (int)(offsets[o + 1] - offsets[o]);
             if (so >= sz) { keep = false; break; }
@@ -165,13 +172,69 @@ int yo_train(const uint64_t* hashes, const uint64_t* offsets, uint32_t n, double
         if (keep) selected.push_back(g);
         else dropped[g] = true;
     }
-
-    out->n_pairs = pairs.size();
-    out->pairs = (yo_pair*)malloc(sizeof(yo_pair) * (pairs.size() ? pairs.size() : 1));
-    if (!pairs.empty()) memcpy(out->pairs, pairs.data(), sizeof(yo_pair) * pairs.size());
     out->n_selected = (uint32_t)selected.size();
     out->selected = (int32_t*)malloc(sizeof(int32_t) * (selected.size() ? selected.size() : 1));
     if (!selected.empty()) memcpy(out->selected, selected.data(), sizeof(int32_t) * selected.size());
+}
+
+static void emit_pairs(const std::vector<yo_pair>& pairs, yo_result* out) {
+    out->n_pairs = pairs.size();
+    out->pairs = (yo_pair*)malloc(sizeof(yo_pair) * (pairs.size() ? pairs.size() : 1));
+    if (!pairs.empty()) memcpy(out->pairs, pairs.data(), sizeof(yo_pair) * pairs.size());
+}
+
+extern "C" {
+
+// hashes: concatenated sketches (any order inside a sketch, duplicates allowed);
+// offsets: n+1 prefix offsets into hashes.
+int yo_train(const uint64_t* hashes, const uint64_t* offsets, uint32_t n, double thr, yo_result* out) {
+    memset(out, 0, sizeof(*out));
+    yo_index ix;
+    build_index(hashes, offsets, n, ix, out);
+
+    // ---- counts + threshold (main.cpp:252-308): a dense row of n counters, scanned in full -----
+    std::vector<yo_pair> pairs;
+    std::vector<int32_t> row(n, 0);
+    for (uint32_t i = 0; i < n; i++) {
+        std::fill(row.begin(), row.end(), 0);
+        for_each_posting(hashes, offsets, ix, i, [&](int32_t g) { row[g]++; });
+        for (uint32_t j = 0; j < n; j++) test_pair(offsets, i, j, row[j], thr, pairs);
+    }
+    emit_pairs(pairs, out);
+    greedy(offsets, n, pairs, out);
+    return 0;
+}
+
+// The same result in O(sum of L^2) instead of O(n^2): per row, only the columns a posting touched are
+// visited, so databases of millions of genomes can be checked.  With a row range [row_begin, row_end) it
+// returns what ygpu_pairwise_flag does for that range: both ordered pairs of every {i, j} whose smaller
+// genome i lies in the range (the counts are symmetric), ordered by (i, j); the full range is yo_train's
+// pair list.  `selected` is the greedy order over the returned pairs (the reference's for the full range).
+int yo_train_sparse(const uint64_t* hashes, const uint64_t* offsets, uint32_t n, double thr, uint32_t row_begin,
+                    uint32_t row_end, yo_result* out) {
+    memset(out, 0, sizeof(*out));
+    if (row_begin > row_end || row_end > n) return 1;
+    yo_index ix;
+    build_index(hashes, offsets, n, ix, out);
+
+    std::vector<yo_pair> pairs;
+    std::vector<int32_t> row(n, 0);
+    std::vector<int32_t> touched;
+    for (uint32_t i = row_begin; i < row_end; i++) {
+        touched.clear();
+        for_each_posting(hashes, offsets, ix, i, [&](int32_t g) { if (row[g]++ == 0) touched.push_back(g); });
+        std::sort(touched.begin(), touched.end());
+        for (int32_t j : touched) {
+            if ((uint32_t)j > i) {
+                test_pair(offsets, i, (uint32_t)j, row[j], thr, pairs);
+                test_pair(offsets, (uint32_t)j, i, row[j], thr, pairs);
+            }
+            row[j] = 0;
+        }
+    }
+    std::sort(pairs.begin(), pairs.end(), [](const yo_pair& a, const yo_pair& b) { return a.i != b.i ? a.i < b.i : a.j < b.j; });
+    emit_pairs(pairs, out);
+    greedy(offsets, n, pairs, out);
     return 0;
 }
 

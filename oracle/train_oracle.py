@@ -1,6 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- Python handle on the CPU oracles of the train path.
 
-* :func:`oracle_train`  calls the C++ restatement (oracle/train_oracle.cpp) through ctypes.
+* :func:`oracle_train`  calls the C++ restatement (oracle/train_oracle.cpp) through ctypes;
+  :func:`oracle_train_sparse` the same restatement with a sparse row accumulator, for large databases.
 * :func:`reference_train` runs the UNMODIFIED reference core (oracle/_ref/run_yacht_train_core_ref,
   compiled from /root/reference/src/cpp by oracle/Makefile) on signature files written to a
   scratch directory, and parses what it wrote.
@@ -85,6 +86,9 @@ def _load():
         lib.yo_train.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.c_double,
                                  ctypes.POINTER(_YoResult)]
         lib.yo_train.restype = ctypes.c_int
+        lib.yo_train_sparse.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint32, ctypes.c_double, ctypes.c_uint32,
+                                        ctypes.c_uint32, ctypes.POINTER(_YoResult)]
+        lib.yo_train_sparse.restype = ctypes.c_int
         lib.yo_free_result.argtypes = [ctypes.POINTER(_YoResult)]
         lib.yo_format_pair.argtypes = [ctypes.POINTER(_YoPair), ctypes.c_char_p, ctypes.c_int]
         lib.yo_format_pair.restype = ctypes.c_int
@@ -107,6 +111,29 @@ def oracle_train(hashes: np.ndarray, offsets: np.ndarray, thr: float) -> TrainRe
     rc = lib.yo_train(hashes.ctypes.data, offsets.ctypes.data, n, float(thr), ctypes.byref(res))
     if rc != 0:
         raise RuntimeError(f"yo_train failed rc={rc}")
+    return _take(lib, res)
+
+
+def oracle_train_sparse(hashes: np.ndarray, offsets: np.ndarray, thr: float, row_begin: int = 0,
+                        row_end: Optional[int] = None) -> TrainResult:
+    """oracle_train with a sparse row accumulator (yo_train_sparse): O(sum of L^2) instead of O(n^2), so databases of
+    millions of genomes can be checked.  A row range returns what GpuContext.pairwise_flag does for it: both ordered pairs
+    of every {i, j} whose smaller genome lies in [row_begin, row_end).  `selected` is the greedy order over the returned
+    pairs (the reference's when the range is the whole database)."""
+    lib = _load()
+    hashes = np.ascontiguousarray(hashes, dtype=np.uint64)
+    offsets = np.ascontiguousarray(offsets, dtype=np.uint64)
+    n = offsets.shape[0] - 1
+    res = _YoResult()
+    rc = lib.yo_train_sparse(hashes.ctypes.data, offsets.ctypes.data, n, float(thr), int(row_begin),
+                             n if row_end is None else int(row_end), ctypes.byref(res))
+    if rc != 0:
+        raise RuntimeError(f"yo_train_sparse failed rc={rc}")
+    return _take(lib, res)
+
+
+def _take(lib, res: _YoResult) -> TrainResult:
+    """Copy a yo_result into numpy and release it."""
     try:
         npairs = int(res.n_pairs)
         if npairs:

@@ -19,7 +19,7 @@ ABI_SYMBOLS = [
     "ygpu_device_count", "ygpu_ctx_create", "ygpu_ctx_destroy", "ygpu_last_error", "ygpu_free",
     "ygpu_host_alloc", "ygpu_host_free", "ygpu_read_signatures", "ygpu_read_signatures_ksize", "ygpu_sketch_set_free", "ygpu_alt_mut_rate", "ygpu_reset_timers", "ygpu_get_timings", "ygpu_load_sketches", "ygpu_load_sketch_blocks", "ygpu_load_sketches_device",
     "ygpu_build_index", "ygpu_pairwise_flag", "ygpu_pairwise_flag_device", "ygpu_pairs_copy", "ygpu_row_partition",
-    "ygpu_mark", "ygpu_elapsed_ms", "ygpu_set_option", "ygpu_exclusive_hashes",
+    "ygpu_mark", "ygpu_elapsed_ms", "ygpu_set_option", "ygpu_get_option", "ygpu_exclusive_hashes",
     "ygpu_hyp_test",
     "ygpu_upload_begin", "ygpu_upload_block", "ygpu_upload_finish", "ygpu_greedy_select",
     "ygpu_comm_get_unique_id", "ygpu_comm_init", "ygpu_comm_destroy", "ygpu_load_sketches_sharded", "ygpu_load_sketches_sharded_device",
@@ -138,6 +138,7 @@ def load_library() -> ctypes.CDLL:
     lib.ygpu_mark.argtypes = [vp, ctypes.c_int]
     lib.ygpu_elapsed_ms.argtypes = [vp, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_double)]
     lib.ygpu_set_option.argtypes = [vp, ctypes.c_char_p, ctypes.c_int64]
+    lib.ygpu_get_option.argtypes = [vp, ctypes.c_char_p, ctypes.POINTER(ctypes.c_int64)]
     lib.ygpu_exclusive_hashes.argtypes = [vp, vp, u64, vp, vp]
     lib.ygpu_hyp_test.argtypes = [vp, vp, vp, u64, ctypes.c_int, ctypes.c_double, ctypes.c_double, vp, ctypes.c_int, vp]
     lib.ygpu_greedy_select.argtypes = [vp, u32, vp, u64, vp, ctypes.POINTER(u32)]
@@ -340,6 +341,12 @@ class GpuContext:
 
     def set_option(self, name: str, value: int) -> None:
         self._check(self.lib.ygpu_set_option(self.h, name.encode(), int(value)), "ygpu_set_option")
+
+    def get_option(self, name: str) -> int:
+        """Read-only state of the last count call (include/yacht_gpu.h: ygpu_get_option)."""
+        v = ctypes.c_int64(0)
+        self._check(self.lib.ygpu_get_option(self.h, name.encode(), ctypes.byref(v)), "ygpu_get_option")
+        return int(v.value)
 
     def row_partition(self, nparts: int) -> np.ndarray:
         b = np.zeros(nparts + 1, dtype=np.uint32)

@@ -70,6 +70,9 @@ struct ygpu_ctx {
     int count_kernel = 0;           // 0: automatic, 1: dense row accumulator per CTA, 2: one warp per row (hash table)
     int last_count_kernel = 0;
     unsigned long long last_count_overflow_rows = 0;
+    uint32_t last_count_tile_w = 0; // accumulator geometry of the last dense count launch: columns per tile, tiles, packed u16
+    uint32_t last_count_n_tiles = 0;
+    int last_count_u16 = 0;
     uint32_t* d_ovf_rows = nullptr; // rows the warp kernel deferred to the dense kernel
     uint32_t* d_tc = nullptr;       // [n] smallest shared-hash count that passes the containment test of genome g
     bool skip_pair_sort = false;    // sharded step: the pair lists of all ranks are ordered once, after the gather

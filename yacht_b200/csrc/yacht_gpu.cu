@@ -1304,6 +1304,9 @@ static int pairwise_device(ygpu_ctx* ctx, double threshold, uint32_t row_begin, 
             ctx->tm.n_count_launches++;
             ctx->last_count_kernel = use_warp ? 2 : 1;
             ctx->last_count_overflow_rows = novf;
+            ctx->last_count_tile_w = tile_w;
+            ctx->last_count_n_tiles = n_tiles;
+            ctx->last_count_u16 = use_u16 ? 1 : 0;
             npairs = cnt;
             if (npairs <= ctx->out_cap) break;
             if (attempt == 1) return ygpu_fail(ctx, YGPU_ERR_CUDA, "pair buffer overflow after resize");
@@ -1415,6 +1418,16 @@ extern "C" int ygpu_set_option(ygpu_ctx* ctx, const char* name, int64_t value) {
     }
     if (!strcmp(name, "group_ctas")) { ctx->group_ctas = (int)value; return 0; }
     if (!strcmp(name, "count_thresholds")) { ctx->count_thresholds = (int)value; return 0; }
+    return ygpu_fail(ctx, YGPU_ERR_ARG, "unknown option %s", name);
+}
+
+extern "C" int ygpu_get_option(ygpu_ctx* ctx, const char* name, int64_t* out) {
+    if (!ctx || !name || !out) return YGPU_ERR_ARG;
+    if (!strcmp(name, "last_count_kernel")) { *out = ctx->last_count_kernel; return 0; }
+    if (!strcmp(name, "last_count_overflow_rows")) { *out = (int64_t)ctx->last_count_overflow_rows; return 0; }
+    if (!strcmp(name, "last_count_tile_w")) { *out = ctx->last_count_tile_w; return 0; }
+    if (!strcmp(name, "last_count_n_tiles")) { *out = ctx->last_count_n_tiles; return 0; }
+    if (!strcmp(name, "last_count_u16")) { *out = ctx->last_count_u16; return 0; }
     return ygpu_fail(ctx, YGPU_ERR_ARG, "unknown option %s", name);
 }
 
