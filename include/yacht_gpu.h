@@ -311,6 +311,12 @@ void ygpu_sketch_result_free(ygpu_sketch_result* r);
  *                                        fastest); reading the next piece on another thread overlaps the device work
  *   ygpu_stream_end_file(ctx)            end of the current file and its checks; the next feed starts a new file
  *   ygpu_stream_finish(ctx, &result, &stats, &names, &name_offsets, &n_names)
+ * Several k-mer sizes in one pass: ygpu_stream_begin_k(ctx, ksizes, n_k, ...) takes 1 to 8 distinct sizes in [1, 256]
+ * (otherwise YGPU_ERR_ARG); the text is parsed once and every size is hashed on it.  ygpu_stream_finish_k fills
+ * result[0 .. n_k), in the order of ksizes, each exactly the result of a stream begun with that size alone (n_kmers: that
+ * size's valid windows); stats.n_kmers is their sum, ms_hash covers every size's kernel, the names are shared.  Per-record
+ * mode needs records x n_k < 2^32.  ygpu_stream_begin / _finish are the n_k = 1 case; ygpu_stream_finish refuses a stream
+ * of several sizes.
  * Malformed input fails with YGPU_ERR_ARG and one of "neither FASTA ('>') nor FASTQ ('@')", "malformed FASTQ record at
  * line N", "FASTQ with N lines (not a multiple of 4)" (lines counted from the first byte after the leading whitespace);
  * the stream must then be begun again.  Names (the header line without its first byte and without '\r') are kept for
@@ -326,7 +332,8 @@ typedef struct {
     uint64_t n_chunks;      /* device chunks parsed                                                 */
     double ms_h2d;          /* host -> device copies of the raw text                                */
     double ms_parse;        /* line scan, classification, compaction                                */
-    double ms_hash;         /* the K7 hashing kernel                                                */
+    double ms_hash;         /* the K7 hashing kernel; with several k-mer sizes every size's kernel, and the packing of
+                               each size's kept hashes but the last one's                                                  */
     double ms_merge;        /* sort + reduce of each chunk's kept hashes into the resident sketch   */
 } ygpu_stream_stats;
 int ygpu_stream_begin(ygpu_ctx* ctx, int ksize, uint64_t max_hash, uint32_t seed, int mode);
@@ -334,6 +341,9 @@ int ygpu_stream_feed(ygpu_ctx* ctx, const uint8_t* bytes, uint64_t n);
 int ygpu_stream_end_file(ygpu_ctx* ctx);
 int ygpu_stream_finish(ygpu_ctx* ctx, ygpu_sketch_result* out, ygpu_stream_stats* stats /* may be NULL */,
                        char** names, uint64_t** name_offsets, uint64_t* n_names);
+int ygpu_stream_begin_k(ygpu_ctx* ctx, const int* ksizes, int n_k, uint64_t max_hash, uint32_t seed, int mode);
+int ygpu_stream_finish_k(ygpu_ctx* ctx, ygpu_sketch_result* out /* [n_k], order of ksizes */, ygpu_stream_stats* stats /* may be NULL */,
+                         char** names, uint64_t** name_offsets, uint64_t* n_names);
 
 #ifdef __cplusplus
 }

@@ -26,6 +26,7 @@ ABI_SYMBOLS = [
     "ygpu_train_step_sharded", "ygpu_upload_finish_sharded", "ygpu_load_sketches_hashrange", "ygpu_load_sketches_hashrange_device",
     "ygpu_train_step_replicated", "ygpu_sketch_sequences", "ygpu_sketch_result_free",
     "ygpu_stream_begin", "ygpu_stream_feed", "ygpu_stream_end_file", "ygpu_stream_finish",
+    "ygpu_stream_begin_k", "ygpu_stream_finish_k",
 ]
 STREAM_WHOLE, STREAM_PER_RECORD = 0, 1
 COMM_ID_BYTES = 128
@@ -160,6 +161,9 @@ def load_library() -> ctypes.CDLL:
     lib.ygpu_stream_end_file.argtypes = [vp]
     lib.ygpu_stream_finish.argtypes = [vp, ctypes.POINTER(SketchResult), ctypes.POINTER(StreamStats), ctypes.POINTER(vp),
                                        ctypes.POINTER(vp), ctypes.POINTER(u64)]
+    lib.ygpu_stream_begin_k.argtypes = [vp, vp, ctypes.c_int, u64, u32, ctypes.c_int]
+    lib.ygpu_stream_finish_k.argtypes = [vp, ctypes.POINTER(SketchResult), ctypes.POINTER(StreamStats), ctypes.POINTER(vp),
+                                         ctypes.POINTER(vp), ctypes.POINTER(u64)]
     for name in ABI_SYMBOLS:
         getattr(lib, name)  # AttributeError here means the .so does not match include/yacht_gpu.h
     _lib = lib
@@ -394,9 +398,18 @@ class GpuContext:
         mv = memoryview((ctypes.c_uint8 * int(nbytes)).from_address(ptr)).cast("B")
         return mv, int(ptr), lambda: self.lib.ygpu_host_free(ctypes.c_void_p(ptr))
 
-    def stream_begin(self, ksize: int, max_hash: int, seed: int = 42, per_record: bool = False) -> None:
-        self._check(self.lib.ygpu_stream_begin(self.h, int(ksize), int(max_hash), int(seed),
-                                               STREAM_PER_RECORD if per_record else STREAM_WHOLE), "ygpu_stream_begin")
+    def stream_begin(self, ksize, max_hash: int, seed: int = 42, per_record: bool = False) -> None:
+        """ksize: one k-mer size (ygpu_stream_begin) or a sequence of them (ygpu_stream_begin_k: one pass, a result per k)."""
+        mode = STREAM_PER_RECORD if per_record else STREAM_WHOLE
+        if isinstance(ksize, (int, np.integer)):
+            self._stream_nk = None
+            self._check(self.lib.ygpu_stream_begin(self.h, int(ksize), int(max_hash), int(seed), mode), "ygpu_stream_begin")
+            return
+        ks = np.ascontiguousarray([int(k) for k in ksize], dtype=np.int32)
+        self._stream_nk = None
+        self._check(self.lib.ygpu_stream_begin_k(self.h, ks.ctypes.data if ks.size else None, int(ks.size), int(max_hash), int(seed), mode),
+                    "ygpu_stream_begin_k")
+        self._stream_nk = int(ks.size)
 
     def stream_feed(self, ptr: int, n: int, path: Optional[str] = None) -> None:
         """The next n bytes of the current file at host address ptr (free to reuse when this returns)."""
@@ -406,29 +419,38 @@ class GpuContext:
         self._stream_error(self.lib.ygpu_stream_end_file(self.h), "ygpu_stream_end_file", path)
 
     def stream_finish(self, path: Optional[str] = None):
-        """-> (hashes, abundances, offsets, names or None, stats dict); names are bytes, one per record that kept its name."""
-        res, st = SketchResult(), StreamStats()
+        """-> (hashes, abundances, offsets, names or None, stats dict); names are bytes, one per record that kept its name.
+        A stream begun with a sequence of k-mer sizes returns ([(hashes, abundances, offsets, n_kmers) per k, in the order
+        given], names or None, stats dict) instead."""
+        nk = getattr(self, "_stream_nk", None)
+        res, st = (SketchResult * (nk or 1))(), StreamStats()
         names, name_off, n_names = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_uint64()
-        self._stream_error(self.lib.ygpu_stream_finish(self.h, ctypes.byref(res), ctypes.byref(st), ctypes.byref(names),
-                                                       ctypes.byref(name_off), ctypes.byref(n_names)), "ygpu_stream_finish", path)
+        fn, what = (self.lib.ygpu_stream_finish, "ygpu_stream_finish") if nk is None else (self.lib.ygpu_stream_finish_k, "ygpu_stream_finish_k")
+        self._stream_error(fn(self.h, res, ctypes.byref(st), ctypes.byref(names), ctypes.byref(name_off), ctypes.byref(n_names)), what, path)
         try:
-            ns = int(res.n_sketches)
-            offsets = np.ctypeslib.as_array(res.offsets, shape=(ns + 1,)).copy()
-            total = int(offsets[-1])
-            if total:
-                hashes = np.ctypeslib.as_array(res.hashes, shape=(total,)).copy()
-                abund = np.ctypeslib.as_array(res.abundances, shape=(total,)).copy()
-            else:
-                hashes, abund = np.zeros(0, np.uint64), np.zeros(0, np.uint32)
+            per_k = []
+            for r in res:
+                ns = int(r.n_sketches)
+                offsets = np.ctypeslib.as_array(r.offsets, shape=(ns + 1,)).copy()
+                total = int(offsets[-1])
+                if total:
+                    hashes = np.ctypeslib.as_array(r.hashes, shape=(total,)).copy()
+                    abund = np.ctypeslib.as_array(r.abundances, shape=(total,)).copy()
+                else:
+                    hashes, abund = np.zeros(0, np.uint64), np.zeros(0, np.uint32)
+                per_k.append((hashes, abund, offsets, int(r.n_kmers)))
             out_names = None
             nn = int(n_names.value)
             if nn:
                 off = np.ctypeslib.as_array(ctypes.cast(name_off, ctypes.POINTER(ctypes.c_uint64)), shape=(nn + 1,)).copy()
                 blob = ctypes.string_at(names, int(off[-1])) if int(off[-1]) else b""
                 out_names = [blob[int(off[i]):int(off[i + 1])] for i in range(nn)]
-            return hashes, abund, offsets, out_names, st.as_dict()
+            if nk is None:
+                return per_k[0][0], per_k[0][1], per_k[0][2], out_names, st.as_dict()
+            return per_k, out_names, st.as_dict()
         finally:
-            self.lib.ygpu_sketch_result_free(ctypes.byref(res))
+            for r in res:
+                self.lib.ygpu_sketch_result_free(ctypes.byref(r))
             self.lib.ygpu_free(names)
             self.lib.ygpu_free(name_off)
 

@@ -181,6 +181,27 @@ static inline int dev_alloc(ygpu_ctx* ctx, T** p, uint64_t count) {
     ctx->caps[(void*)p] = want;
     return 0;
 }
+// dev_alloc that keeps the first `keep` elements: a buffer too small for `count` is replaced by a larger one and the kept
+// elements are copied over on `st` before the old buffer is freed (cudaFree waits for the copy).
+template <typename T>
+static inline int dev_grow_keep(ygpu_ctx* ctx, T** p, uint64_t count, uint64_t keep, cudaStream_t st) {
+    auto it = ctx->caps.find((void*)p);
+    if (!keep || !*p || it == ctx->caps.end() || it->second >= std::max<uint64_t>(count, 1) * sizeof(T)) return dev_alloc(ctx, p, count);
+    T* old = *p;
+    const size_t old_cap = it->second;
+    *p = nullptr;                                   // dev_alloc makes a new buffer and leaves the old one alone
+    ctx->caps.erase((void*)p);
+    const int rc = dev_alloc(ctx, p, count);
+    if (rc) {
+        *p = old;
+        ctx->caps[(void*)p] = old_cap;
+        return rc;
+    }
+    const cudaError_t e = cudaMemcpyAsync(*p, old, keep * sizeof(T), cudaMemcpyDeviceToDevice, st);
+    cudaFree(old);
+    if (e != cudaSuccess) return ygpu_fail(ctx, YGPU_ERR_CUDA, "dev_grow_keep: %s", cudaGetErrorString(e));
+    return 0;
+}
 template <typename T>
 static inline void dev_free(ygpu_ctx* ctx, T** p) {
     if (*p) cudaFree(*p);
@@ -242,7 +263,8 @@ void ygpu_stream_release(ygpu_ctx* ctx);
 // K7 on a device buffer (d_bases zero-padded by YG_SKETCH_PAD bytes behind n_bases); survivors stay in the sketch scratch
 constexpr uint64_t YG_SKETCH_PAD = 4096 + 256 + 16;
 constexpr uint64_t YG_STREAM_CHUNK_MAX = 1ull << 30;
-int ygpu_sketch_hash_device(ygpu_ctx* ctx, const uint8_t* d_bases, uint64_t n_bases, const uint64_t* d_off, uint32_t n_sketches,
-                            int ksize, uint64_t max_hash, uint32_t seed, cudaEvent_t ev_done, uint64_t* m, uint64_t* n_kmers);
+int ygpu_sketch_hash_device(ygpu_ctx* ctx, const uint8_t* d_bases, uint64_t n_bases, uint64_t* d_off, uint32_t n_sketches,
+                            int ksize, uint64_t max_hash, uint32_t seed, uint64_t first_new, cudaEvent_t ev_done, uint64_t* m,
+                            uint64_t* n_kmers);
 void ygpu_sketch_survivors(ygpu_ctx* ctx, uint64_t** d_key, uint32_t** d_sid);
 void ygpu_upload_release(ygpu_ctx* ctx);

@@ -8,13 +8,17 @@
 //   scans         : output positions of the sequence and name bytes, record ordinals
 //   k_sq_scatter  : compacted hashing buffer = carried bases of the open record + this chunk's sequence bytes, one '\n'
 //                   per record start; record start offsets; name bytes
-//   k_sq_finish   : chunk totals, the carried state for the next chunk (line number, open line, last k - 1 bases)
-// then the K7 hashing kernels (ygpu_sketch_hash_device) and a merge of the chunk's kept hashes into the resident sketch:
-// radix sort of (resident + new) by hash, stably by record, and a reduction that adds the abundances.
+//   k_sq_finish   : chunk totals, the carried state for the next chunk (line number, open line, last k_max - 1 bases)
+// then, for every k-mer size of the stream, the K7 hashing kernel (ygpu_sketch_hash_device) on the same compacted buffer; a
+// window that lies inside the carried bases was hashed with the previous chunk and is skipped (ysq_window_new).  The kept
+// hashes of all sizes go into one buffer under a composite id cid = record * n_k + k index, and one merge orders them into the
+// resident sketch: radix sort of (resident + new) by hash, stably by cid, and a reduction that adds the abundances.
 #include "common.cuh"
 #include "seq_stream.cuh"
+#include "sketch_hash.cuh"
 
 #include <cub/cub.cuh>
+#include <algorithm>
 #include <cstddef>
 #include <cstdio>
 #include <cstdlib>
@@ -35,7 +39,10 @@ struct ysq_chunk {
 
 struct StreamState {
     bool active = false;
-    int ksize = 0;
+    int n_k = 0;                      // k-mer sizes, in the caller's order
+    int ks[YSQ_MAX_K] = {};
+    int k_max = 0;
+    uint64_t n_kmers_k[YSQ_MAX_K] = {};   // valid windows hashed, per k
     uint64_t max_hash = 0;
     uint32_t seed = 0;
     int mode = YGPU_STREAM_WHOLE;
@@ -64,7 +71,7 @@ struct StreamState {
     uint64_t* d_off = nullptr;
     uint8_t* d_names = nullptr;
     uint32_t* d_name_start = nullptr;
-    // resident sketch: hash, (record << 32) | abundance, sorted by (record, hash)
+    // resident sketch: hash, (cid << 32) | abundance, sorted by (cid, hash); cid = record * n_k + k index (record 0 in whole mode)
     uint64_t* d_rh = nullptr;
     uint64_t* d_rv = nullptr;
     uint64_t n_res = 0;
@@ -196,11 +203,12 @@ __global__ void k_sq_finish(const uint8_t* __restrict__ raw, uint64_t n, const u
 }
 
 __global__ void __launch_bounds__(256) k_sq_pack(const uint64_t* __restrict__ key, const uint32_t* __restrict__ sid, uint64_t m,
-                                                  uint32_t sid_base, int whole, uint64_t* __restrict__ h, uint64_t* __restrict__ v) {
+                                                  uint32_t sid_base, int whole, uint32_t n_k, uint32_t ki, uint64_t* __restrict__ h,
+                                                  uint64_t* __restrict__ v) {
     for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < m; i += (uint64_t)gridDim.x * blockDim.x) {
         const uint32_t rec = whole ? 0u : sid[i] + sid_base;      // local sketch 0 is the record open at the chunk's start
         h[i] = key[i];
-        v[i] = ((uint64_t)rec << 32) | 1ull;
+        v[i] = ((uint64_t)(rec * n_k + ki) << 32) | 1ull;
     }
 }
 
@@ -259,31 +267,42 @@ int sq_alloc_chunk(ygpu_ctx* ctx, StreamState* S) {
     return ygpu_temp_reserve(ctx, std::max(std::max(t1, t2), std::max(t3, t4)));
 }
 
-// Kept hashes of the chunk (sketch scratch) -> resident sketch.
-int sq_merge(ygpu_ctx* ctx, StreamState* S, uint64_t m, uint32_t sid_base) {
+// The m kept hashes of k index ki (sketch scratch) -> the merge input d_ah / d_av behind the resident sketch and the `added`
+// kept hashes of the chunk's earlier k-mer sizes, which stay where they are.
+int sq_add(ygpu_ctx* ctx, StreamState* S, uint64_t added, uint64_t m, uint32_t sid_base, int ki) {
     cudaStream_t st = ctx->stream;
     uint64_t* d_key;
     uint32_t* d_sid;
     ygpu_sketch_survivors(ctx, &d_key, &d_sid);
-    const uint64_t r = S->n_res, t = r + m;
+    const uint64_t r = S->n_res, used = r + added, t = used + m;
     if (t >= (1ull << 32)) return sq_fail(ctx, S, YGPU_ERR_ARG, "ygpu_stream: more than 2^32 kept hashes");
-    YG_CHECK(dev_alloc(ctx, &S->d_ah, t));
-    YG_CHECK(dev_alloc(ctx, &S->d_av, t));
+    YG_CHECK(dev_grow_keep(ctx, &S->d_ah, t, added ? used : 0, st));
+    YG_CHECK(dev_grow_keep(ctx, &S->d_av, t, added ? used : 0, st));
+    if (!added && r) {
+        YG_CUDA(ctx, cudaMemcpyAsync(S->d_ah, S->d_rh, r * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+        YG_CUDA(ctx, cudaMemcpyAsync(S->d_av, S->d_rv, r * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+    }
+    k_sq_pack<<<grid_for(ctx, m, 256), 256, 0, st>>>(d_key, d_sid, m, sid_base, S->mode == YGPU_STREAM_WHOLE ? 1 : 0, (uint32_t)S->n_k,
+                                                     (uint32_t)ki, S->d_ah + used, S->d_av + used);
+    YG_CUDA(ctx, cudaGetLastError());
+    ctx->tm.n_kernel_launches++;
+    return 0;
+}
+
+// Resident sketch + the chunk's m kept hashes (all k-mer sizes, in d_ah / d_av behind it) -> resident sketch.
+int sq_merge(ygpu_ctx* ctx, StreamState* S, uint64_t m) {
+    cudaStream_t st = ctx->stream;
+    const uint64_t t = S->n_res + m;
     YG_CHECK(dev_alloc(ctx, &S->d_bh, t));
     YG_CHECK(dev_alloc(ctx, &S->d_bv, t));
     YG_CHECK(dev_alloc(ctx, &S->d_mflag, t));
     YG_CHECK(dev_alloc(ctx, &S->d_mpos, t));
-    if (r) {
-        YG_CUDA(ctx, cudaMemcpyAsync(S->d_ah, S->d_rh, r * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
-        YG_CUDA(ctx, cudaMemcpyAsync(S->d_av, S->d_rv, r * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
-    }
     const bool whole = S->mode == YGPU_STREAM_WHOLE;
-    k_sq_pack<<<grid_for(ctx, m, 256), 256, 0, st>>>(d_key, d_sid, m, sid_base, whole ? 1 : 0, S->d_ah + r, S->d_av + r);
-    YG_CUDA(ctx, cudaGetLastError());
     int hash_bits = 64;
     while (hash_bits > 1 && !((S->max_hash >> (hash_bits - 1)) & 1)) hash_bits--;
+    const uint64_t n_cid = (whole ? 1 : S->h_state->n_records + 1) * (uint64_t)S->n_k;
     int sid_bits = 1;
-    while (sid_bits < 32 && (1ull << sid_bits) < S->h_state->n_records + 1) sid_bits++;
+    while (sid_bits < 32 && (1ull << sid_bits) < n_cid) sid_bits++;
     size_t tb1 = 0, tb2 = 0, tb3 = 0;
     YG_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, tb1, S->d_ah, S->d_bh, S->d_av, S->d_bv, (int64_t)t, 0, hash_bits, st));
     YG_CUDA(ctx, cub::DeviceRadixSort::SortPairs(nullptr, tb2, S->d_bv, S->d_av, S->d_bh, S->d_ah, (int64_t)t, 32, 32 + sid_bits, st));
@@ -294,7 +313,7 @@ int sq_merge(ygpu_ctx* ctx, StreamState* S, uint64_t m, uint32_t sid_base) {
     const uint64_t* h = S->d_bh;
     const uint64_t* v = S->d_bv;
     ctx->tm.n_library_launches += 3;
-    if (!whole) {       // stable by record: (record, hash) order
+    if (!whole || S->n_k > 1) {       // stable by cid: (cid, hash) order
         tb = ctx->temp_bytes;
         YG_CUDA(ctx, cub::DeviceRadixSort::SortPairs(ctx->d_temp, tb, S->d_bv, S->d_av, S->d_bh, S->d_ah, (int64_t)t, 32, 32 + sid_bits, st));
         h = S->d_ah;
@@ -314,7 +333,7 @@ int sq_merge(ygpu_ctx* ctx, StreamState* S, uint64_t m, uint32_t sid_base) {
     YG_CUDA(ctx, cudaMemsetAsync(S->d_rv, 0, (size_t)nd * sizeof(uint64_t), st));
     k_sq_reduce<<<g, 256, 0, st>>>(h, v, S->d_mflag, S->d_mpos, t, S->d_rh, (unsigned long long*)S->d_rv);
     YG_CUDA(ctx, cudaGetLastError());
-    ctx->tm.n_kernel_launches += 3;
+    ctx->tm.n_kernel_launches += 2;
     S->n_res = nd;
     return 0;
 }
@@ -326,6 +345,9 @@ int sq_chunk(ygpu_ctx* ctx, StreamState* S, const uint8_t* p, uint64_t n) {
     const int g = grid_for(ctx, n, SQ_NT);
     const int want_names = S->mode == YGPU_STREAM_PER_RECORD ? 2 : 1;
     const uint64_t rec_before = S->h_state->n_records;
+    const uint64_t n_carry = S->h_state->n_carry;                 // bases the previous chunk hashed already lead this one
+    uint8_t carry_in[YSQ_CARRY_MAX];
+    memcpy(carry_in, S->h_state->carry, n_carry);
     YG_CUDA(ctx, cudaEventRecord(S->ev[0], st));
     YG_CUDA(ctx, cudaMemcpyAsync(S->d_raw, p, n, cudaMemcpyHostToDevice, st));
     YG_CUDA(ctx, cudaEventRecord(S->ev[1], st));
@@ -351,7 +373,7 @@ int sq_chunk(ygpu_ctx* ctx, StreamState* S, const uint8_t* p, uint64_t n) {
                                       S->d_name_start);
     YG_CUDA(ctx, cudaGetLastError());
     k_sq_finish<<<1, 1, 0, st>>>(S->d_raw, n, S->d_line, S->d_flags, S->d_pos_a, S->d_pos_b, S->d_first, S->d_out, S->d_off,
-                                 S->d_state, S->d_chunk, S->ksize);
+                                 S->d_state, S->d_chunk, S->k_max);
     YG_CUDA(ctx, cudaGetLastError());
     ctx->tm.n_kernel_launches += 5;
     ctx->tm.n_library_launches += 4;
@@ -376,18 +398,41 @@ int sq_chunk(ygpu_ctx* ctx, StreamState* S, const uint8_t* p, uint64_t n) {
         for (uint64_t r = 0; r < c.n_rec; r++) S->name_off.push_back(base + S->h_name_start[r]);
     }
 
-    if (c.n_out < (uint64_t)S->ksize) return 0;
     YG_CUDA(ctx, cudaMemsetAsync(S->d_out + c.n_out, 0, YG_SKETCH_PAD, st));
-    uint64_t m = 0, n_kmers = 0;
-    YG_CHECK(ygpu_sketch_hash_device(ctx, S->d_out, c.n_out, S->d_off, (uint32_t)(c.n_rec + 1), S->ksize, S->max_hash, S->seed,
-                                     S->ev[3], &m, &n_kmers));
-    S->st.ms_hash += ev_ms(S->ev[2], S->ev[3]);
-    S->st.n_kmers += n_kmers;
-    if (m == 0) return 0;
-    YG_CHECK(sq_merge(ctx, S, m, (uint32_t)(rec_before - 1)));
+    // every k on the same buffer; the kept hashes of all of them are merged once.  Each hashing call records its end in ev[3]
+    // or ev[0] in turn (ev[0] is free once ms_h2d is read), so ms_hash takes every hashing kernel, with the packing of the
+    // previous size's kept hashes, and no host round trip is added per k; the last end -> ev[4] is the last packing + merge.
+    cudaEvent_t t0 = S->ev[2];
+    uint64_t added = 0;
+    for (int ki = 0; ki < S->n_k; ki++) {
+        const int k = S->ks[ki];
+        if (c.n_out < (uint64_t)k) continue;
+        uint64_t m = 0, n_kmers = 0;
+        cudaEvent_t done = t0 == S->ev[3] ? S->ev[0] : S->ev[3];
+        const uint64_t first_new = ysq_first_new(k, n_carry);
+        YG_CHECK(ygpu_sketch_hash_device(ctx, S->d_out, c.n_out, S->d_off, (uint32_t)(c.n_rec + 1), k, S->max_hash, S->seed,
+                                         first_new, done, &m, &n_kmers));
+        if (first_new) {            // the valid windows inside the carried bases were counted with the previous chunk
+            uint64_t old = 0;
+            for (uint64_t p = 0; p < first_new; p++) {
+                bool ok = true;
+                for (int q = 0; q < k && ok; q++) ok = ysk_code(carry_in[p + q]) < 4;
+                old += ok;
+            }
+            n_kmers -= old;
+        }
+        S->st.ms_hash += ev_ms(t0, done);
+        S->st.n_kmers += n_kmers;
+        S->n_kmers_k[ki] += n_kmers;
+        if (m) YG_CHECK(sq_add(ctx, S, added, m, (uint32_t)(rec_before - 1), ki));
+        added += m;
+        t0 = done;
+    }
+    if (added == 0) return 0;
+    YG_CHECK(sq_merge(ctx, S, added));
     YG_CUDA(ctx, cudaEventRecord(S->ev[4], st));
     YG_CUDA(ctx, cudaEventSynchronize(S->ev[4]));
-    S->st.ms_merge += ev_ms(S->ev[3], S->ev[4]);
+    S->st.ms_merge += ev_ms(t0, S->ev[4]);
     return 0;
 }
 
@@ -431,9 +476,14 @@ void ygpu_stream_release(ygpu_ctx* ctx) {
     ctx->seq_stream = nullptr;
 }
 
-extern "C" int ygpu_stream_begin(ygpu_ctx* ctx, int ksize, uint64_t max_hash, uint32_t seed, int mode) {
+extern "C" int ygpu_stream_begin_k(ygpu_ctx* ctx, const int* ksizes, int n_k, uint64_t max_hash, uint32_t seed, int mode) {
     if (!ctx) return YGPU_ERR_ARG;
-    if (ksize < 1 || ksize > YSQ_CARRY_MAX) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_stream_begin: ksize %d outside [1, %d]", ksize, YSQ_CARRY_MAX);
+    if (!ksizes || n_k < 1 || n_k > YSQ_MAX_K) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_stream_begin: %d k-mer sizes (1 to %d)", n_k, YSQ_MAX_K);
+    for (int i = 0; i < n_k; i++) {
+        if (ksizes[i] < 1 || ksizes[i] > YSQ_CARRY_MAX) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_stream_begin: ksize %d outside [1, %d]", ksizes[i], YSQ_CARRY_MAX);
+        for (int j = 0; j < i; j++)
+            if (ksizes[j] == ksizes[i]) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_stream_begin: ksize %d given twice", ksizes[i]);
+    }
     if (mode != YGPU_STREAM_WHOLE && mode != YGPU_STREAM_PER_RECORD) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_stream_begin: unknown mode %d", mode);
     YG_CUDA(ctx, cudaSetDevice(ctx->device));
     StreamState* S = sq_get(ctx);
@@ -446,7 +496,13 @@ extern "C" int ygpu_stream_begin(ygpu_ctx* ctx, int ksize, uint64_t max_hash, ui
     S->cap = ctx->stream_chunk_bytes;
     if (!S->h_stage) YG_CUDA(ctx, cudaHostAlloc((void**)&S->h_stage, S->cap, cudaHostAllocDefault));
     YG_CHECK(sq_alloc_chunk(ctx, S));
-    S->ksize = ksize;
+    S->n_k = n_k;
+    S->k_max = 0;
+    for (int i = 0; i < n_k; i++) {
+        S->ks[i] = ksizes[i];
+        S->k_max = std::max(S->k_max, ksizes[i]);
+        S->n_kmers_k[i] = 0;
+    }
     S->max_hash = max_hash;
     S->seed = seed;
     S->mode = mode;
@@ -460,6 +516,10 @@ extern "C" int ygpu_stream_begin(ygpu_ctx* ctx, int ksize, uint64_t max_hash, ui
     S->h_state->n_records = 0;
     S->active = true;
     return 0;
+}
+
+extern "C" int ygpu_stream_begin(ygpu_ctx* ctx, int ksize, uint64_t max_hash, uint32_t seed, int mode) {
+    return ygpu_stream_begin_k(ctx, &ksize, 1, max_hash, seed, mode);
 }
 
 extern "C" int ygpu_stream_feed(ygpu_ctx* ctx, const uint8_t* bytes, uint64_t n) {
@@ -524,46 +584,72 @@ extern "C" int ygpu_stream_end_file(ygpu_ctx* ctx) {
     return 0;
 }
 
-extern "C" int ygpu_stream_finish(ygpu_ctx* ctx, ygpu_sketch_result* out, ygpu_stream_stats* stats, char** names,
-                                  uint64_t** name_offsets, uint64_t* n_names) {
+extern "C" int ygpu_stream_finish_k(ygpu_ctx* ctx, ygpu_sketch_result* out, ygpu_stream_stats* stats, char** names,
+                                    uint64_t** name_offsets, uint64_t* n_names) {
     StreamState* S;
     YG_CHECK(sq_active(ctx, &S, "ygpu_stream_finish"));
     if (!out || !names || !name_offsets || !n_names) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_stream_finish: bad argument");
     if (S->file_started || S->staged) YG_CHECK(ygpu_stream_end_file(ctx));
     YG_CUDA(ctx, cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    memset(out, 0, sizeof *out);
+    const int n_k = S->n_k;
+    memset(out, 0, n_k * sizeof *out);
     *names = nullptr;
     *name_offsets = nullptr;
     *n_names = 0;
     const uint64_t n_rec = S->h_state->n_records;
     const uint64_t ns = S->mode == YGPU_STREAM_WHOLE ? 1 : n_rec;
-    if (ns >= (1ull << 32)) return sq_fail(ctx, S, YGPU_ERR_ARG, "ygpu_stream_finish: more than 2^32 records");
+    if (ns * n_k >= (1ull << 32)) {
+        if (n_k == 1) return sq_fail(ctx, S, YGPU_ERR_ARG, "ygpu_stream_finish: more than 2^32 records");
+        return sq_fail(ctx, S, YGPU_ERR_ARG, "ygpu_stream_finish: records x k-mer sizes reach 2^32");
+    }
+    // the resident sketch is in (cid, hash) order, cid = record * n_k + k index: k index i's entries, taken in that order,
+    // are its sketch in (record, hash) order
     const uint64_t nd = S->n_res;
-    out->offsets = (uint64_t*)calloc(ns + 1, sizeof(uint64_t));
-    out->hashes = (uint64_t*)malloc(std::max<uint64_t>(nd, 1) * sizeof(uint64_t));
-    out->abundances = (uint32_t*)malloc(std::max<uint64_t>(nd, 1) * sizeof(uint32_t));
     std::vector<uint64_t> v(nd);
-    if (!out->offsets || !out->hashes || !out->abundances) { ygpu_sketch_result_free(out); return sq_fail(ctx, S, YGPU_ERR_NOMEM, "out of host memory"); }
-    out->n_sketches = (uint32_t)ns;
-    out->n_kmers = S->st.n_kmers;
     if (nd) {
-        YG_CUDA(ctx, cudaMemcpyAsync(out->hashes, S->d_rh, nd * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
         YG_CUDA(ctx, cudaMemcpyAsync(v.data(), S->d_rv, nd * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
         YG_CUDA(ctx, cudaStreamSynchronize(st));
     }
-    for (uint64_t i = 0; i < nd; i++) {
-        out->abundances[i] = (uint32_t)v[i];
-        out->offsets[(v[i] >> 32) + 1]++;
+    std::vector<uint64_t> count(n_k, 0);
+    for (uint64_t i = 0; i < nd; i++) count[(v[i] >> 32) % n_k]++;
+    bool ok = true;
+    for (int ki = 0; ki < n_k; ki++) {
+        out[ki].offsets = (uint64_t*)calloc(ns + 1, sizeof(uint64_t));
+        out[ki].hashes = (uint64_t*)malloc(std::max<uint64_t>(count[ki], 1) * sizeof(uint64_t));
+        out[ki].abundances = (uint32_t*)malloc(std::max<uint64_t>(count[ki], 1) * sizeof(uint32_t));
+        ok = ok && out[ki].offsets && out[ki].hashes && out[ki].abundances;
+        out[ki].n_sketches = (uint32_t)ns;
+        out[ki].n_kmers = S->n_kmers_k[ki];
     }
-    for (uint64_t s = 0; s < ns; s++) out->offsets[s + 1] += out->offsets[s];
+    if (!ok) {
+        for (int ki = 0; ki < n_k; ki++) ygpu_sketch_result_free(&out[ki]);
+        return sq_fail(ctx, S, YGPU_ERR_NOMEM, "out of host memory");
+    }
+    // one k: the hashes go straight into the result; several: through a host copy that is split by k index
+    std::vector<uint64_t> h(n_k > 1 ? nd : 0);
+    if (nd) {
+        YG_CUDA(ctx, cudaMemcpyAsync(n_k > 1 ? h.data() : out[0].hashes, S->d_rh, nd * sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
+        YG_CUDA(ctx, cudaStreamSynchronize(st));
+    }
+    std::fill(count.begin(), count.end(), 0);
+    for (uint64_t i = 0; i < nd; i++) {
+        const uint64_t cid = v[i] >> 32;
+        ygpu_sketch_result& o = out[cid % n_k];
+        const uint64_t j = count[cid % n_k]++;
+        if (n_k > 1) o.hashes[j] = h[i];
+        o.abundances[j] = (uint32_t)v[i];
+        o.offsets[cid / n_k + 1]++;
+    }
+    for (int ki = 0; ki < n_k; ki++)
+        for (uint64_t s = 0; s < ns; s++) out[ki].offsets[s + 1] += out[ki].offsets[s];
     const uint64_t nn = S->name_off.size();
     if (nn) {
         *names = (char*)malloc(std::max<size_t>(S->names.size(), 1));
         *name_offsets = (uint64_t*)malloc((nn + 1) * sizeof(uint64_t));
         if (!*names || !*name_offsets) {
             free(*names); free(*name_offsets); *names = nullptr; *name_offsets = nullptr;
-            ygpu_sketch_result_free(out);
+            for (int ki = 0; ki < n_k; ki++) ygpu_sketch_result_free(&out[ki]);
             return sq_fail(ctx, S, YGPU_ERR_NOMEM, "out of host memory");
         }
         memcpy(*names, S->names.data(), S->names.size());
@@ -576,4 +662,12 @@ extern "C" int ygpu_stream_finish(ygpu_ctx* ctx, ygpu_sketch_result* out, ygpu_s
     S->active = false;
     S->n_res = 0;
     return 0;
+}
+
+extern "C" int ygpu_stream_finish(ygpu_ctx* ctx, ygpu_sketch_result* out, ygpu_stream_stats* stats, char** names,
+                                  uint64_t** name_offsets, uint64_t* n_names) {
+    StreamState* S;
+    YG_CHECK(sq_active(ctx, &S, "ygpu_stream_finish"));
+    if (S->n_k != 1) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_stream_finish: the stream has %d k-mer sizes; finish it with ygpu_stream_finish_k", S->n_k);
+    return ygpu_stream_finish_k(ctx, out, stats, names, name_offsets, n_names);
 }

@@ -22,6 +22,7 @@ enum { YSQ_ROLE_DROP = 0, YSQ_ROLE_SEQ = 1, YSQ_ROLE_HEADER = 2 };
 // per-byte flags: the byte goes to the hashing buffer / starts a record (it is written as the '\n' separator) / is a name byte
 enum { YSQ_F_SEQ = 1, YSQ_F_REC = 2, YSQ_F_NAME = 4 };
 constexpr int YSQ_CARRY_MAX = 256;             // room for k - 1 bases at the largest k
+constexpr int YSQ_MAX_K = 8;                    // k-mer sizes one stream hashes
 
 // Carried from one chunk to the next (and from one file to the next): state, never partial lines.
 struct ysq_state {
@@ -32,7 +33,7 @@ struct ysq_state {
     uint64_t first_bad_empty; // FASTQ: first empty line at a place where '@' or '+' is due (~0: none)
     uint32_t fmt;             // YSQ_FASTA / YSQ_FASTQ of the current file
     uint32_t open_first;      // first byte of the open line, 0 while it has none
-    uint32_t n_carry;         // bases of the open record carried into the next chunk (<= k - 1)
+    uint32_t n_carry;         // bases of the open record carried into the next chunk (<= k_max - 1)
     uint32_t _pad;
     uint8_t carry[YSQ_CARRY_MAX];
 };
@@ -72,8 +73,9 @@ YSQ_HD uint32_t ysq_byte_flags(uint8_t c, int role, bool is_first, bool want_nam
 }
 YSQ_HD uint8_t ysq_out_byte(uint8_t c, uint32_t flags) { return (flags & YSQ_F_REC) ? (uint8_t)'\n' : c; }
 
-// The bases carried into the next chunk: the last min(k - 1, bases of the open record) bytes of the compacted buffer.
-// open_begin = where the open record's bases start in it (just behind its separator; 0 when it began in an earlier chunk).
+// The bases carried into the next chunk: the last min(k - 1, bases of the open record) bytes of the compacted buffer, k the
+// largest k-mer size of the stream.  open_begin = where the open record's bases start in it (just behind its separator; 0 when
+// it began in an earlier chunk).
 YSQ_HD uint64_t ysq_carry_begin(uint64_t n_out, uint64_t open_begin, int k) {
     const uint64_t keep = (uint64_t)(k - 1);
     const uint64_t b = n_out > keep ? n_out - keep : 0;
@@ -92,6 +94,15 @@ YSQ_HD void ysq_advance(ysq_state* s, uint64_t n_nl, uint64_t n_rec, uint32_t la
     s->line += n_nl;
     s->n_records += n_rec;
 }
+
+// Whether the window of k bases at start p of a chunk's compacted buffer, which the chunk's n_carry carried bases lead, is new:
+// it is not when it lies entirely inside the carried bases, which the previous chunk hashed already.  That happens only for a
+// k below the largest of the stream (the carry is up to k_max - 1 bases); for one k, n_carry <= k - 1 and every window is new.
+YSQ_HD bool ysq_window_new(uint64_t p, int k, uint64_t n_carry) { return p + (uint64_t)k > n_carry; }
+// The first start whose window is new: 0 unless the carried bases hold a whole window.  The hashing launch passes it to the
+// kernels as the start of the chunk's first sketch range; ysq_window_new(p) == (p >= ysq_first_new).  The valid windows that
+// start before it (all inside the carried bases) are taken out of the chunk's count with ysq_carried_windows.
+YSQ_HD uint64_t ysq_first_new(int k, uint64_t n_carry) { return n_carry >= (uint64_t)k ? n_carry - (uint64_t)k + 1 : 0; }
 
 // End of a FASTQ file: 0 = fine; 1 = the line count (trailing empty lines dropped) is not a multiple of 4, *value = that
 // count; 2 = a record breaks the structure, *value = the 1-based number of its first line.

@@ -231,8 +231,12 @@ __global__ void __launch_bounds__(SK_NT) k_sketch_hash_packed2(const uint8_t* __
 // K7 on a device buffer: d_bases[0, n_bases) followed by SK_PAD zero bytes (16-byte aligned), d_off[0 .. n_sketches] on the
 // device.  Leaves the m survivors in the context's scratch (sketch_survivors) and the valid windows in *n_kmers; records
 // ev_done behind the hashing kernel.  ygpu_sketch_sequences and the stream (seq_stream.cu) both hash through here.
-int ygpu_sketch_hash_device(ygpu_ctx* ctx, const uint8_t* d_bases, uint64_t n_bases, const uint64_t* d_off, uint32_t n_sketches,
-                            int ksize, uint64_t max_hash, uint32_t seed, cudaEvent_t ev_done, uint64_t* m, uint64_t* n_kmers) {
+// first_new > 0 (the stream's window rule, ysq_first_new): d_off[0] holds it during the launch, so that no window starting
+// before it is kept -- the kernels keep a survivor only inside its sketch range -- and is 0 again after; such windows are
+// still in *n_kmers, the caller takes them out.
+int ygpu_sketch_hash_device(ygpu_ctx* ctx, const uint8_t* d_bases, uint64_t n_bases, uint64_t* d_off, uint32_t n_sketches,
+                            int ksize, uint64_t max_hash, uint32_t seed, uint64_t first_new, cudaEvent_t ev_done, uint64_t* m,
+                            uint64_t* n_kmers) {
     SketchScratch* S = sk_scratch(ctx);
     cudaStream_t st = ctx->stream;
     YG_CHECK(dev_alloc(ctx, &S->d_cnt, 2));
@@ -248,6 +252,7 @@ int ygpu_sketch_hash_device(ygpu_ctx* ctx, const uint8_t* d_bases, uint64_t n_ba
         YG_CHECK(dev_alloc(ctx, &S->d_key, cap));
         YG_CHECK(dev_alloc(ctx, &S->d_sid, cap));
         YG_CUDA(ctx, cudaMemsetAsync(S->d_cnt, 0, 2 * sizeof(unsigned long long), st));
+        if (first_new) YG_CUDA(ctx, cudaMemcpyAsync(d_off, &first_new, sizeof first_new, cudaMemcpyHostToDevice, st));
         if (ksize <= 32 && ctx->sketch_kernel != 2)
             k_sketch_hash_packed<<<grid, SK_NT, 0, st>>>(d_bases, n_bases, d_off, n_sketches, ksize, seed, max_hash, S->d_key, S->d_sid, cap, S->d_cnt);
         else if (ksize <= 64 && ctx->sketch_kernel != 2)
@@ -257,6 +262,7 @@ int ygpu_sketch_hash_device(ygpu_ctx* ctx, const uint8_t* d_bases, uint64_t n_ba
         YG_CUDA(ctx, cudaGetLastError());
         ctx->tm.n_kernel_launches++;
         YG_CUDA(ctx, cudaEventRecord(ev_done, st));
+        if (first_new) YG_CUDA(ctx, cudaMemsetAsync(d_off, 0, sizeof(uint64_t), st));
         YG_CUDA(ctx, cudaMemcpyAsync(h_cnt, S->d_cnt, sizeof h_cnt, cudaMemcpyDeviceToHost, st));
         YG_CUDA(ctx, cudaStreamSynchronize(st));
         if (h_cnt[0] <= cap) break;
@@ -339,7 +345,7 @@ extern "C" int ygpu_sketch_sequences(ygpu_ctx* ctx, const uint8_t* bases, uint64
     YG_CUDA(ctx, cudaEventRecord(ctx->ev[1], st));
 
     uint64_t m = 0, n_kmers = 0;
-    YG_CHECK(ygpu_sketch_hash_device(ctx, S->d_bases, n_bases, S->d_off, n_sketches, ksize, max_hash, seed, ctx->ev[2], &m, &n_kmers));
+    YG_CHECK(ygpu_sketch_hash_device(ctx, S->d_bases, n_bases, S->d_off, n_sketches, ksize, max_hash, seed, 0, ctx->ev[2], &m, &n_kmers));
     ctx->tm.ms_h2d = elapsed(ctx, 0, 1);
     ctx->tm.ms_sketch = elapsed(ctx, 1, 2);
     out->n_kmers = n_kmers;

@@ -218,10 +218,11 @@ def write_signature(path: str, name: str, mins: Sequence[int], ksize: int = 31,
 def write_signatures(path: str, sketches: Sequence[dict], ksize: int = 31, max_hash: int = MAX_HASH_SCALED_1000) -> None:
     """One JSON signature file holding several sketches (what ``sourmash sketch dna -o x.sig`` writes for several
     records); gzip when ``path`` ends in .gz.  ``sketches``: dicts with ``name``, ``mins`` and optional ``abundances``,
-    ``filename``."""
+    ``filename`` and ``ksize`` (default: the argument), one JSON record each, in order."""
     recs = []
     for sk in sketches:
-        recs.extend(json.loads(signature_json(sk["name"], sk["mins"], ksize, sk.get("abundances"), max_hash, sk.get("filename", ""))))
+        recs.extend(json.loads(signature_json(sk["name"], sk["mins"], sk.get("ksize", ksize), sk.get("abundances"), max_hash,
+                                              sk.get("filename", ""))))
     data = json.dumps(recs, separators=(",", ":")).encode()
     if path.endswith(".gz"):
         with gzip.open(path, "wb", compresslevel=1) as f:
@@ -235,7 +236,8 @@ def write_sig_zip(zip_path: str, sketches: Sequence[dict], ksize: int = 31,
                   max_hash: int = MAX_HASH_SCALED_1000) -> None:
     """Write a sourmash-style zip database (manifest + signatures/<md5>.sig.gz).
 
-    ``sketches``: dicts with ``name``, ``mins`` and optional ``abundances``.
+    ``sketches``: dicts with ``name``, ``mins`` and optional ``abundances``, ``filename`` and ``ksize`` (default: the
+    argument); one signature file and one manifest row each, in order.
     """
     scaled = int(round((2 ** 64 - 1) / max_hash)) if max_hash else 0
     with zipfile.ZipFile(zip_path, "w", zipfile.ZIP_STORED) as z:
@@ -244,11 +246,12 @@ def write_sig_zip(zip_path: str, sketches: Sequence[dict], ksize: int = 31,
         w = csv.writer(buf, lineterminator="\n")
         w.writerow(MANIFEST_COLUMNS)
         for sk in sketches:
-            text = signature_json(sk["name"], sk["mins"], ksize, sk.get("abundances"), max_hash,
+            k = sk.get("ksize", ksize)
+            text = signature_json(sk["name"], sk["mins"], k, sk.get("abundances"), max_hash,
                                   sk.get("filename", ""))
-            md5 = compute_md5sum(ksize, [int(x) for x in sk["mins"]])
+            md5 = compute_md5sum(k, [int(x) for x in sk["mins"]])
             loc = f"signatures/{md5}.sig.gz"
             z.writestr(loc, gzip.compress(text.encode(), compresslevel=1))
-            w.writerow([loc, md5, md5[:8], ksize, "DNA", 0, scaled, len(sk["mins"]),
+            w.writerow([loc, md5, md5[:8], k, "DNA", 0, scaled, len(sk["mins"]),
                         1 if sk.get("abundances") is not None else 0, sk["name"], sk.get("filename", "")])
         z.writestr(MANIFEST_NAME, buf.getvalue())

@@ -33,12 +33,17 @@ def _context() -> _lib.GpuContext:
     return _ctx
 
 
-def add_cli_arguments(parser, infile_help: str, nargs=None) -> None:
-    """The four options both `yacht sketch` sub-commands take (names and defaults of the reference's wrappers)."""
+def add_cli_arguments(parser, infile_help: str, nargs=None, multi_kmer: bool = False) -> None:
+    """The four options both `yacht sketch` sub-commands take (names and defaults of the reference's wrappers).
+    With `multi_kmer`, --kmer takes one or more values and is always a list (default [31])."""
     kw = {"nargs": nargs} if nargs else {}
     parser.add_argument("--infile", help=infile_help, required=True, **kw)
-    for flag, default, text in (("--kmer", 31, "K-mer size."), ("--scaled", 1000, "Scaled factor.")):
-        parser.add_argument(flag, type=int, default=default, help=text)
+    if multi_kmer:
+        parser.add_argument("--kmer", type=int, nargs="+", default=[31],
+                            help="K-mer size(s). Several distinct sizes are sketched in one pass into one output file.")
+    else:
+        parser.add_argument("--kmer", type=int, default=31, help="K-mer size.")
+    parser.add_argument("--scaled", type=int, default=1000, help="Scaled factor.")
     parser.add_argument("--outfile", help="Output file name.", required=True)
 
 
@@ -119,12 +124,14 @@ def _reader(path: str, bufs, free: "queue.Queue", full: "queue.Queue") -> None:
         full.put((None, e))
 
 
-def sketch_stream(paths: Sequence[str], ksize: int, scaled: int, per_record: bool = False, seed: int = SEED,
+def sketch_stream(paths: Sequence[str], ksize, scaled: int, per_record: bool = False, seed: int = SEED,
                   stats: Optional[dict] = None):
     """Sketch the files one after another through the device stream (ygpu_stream_*): the text is read and gunzipped on a
     reader thread into STREAM_BUFFERS page-locked buffers and parsed, hashed and accumulated on the device, so host memory
     stays at a few buffers plus the sketch whatever the size of the input.
     Returns ([(mins, abundances)], names): one sketch of all records, or with `per_record` one per record with its name.
+    With a sequence of k-mer sizes for `ksize` the input is still read and parsed once, and the result is
+    ([[(mins, abundances)] per k, in the order given], names).
     `stats`, when given, receives the stream's counters and device times (ygpu_stream_stats)."""
     ctx = _context()
     ctx.stream_begin(ksize, max_hash_for_scaled(scaled), seed, per_record)
@@ -150,7 +157,11 @@ def sketch_stream(paths: Sequence[str], ksize: int, scaled: int, per_record: boo
                 free.put(None)
                 th.join()
             ctx.stream_end_file(path)
-        hashes, abund, offsets, names, st = ctx.stream_finish(paths[-1] if paths else None)
+        if isinstance(ksize, (int, np.integer)):
+            hashes, abund, offsets, names, st = ctx.stream_finish(paths[-1] if paths else None)
+            per_k = None
+        else:
+            per_k, names, st = ctx.stream_finish(paths[-1] if paths else None)
         if stats is not None:
             stats.update(st)
     finally:
@@ -158,8 +169,11 @@ def sketch_stream(paths: Sequence[str], ksize: int, scaled: int, per_record: boo
             release()
     # names come back as bytes; decoding them raises on invalid UTF-8 as the record path's reader does
     names = [b.decode() for b in names] if names else []
-    sketches = [(hashes[int(offsets[s]):int(offsets[s + 1])], abund[int(offsets[s]):int(offsets[s + 1])]) for s in range(len(offsets) - 1)]
-    return sketches, names
+    split = lambda hashes, abund, offsets: [(hashes[int(offsets[s]):int(offsets[s + 1])], abund[int(offsets[s]):int(offsets[s + 1])])
+                                            for s in range(len(offsets) - 1)]
+    if per_k is None:
+        return split(hashes, abund, offsets), names
+    return [split(h, a, o) for h, a, o, _ in per_k], names
 
 
 def sketch_record_groups(groups: Sequence[Sequence[bytes]], ksize: int, scaled: int, seed: int = SEED):
@@ -270,7 +284,8 @@ def sketch_files(paths: Sequence[str], ksize: int, scaled: int, singleton: bool 
 
 
 def write_sketches(outfile: str, sketches: Sequence[dict], ksize: int, scaled: int) -> None:
-    """``.zip`` -> a sourmash zip database (manifest + signatures/<md5>.sig.gz); anything else -> one JSON signature file."""
+    """``.zip`` -> a sourmash zip database (manifest + signatures/<md5>.sig.gz); anything else -> one JSON signature file.
+    A sketch dict's own ``"ksize"`` takes the place of `ksize`."""
     max_hash = max_hash_for_scaled(scaled)
     if outfile.endswith(".zip"):
         sigio.write_sig_zip(outfile, sketches, ksize, max_hash)

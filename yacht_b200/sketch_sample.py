@@ -3,7 +3,9 @@
 
 Same command line as the reference's wrapper (src/yacht/sketch_sample.py): one or two FASTA/FASTQ files in, ONE sketch with
 abundances out.  For paired-end input the reference first concatenates both files into a temporary file (:42-57); here the
-records of both files simply go into the same sketch.
+records of both files simply go into the same sketch.  ``--kmer`` may also name several k-mer sizes (``--kmer 21 31 51``):
+the input is then read once and the output holds one signature per size, in the order given, each what a run with that
+size alone writes (``sourmash sketch dna -p k=21,k=31,k=51,...`` makes such files too).
 """
 import argparse
 
@@ -12,7 +14,8 @@ from .utils import _log
 
 
 def add_arguments(parser):
-    sketch.add_cli_arguments(parser, infile_help="Input FASTA/Q file(s). For paired-end reads, provide two files.", nargs="+")
+    sketch.add_cli_arguments(parser, infile_help="Input FASTA/Q file(s). For paired-end reads, provide two files.", nargs="+",
+                             multi_kmer=True)
 
 
 def sketch_reads(infiles, kmer, scaled, outfile):
@@ -27,13 +30,29 @@ def sketch_reads(infiles, kmer, scaled, outfile):
     sketch.write_sketches(outfile, [dict(name="", filename=infiles[0], mins=mins, abundances=abundances)], kmer, scaled)
 
 
+def sketch_reads_multik(infiles, kmers, scaled, outfile):
+    """`sketch_reads` at several k-mer sizes: the files are streamed through the device parser once, every size is hashed
+    on the same parsed text, and `outfile` holds one signature per size, in the order of `kmers`."""
+    per_k, _ = sketch.sketch_stream(list(infiles), list(kmers), scaled)
+    sketches = [dict(name="", filename=infiles[0], mins=mins, abundances=abundances, ksize=k) for k, [(mins, abundances)] in zip(kmers, per_k)]
+    sketch.write_sketches(outfile, sketches, kmers[0], scaled)
+
+
 def main(args):
     files = list(args.infile)
     if len(files) not in (1, 2):
         raise ValueError("Please provide either one file for single-end reads or two files for paired-end reads.")
+    # the command line gives a list; a caller that builds the namespace itself may still pass one int
+    kmers = list(args.kmer) if isinstance(args.kmer, (list, tuple)) else [args.kmer]
+    dup = sorted({k for k in kmers if kmers.count(k) > 1})
+    if dup:
+        raise ValueError(f"--kmer: k-mer size(s) {', '.join(map(str, dup))} given more than once.")
     kind = "a single-end FASTA/Q file" if len(files) == 1 else "paired-end FASTA/Q files"
     _log("INFO", f"Starting sketching {kind}: {' '.join(files)}")
-    sketch_reads(files, args.kmer, args.scaled, args.outfile)
+    if len(kmers) == 1:
+        sketch_reads(files, kmers[0], args.scaled, args.outfile)
+    else:
+        sketch_reads_multik(files, kmers, args.scaled, args.outfile)
     _log("SUCCESS", "Successfully sketched!!")
 
 
