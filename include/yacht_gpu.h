@@ -161,7 +161,10 @@ int ygpu_set_option(ygpu_ctx* ctx, const char* name, int64_t value);
 /* Read-only state of the last count call (ygpu_pairwise_flag / _device): "last_count_kernel" (1 = dense row accumulator,
  * 2 = warp per row), "last_count_overflow_rows" (rows the warp kernel deferred to the dense kernel), and the dense kernel's
  * accumulator geometry "last_count_tile_w" (columns per tile), "last_count_n_tiles" and "last_count_u16" (1 = packed 16-bit
- * counters).  An unknown name fails with YGPU_ERR_ARG.                                                                    */
+ * counters).  Read-only state of the last ygpu_build_index on the partition path: "last_group2_grid" and "last_group_grid"
+ * (CTAs of the k2_group2 and of the general k2_group launch; CTA c groups final buckets c, c + grid, ...) and
+ * "last_big_chunks" (sorted chunks of the oversized-bucket route); each is 0 when that kernel or route did not run.
+ * An unknown name fails with YGPU_ERR_ARG.                                                                                 */
 int ygpu_get_option(ygpu_ctx* ctx, const char* name, int64_t* out);
 
 /* ---- ingest (host side of the path) ------------------------------------------------------------ */

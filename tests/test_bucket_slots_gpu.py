@@ -6,37 +6,16 @@ Covered here: synthetic databases that take the slotted path end to end (train s
 exclusive-hash counts against the CPU oracles); a final bucket that fills its slot exactly (slotted) and one a word over it (level-2
 retry), with both grouping kernels; a top level-1 digit over its slot (full retry).  The crafted databases of
 test_group2_edges_gpu.py overflow their level-2 slots, so they keep covering the exact layout's bucket boundaries."""
-import math
-
 import numpy as np
 import pytest
 
 from oracle import train_oracle as to
-from test_group2_edges_gpu import A_TARGET, bucket_db
+from harness.group_routes import bucket_db, plan
 from yacht_b200 import synth
 
 pytestmark = pytest.mark.gpu
 
 THR = 0.95 ** 31
-SC_TILE = 4096          # index_msd.cu: words per scatter tile
-
-
-def plan(hashes, n):
-    """msd_build's plan: (hb, d1, d2, C1, C2)."""
-    T = len(hashes)
-    maxkey = int(hashes.max())
-    hb = max(1, maxkey.bit_length())
-    D = 0
-    while D < hb and D < 22 and T // ((maxkey >> (hb - D)) + 1 if D else 1) > A_TARGET:
-        D += 1
-    d1 = max(D if D <= 8 else (D + 1) // 2, hb + (n - 1).bit_length() - 64)      # packing: hb - d1 + gb <= 64
-    d2 = max(0, D - d1)
-
-    def cap(bits, f, add):       # f * (expected words of a full bucket) + add, rounded up to 16 words
-        mean = float(T) * 2.0 ** (hb - bits) / (float(maxkey) + 1.0)
-        return (math.ceil(f * mean + add) + 15) // 16 * 16
-
-    return hb, d1, d2, cap(d1, 1.02, SC_TILE), cap(d1 + d2, 1.25, 64.0)
 
 
 def build(ctx, hashes, offsets):

@@ -10,44 +10,10 @@ the sharded step's launch, whose grid is always SMs x CTAs per SM, is exercised 
 import numpy as np
 import pytest
 
+from harness.group_routes import bucket_db
 from oracle import train_oracle as to
 
 pytestmark = pytest.mark.gpu
-
-A_TARGET = 900          # index_msd.cu: the plan takes the fewest leading hash bits D with T / 2^D <= A_TARGET
-N_GENOMES = 211         # prime: the members of a group, g0 + 7 k mod N, are distinct genomes
-
-
-def bucket_db(hb, D, sizes, seed):
-    """Sketches whose words fall into final bucket b = hash >> (hb - D) exactly sizes[b] times.  Inside a bucket, hashes
-    are held by 1..12 genomes (mostly 1 or 2, as in real databases), and about 1 % of the words repeat their neighbour's
-    (hash, genome): in-sketch duplicates."""
-    assert len(sizes) == 1 << D and sizes[-1] > 0          # the last bucket sets the hash width hb
-    T = int(sum(sizes))
-    assert A_TARGET * (1 << D) >= T > A_TARGET * (1 << (D - 1)), "the plan would pick another bucket count"
-    rng = np.random.default_rng(seed)
-    shift = hb - D
-    hs, gs = [], []
-    for b, m in enumerate(sizes):
-        if not m:
-            continue
-        L = rng.choice([1, 2, 3, 4, 6, 12], size=m, p=[0.60, 0.25, 0.08, 0.04, 0.02, 0.01])
-        L = L[:np.searchsorted(np.cumsum(L), m) + 1]
-        L[-1] -= int(L.sum()) - m
-        grp = np.repeat(np.arange(len(L)), L)
-        rank = np.arange(m) - np.repeat(np.cumsum(L) - L, L)
-        h = (np.uint64(b) << np.uint64(shift)) + rng.integers(0, 1 << shift, size=len(L), dtype=np.uint64)[grp]
-        g = (rng.integers(0, N_GENOMES, size=len(L))[grp] + 7 * rank) % N_GENOMES
-        dup = np.flatnonzero(rng.random(m) < 0.01)
-        dup = dup[dup > 0]
-        h[dup], g[dup] = h[dup - 1], g[dup - 1]
-        hs.append(h)
-        gs.append(g)
-    h, g = np.concatenate(hs), np.concatenate(gs)
-    order = np.lexsort((h, g))
-    offsets = np.zeros(N_GENOMES + 1, dtype=np.uint64)
-    offsets[1:] = np.cumsum(np.bincount(g, minlength=N_GENOMES))
-    return h[order], offsets
 
 
 def check_both_kernels(ctx, hashes, offsets):

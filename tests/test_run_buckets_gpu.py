@@ -22,8 +22,8 @@ import pytest
 
 from oracle import run_oracle as ro
 from oracle import train_oracle as to
-from test_bucket_slots_gpu import level2_db, plan
-from test_group2_edges_gpu import bucket_db
+from harness.group_routes import bucket_db, plan
+from test_bucket_slots_gpu import level2_db
 from test_run_parity_gpu import _check_counts
 from yacht_b200 import synth
 from yacht_b200._lib import YgpuError

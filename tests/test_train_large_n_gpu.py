@@ -239,5 +239,8 @@ def test_sharded_step_past_2pow20(dbs):
 
 
 def test_get_option_rejects_unknown_names(gpu_ctx):
-    with pytest.raises(_lib.YgpuError, match=r"\(-3\)"):
-        gpu_ctx.get_option("count_kernel")
+    for name in ("count_kernel", "group_kernel", "group_grid", "last_group3_grid", "last_big_buckets"):
+        with pytest.raises(_lib.YgpuError, match=r"\(-3\)"):
+            gpu_ctx.get_option(name)
+    for name in ("last_group2_grid", "last_group_grid", "last_big_chunks"):
+        assert gpu_ctx.get_option(name) >= 0

@@ -347,7 +347,7 @@ class GpuContext:
         self._check(self.lib.ygpu_set_option(self.h, name.encode(), int(value)), "ygpu_set_option")
 
     def get_option(self, name: str) -> int:
-        """Read-only state of the last count call (include/yacht_gpu.h: ygpu_get_option)."""
+        """Read-only state of the last count call and of the last index build (include/yacht_gpu.h: ygpu_get_option)."""
         v = ctypes.c_int64(0)
         self._check(self.lib.ygpu_get_option(self.h, name.encode(), ctypes.byref(v)), "ygpu_get_option")
         return int(v.value)

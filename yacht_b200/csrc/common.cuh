@@ -63,6 +63,9 @@ struct ygpu_ctx {
     uint64_t* d_big_b = nullptr;
     int big_buckets = 1;            // option: 0 = any oversized bucket sends the whole database to the general path
     uint32_t msd_big_buckets = 0;   // oversized buckets of the last build
+    int last_group2_grid = 0;       // grids of the last build's k2_group2 and k2_group launches, chunks of its oversized route (0: did not run)
+    int last_group_grid = 0;
+    uint32_t last_big_chunks = 0;
     uint16_t* d_st_rem = nullptr;   // [T] group stream of a hash-range sharded build: members of the same group that follow
     int index_path = 1;             // 1: MSD partition when the input qualifies, 0: always the general sort path
     int msd_fallbacks = 0;

@@ -1719,6 +1719,7 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
             kern2<<<grid2, G2_THREADS, smem2, st>>>(g);
             YG_CUDA(ctx, cudaGetLastError());
             ctx->tm.n_kernel_launches += 1;
+            ctx->last_group2_grid = grid2;
             g.m_lo = G2_MAXM;
         }
         if (nbk && (!fast2 || largest > G2_MAXM)) {
@@ -1731,6 +1732,7 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
             kern<<<grid, GK_THREADS, smem, st>>>(g);
             YG_CUDA(ctx, cudaGetLastError());
             ctx->tm.n_kernel_launches += 1;
+            ctx->last_group_grid = grid;
         }
         YG_CUDA(ctx, cudaEventRecord(ctx->evp[8], st));
     }
@@ -1776,6 +1778,7 @@ int msd_build(ygpu_ctx* ctx, ygpu_index_stats* S, int* used, bool partition_only
             YG_CUDA(ctx, cudaStreamSynchronize(st));      // `rel` is reused by the next chunk
         }
         ctx->msd_big_buckets = n_big;
+        ctx->last_big_chunks = (uint32_t)chunks.size();
     } else {
         ctx->msd_big_buckets = 0;
     }

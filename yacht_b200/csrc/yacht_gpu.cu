@@ -606,6 +606,9 @@ extern "C" int ygpu_build_index(ygpu_ctx* ctx, ygpu_index_stats* stats) {
     if (!ctx->loaded) return ygpu_fail(ctx, YGPU_ERR_STATE, "build_index: no sketches loaded");
     YG_CUDA(ctx, cudaSetDevice(ctx->device));
     release_index(ctx);
+    ctx->last_group2_grid = 0;
+    ctx->last_group_grid = 0;
+    ctx->last_big_chunks = 0;
     const uint64_t T = ctx->T;
     const uint32_t n = ctx->n;
     cudaStream_t st = ctx->stream;
@@ -1428,6 +1431,9 @@ extern "C" int ygpu_get_option(ygpu_ctx* ctx, const char* name, int64_t* out) {
     if (!strcmp(name, "last_count_tile_w")) { *out = ctx->last_count_tile_w; return 0; }
     if (!strcmp(name, "last_count_n_tiles")) { *out = ctx->last_count_n_tiles; return 0; }
     if (!strcmp(name, "last_count_u16")) { *out = ctx->last_count_u16; return 0; }
+    if (!strcmp(name, "last_group2_grid")) { *out = ctx->last_group2_grid; return 0; }
+    if (!strcmp(name, "last_group_grid")) { *out = ctx->last_group_grid; return 0; }
+    if (!strcmp(name, "last_big_chunks")) { *out = ctx->last_big_chunks; return 0; }
     return ygpu_fail(ctx, YGPU_ERR_ARG, "unknown option %s", name);
 }
 
