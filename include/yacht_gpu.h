@@ -97,7 +97,7 @@ typedef struct {
     /* sharded step: work-list build from the complete stream (k2_items_regions), the control collectives + cross-rank
      * waits between the phases, and the gather of the pair lists (inside ms_index / ms_pairsort)            */
     double ms_items, ms_sync, ms_gather;
-    double ms_sketch;       /* ygpu_sketch_sequences: the k-mer hashing kernel                                   */
+    double ms_sketch;       /* ygpu_sketch_sequences: the k-mer hashing kernel (_k: every size's)                 */
 } ygpu_timings;
 
 /* Per reference genome, from ygpu_exclusive_hashes (hypothesis_recovery_src.py:194-204). */
@@ -299,6 +299,13 @@ typedef struct {
 } ygpu_sketch_result;
 int ygpu_sketch_sequences(ygpu_ctx* ctx, const uint8_t* bases, uint64_t n_bases, const uint64_t* sketch_offsets,
                           uint32_t n_sketches, int ksize, uint64_t max_hash, uint32_t seed, ygpu_sketch_result* out);
+/* Several k-mer sizes of one batch: 1 to 8 distinct sizes in [1, 256] (otherwise YGPU_ERR_ARG, as ygpu_stream_begin_k).
+ * The batch is copied to the device once and every size is hashed and ordered on that copy; out[0 .. n_k), in the order
+ * of ksizes, each exactly what ygpu_sketch_sequences returns for that size alone (n_kmers included).  ms_h2d times the
+ * one copy, ms_sketch the sum of the sizes' hashing kernels.  ygpu_sketch_sequences is the n_k = 1 case.           */
+int ygpu_sketch_sequences_k(ygpu_ctx* ctx, const uint8_t* bases, uint64_t n_bases, const uint64_t* sketch_offsets,
+                            uint32_t n_sketches, const int* ksizes, int n_k, uint64_t max_hash, uint32_t seed,
+                            ygpu_sketch_result* out /* [n_k], order of ksizes */);
 void ygpu_sketch_result_free(ygpu_sketch_result* r);
 
 /* Streamed sketching of FASTA / FASTQ text of any size.  The raw (decompressed) text goes to the device in chunks of

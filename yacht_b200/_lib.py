@@ -26,7 +26,7 @@ ABI_SYMBOLS = [
     "ygpu_train_step_sharded", "ygpu_upload_finish_sharded", "ygpu_load_sketches_hashrange", "ygpu_load_sketches_hashrange_device",
     "ygpu_train_step_replicated", "ygpu_sketch_sequences", "ygpu_sketch_result_free",
     "ygpu_stream_begin", "ygpu_stream_feed", "ygpu_stream_end_file", "ygpu_stream_finish",
-    "ygpu_stream_begin_k", "ygpu_stream_finish_k",
+    "ygpu_stream_begin_k", "ygpu_stream_finish_k", "ygpu_sketch_sequences_k",
 ]
 STREAM_WHOLE, STREAM_PER_RECORD = 0, 1
 COMM_ID_BYTES = 128
@@ -64,6 +64,19 @@ class SketchResult(ctypes.Structure):
     _fields_ = [("hashes", ctypes.POINTER(ctypes.c_uint64)), ("abundances", ctypes.POINTER(ctypes.c_uint32)),
                 ("offsets", ctypes.POINTER(ctypes.c_uint64)), ("n_sketches", ctypes.c_uint32), ("_pad", ctypes.c_uint32),
                 ("n_kmers", ctypes.c_uint64)]
+
+
+def _sketch_result_arrays(res: SketchResult):
+    """(hashes, abundances, offsets, n_kmers) copied out of a library-owned result."""
+    ns = int(res.n_sketches)
+    offsets = np.ctypeslib.as_array(res.offsets, shape=(ns + 1,)).copy()
+    total = int(offsets[-1])
+    if total:
+        hashes = np.ctypeslib.as_array(res.hashes, shape=(total,)).copy()
+        abund = np.ctypeslib.as_array(res.abundances, shape=(total,)).copy()
+    else:
+        hashes, abund = np.zeros(0, np.uint64), np.zeros(0, np.uint32)
+    return hashes, abund, offsets, int(res.n_kmers)
 
 
 class StreamStats(ctypes.Structure):
@@ -154,6 +167,7 @@ def load_library() -> ctypes.CDLL:
     lib.ygpu_train_step_replicated.argtypes = [vp, ctypes.c_double, ctypes.POINTER(IndexStats), ctypes.POINTER(u64)]
     lib.ygpu_train_step_sharded.argtypes = [vp, ctypes.c_double, ctypes.POINTER(IndexStats), ctypes.POINTER(u64)]
     lib.ygpu_sketch_sequences.argtypes = [vp, vp, u64, vp, u32, ctypes.c_int, u64, u32, ctypes.POINTER(SketchResult)]
+    lib.ygpu_sketch_sequences_k.argtypes = [vp, vp, u64, vp, u32, vp, ctypes.c_int, u64, u32, ctypes.POINTER(SketchResult)]
     lib.ygpu_sketch_result_free.argtypes = [ctypes.POINTER(SketchResult)]
     lib.ygpu_sketch_result_free.restype = None
     lib.ygpu_stream_begin.argtypes = [vp, ctypes.c_int, u64, u32, ctypes.c_int]
@@ -368,17 +382,25 @@ class GpuContext:
         self._check(self.lib.ygpu_sketch_sequences(self.h, arr.ctypes.data if arr.size else None, arr.size, off.ctypes.data, off.shape[0] - 1,
                                                    int(ksize), int(max_hash), int(seed), ctypes.byref(res)), "ygpu_sketch_sequences")
         try:
-            ns = int(res.n_sketches)
-            offsets = np.ctypeslib.as_array(res.offsets, shape=(ns + 1,)).copy()
-            total = int(offsets[-1])
-            if total:
-                hashes = np.ctypeslib.as_array(res.hashes, shape=(total,)).copy()
-                abund = np.ctypeslib.as_array(res.abundances, shape=(total,)).copy()
-            else:
-                hashes, abund = np.zeros(0, np.uint64), np.zeros(0, np.uint32)
-            return hashes, abund, offsets, int(res.n_kmers)
+            return _sketch_result_arrays(res)
         finally:
             self.lib.ygpu_sketch_result_free(ctypes.byref(res))
+
+    def sketch_sequences_k(self, bases, sketch_offsets: Sequence[int], ksizes: Sequence[int], max_hash: int, seed: int = 42):
+        """`sketch_sequences` at several k-mer sizes with one upload of the batch (ygpu_sketch_sequences_k).
+        Returns [(hashes, abundances, offsets, n_kmers) per k-mer size, in the order of `ksizes`]."""
+        arr = np.frombuffer(bases, dtype=np.uint8) if isinstance(bases, (bytes, bytearray, memoryview)) else np.ascontiguousarray(bases, dtype=np.uint8)
+        off = np.ascontiguousarray(sketch_offsets, dtype=np.uint64)
+        ks = np.ascontiguousarray([int(k) for k in ksizes], dtype=np.int32)
+        res = (SketchResult * max(int(ks.size), 1))()
+        self._check(self.lib.ygpu_sketch_sequences_k(self.h, arr.ctypes.data if arr.size else None, arr.size, off.ctypes.data, off.shape[0] - 1,
+                                                     ks.ctypes.data if ks.size else None, int(ks.size), int(max_hash), int(seed), res),
+                    "ygpu_sketch_sequences_k")
+        try:
+            return [_sketch_result_arrays(r) for r in res[:int(ks.size)]]
+        finally:
+            for r in res:
+                self.lib.ygpu_sketch_result_free(ctypes.byref(r))
 
     # -- streamed sketching (ygpu_stream_*) ------------------------------------------------------
     def _stream_error(self, rc: int, what: str, path: Optional[str]) -> None:
@@ -428,17 +450,7 @@ class GpuContext:
         fn, what = (self.lib.ygpu_stream_finish, "ygpu_stream_finish") if nk is None else (self.lib.ygpu_stream_finish_k, "ygpu_stream_finish_k")
         self._stream_error(fn(self.h, res, ctypes.byref(st), ctypes.byref(names), ctypes.byref(name_off), ctypes.byref(n_names)), what, path)
         try:
-            per_k = []
-            for r in res:
-                ns = int(r.n_sketches)
-                offsets = np.ctypeslib.as_array(r.offsets, shape=(ns + 1,)).copy()
-                total = int(offsets[-1])
-                if total:
-                    hashes = np.ctypeslib.as_array(r.hashes, shape=(total,)).copy()
-                    abund = np.ctypeslib.as_array(r.abundances, shape=(total,)).copy()
-                else:
-                    hashes, abund = np.zeros(0, np.uint64), np.zeros(0, np.uint32)
-                per_k.append((hashes, abund, offsets, int(r.n_kmers)))
+            per_k = [_sketch_result_arrays(r) for r in res]
             out_names = None
             nn = int(n_names.value)
             if nn:

@@ -16,6 +16,7 @@
 //                   neighbours into (hash, first index); the host turns index differences into abundances.
 #include "common.cuh"
 #include "sketch_hash.cuh"
+#include "seq_stream.cuh"   // YSQ_MAX_K: the batch call takes as many k-mer sizes as the stream
 
 #include <cub/cub.cuh>
 #include <algorithm>
@@ -318,23 +319,12 @@ extern "C" void ygpu_sketch_result_free(ygpu_sketch_result* r) {
     memset(r, 0, sizeof *r);
 }
 
-extern "C" int ygpu_sketch_sequences(ygpu_ctx* ctx, const uint8_t* bases, uint64_t n_bases, const uint64_t* sketch_offsets,
-                                     uint32_t n_sketches, int ksize, uint64_t max_hash, uint32_t seed, ygpu_sketch_result* out) {
-    if (!ctx || !out || (!bases && n_bases) || !sketch_offsets || n_sketches == 0) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: bad argument");
-    if (ksize < 1 || ksize > SK_KMAX) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: ksize %d outside [1, %d]", ksize, SK_KMAX);
-    if (sketch_offsets[0] != 0 || sketch_offsets[n_sketches] != n_bases) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: sketch_offsets must run from 0 to n_bases");
-    for (uint32_t s = 0; s < n_sketches; s++)
-        if (sketch_offsets[s] > sketch_offsets[s + 1]) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: sketch_offsets must not decrease");
-    memset(out, 0, sizeof *out);
-    YG_CUDA(ctx, cudaSetDevice(ctx->device));
+namespace {
+
+// The batch and its sketch offsets to the context's resident buffers (d_bases zero-padded by SK_PAD), between ev[0] and ev[1].
+int sk_upload(ygpu_ctx* ctx, const uint8_t* bases, uint64_t n_bases, const uint64_t* sketch_offsets, uint32_t n_sketches) {
     SketchScratch* S = sk_scratch(ctx);
     cudaStream_t st = ctx->stream;
-
-    out->offsets = (uint64_t*)calloc((size_t)n_sketches + 1, sizeof(uint64_t));
-    if (!out->offsets) return ygpu_fail(ctx, YGPU_ERR_NOMEM, "out of host memory");
-    out->n_sketches = n_sketches;
-    if (n_bases < (uint64_t)ksize) return 0;                 // nothing to hash: n_sketches empty sketches
-
     YG_CHECK(dev_alloc(ctx, &S->d_bases, n_bases + SK_PAD));
     YG_CHECK(dev_alloc(ctx, &S->d_off, (uint64_t)n_sketches + 1));
     YG_CHECK(dev_alloc(ctx, &S->d_cnt, 2));
@@ -343,11 +333,20 @@ extern "C" int ygpu_sketch_sequences(ygpu_ctx* ctx, const uint8_t* bases, uint64
     YG_CUDA(ctx, cudaMemsetAsync(S->d_bases + n_bases, 0, SK_PAD, st));
     YG_CUDA(ctx, cudaMemcpyAsync(S->d_off, sketch_offsets, ((size_t)n_sketches + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, st));
     YG_CUDA(ctx, cudaEventRecord(ctx->ev[1], st));
+    return 0;
+}
 
+// One k-mer size on the uploaded batch: hash (ev[3] .. ev[2] brackets the kernel), order by (sketch id, hash),
+// de-duplicate, split per sketch on the host.  out->offsets is allocated and zero, out->n_sketches set; *ms_sketch gets
+// the kernel's time.
+int sk_hash_and_order(ygpu_ctx* ctx, uint64_t n_bases, uint32_t n_sketches, int ksize, uint64_t max_hash, uint32_t seed,
+                      ygpu_sketch_result* out, float* ms_sketch) {
+    SketchScratch* S = sk_scratch(ctx);
+    cudaStream_t st = ctx->stream;
     uint64_t m = 0, n_kmers = 0;
+    YG_CUDA(ctx, cudaEventRecord(ctx->ev[3], st));
     YG_CHECK(ygpu_sketch_hash_device(ctx, S->d_bases, n_bases, S->d_off, n_sketches, ksize, max_hash, seed, 0, ctx->ev[2], &m, &n_kmers));
-    ctx->tm.ms_h2d = elapsed(ctx, 0, 1);
-    ctx->tm.ms_sketch = elapsed(ctx, 1, 2);
+    *ms_sketch = elapsed(ctx, 3, 2);
     out->n_kmers = n_kmers;
     if (m == 0) return 0;
 
@@ -410,4 +409,59 @@ extern "C" int ygpu_sketch_sequences(ygpu_ctx* ctx, const uint8_t* bases, uint64
     }
     for (uint32_t s = 0; s < n_sketches; s++) out->offsets[s + 1] += out->offsets[s];
     return 0;
+}
+
+// The sizes' results on one upload of the batch.  out[] holds the zeroed offsets; the caller frees out[] on failure.
+int sk_sequences_k(ygpu_ctx* ctx, const uint8_t* bases, uint64_t n_bases, const uint64_t* sketch_offsets, uint32_t n_sketches,
+                   const int* ksizes, int n_k, int k_min, uint64_t max_hash, uint32_t seed, ygpu_sketch_result* out) {
+    if (n_bases < (uint64_t)k_min) return 0;                 // nothing to hash at any size: empty sketches
+    YG_CHECK(sk_upload(ctx, bases, n_bases, sketch_offsets, n_sketches));
+    double ms_sketch = 0.0;
+    for (int i = 0; i < n_k; i++) {
+        if (n_bases < (uint64_t)ksizes[i]) continue;          // no window of this size, as with that size alone
+        float ms = 0.f;
+        YG_CHECK(sk_hash_and_order(ctx, n_bases, n_sketches, ksizes[i], max_hash, seed, &out[i], &ms));
+        ms_sketch += ms;
+    }
+    ctx->tm.ms_h2d = elapsed(ctx, 0, 1);
+    ctx->tm.ms_sketch = ms_sketch;
+    return 0;
+}
+
+}  // namespace
+
+// One upload, every size hashed from it.  Each size is ordered on its own (no composite id), so out[k] is exactly the
+// result of ygpu_sketch_sequences at ksizes[k]; ms_h2d is the one copy, ms_sketch the sum of the sizes' kernel times.
+extern "C" int ygpu_sketch_sequences_k(ygpu_ctx* ctx, const uint8_t* bases, uint64_t n_bases, const uint64_t* sketch_offsets,
+                                       uint32_t n_sketches, const int* ksizes, int n_k, uint64_t max_hash, uint32_t seed,
+                                       ygpu_sketch_result* out) {
+    if (!ctx || !out || (!bases && n_bases) || !sketch_offsets || n_sketches == 0) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: bad argument");
+    if (!ksizes || n_k < 1 || n_k > YSQ_MAX_K) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: %d k-mer sizes (1 to %d)", n_k, YSQ_MAX_K);
+    int k_min = SK_KMAX;
+    for (int i = 0; i < n_k; i++) {
+        if (ksizes[i] < 1 || ksizes[i] > SK_KMAX) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: ksize %d outside [1, %d]", ksizes[i], SK_KMAX);
+        for (int j = 0; j < i; j++)
+            if (ksizes[j] == ksizes[i]) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: ksize %d given twice", ksizes[i]);
+        k_min = std::min(k_min, ksizes[i]);
+    }
+    if (sketch_offsets[0] != 0 || sketch_offsets[n_sketches] != n_bases) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: sketch_offsets must run from 0 to n_bases");
+    for (uint32_t s = 0; s < n_sketches; s++)
+        if (sketch_offsets[s] > sketch_offsets[s + 1]) return ygpu_fail(ctx, YGPU_ERR_ARG, "ygpu_sketch_sequences: sketch_offsets must not decrease");
+    memset(out, 0, n_k * sizeof *out);
+    YG_CUDA(ctx, cudaSetDevice(ctx->device));
+    int rc = 0;
+    for (int i = 0; i < n_k && rc == 0; i++) {
+        out[i].offsets = (uint64_t*)calloc((size_t)n_sketches + 1, sizeof(uint64_t));
+        out[i].n_sketches = n_sketches;
+        if (!out[i].offsets) rc = ygpu_fail(ctx, YGPU_ERR_NOMEM, "out of host memory");
+    }
+    if (rc == 0) rc = sk_sequences_k(ctx, bases, n_bases, sketch_offsets, n_sketches, ksizes, n_k, k_min, max_hash, seed, out);
+    if (rc != 0)
+        for (int i = 0; i < n_k; i++) ygpu_sketch_result_free(&out[i]);
+    return rc;
+}
+
+extern "C" int ygpu_sketch_sequences(ygpu_ctx* ctx, const uint8_t* bases, uint64_t n_bases, const uint64_t* sketch_offsets,
+                                     uint32_t n_sketches, int ksize, uint64_t max_hash, uint32_t seed, ygpu_sketch_result* out) {
+    return ygpu_sketch_sequences_k(ctx, bases, n_bases, sketch_offsets, n_sketches, &ksize, 1, max_hash, seed, out);
 }

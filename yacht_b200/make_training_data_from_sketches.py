@@ -52,7 +52,8 @@ def main(args):
 
     _log("INFO", "Unzipping the sourmash signature file to the temporary directory")
     # reference :109-119 (extractall, gunzip pool, collect_signature_info) as ONE parallel pass over the zip members
-    sig_info_dict = utils.extract_signatures_and_info(ref_file, path_to_temp_dir, ksize, num_threads)
+    # signatures of other k-mer sizes (a zip sketched at several sizes) are extracted too but stay out of the comparison
+    sig_info_dict, other_size_files = utils.extract_signatures(ref_file, path_to_temp_dir, ksize, num_threads)
     _log("INFO", "Checking if all signatures have the same scaled")
     scale_set = set([value[-2] for value in sig_info_dict.values()])
     if len(scale_set) != 1:
@@ -61,7 +62,8 @@ def main(args):
 
     _log("INFO", "Finding the closely related genomes with ANI > ani_thresh from the reference database, then remove them, "
                  "and generate a dataframe with the selected genomes.")
-    manifest_df = utils.run_yacht_train_core(num_threads, ani_thresh, ksize, path_to_temp_dir, sig_info_dict)
+    manifest_df = utils.run_yacht_train_core(num_threads, ani_thresh, ksize, path_to_temp_dir, sig_info_dict,
+                                             other_size_files=other_size_files)
 
     _log("INFO", "Writing out the manifest file")
     manifest_file_path = os.path.join(outdir, f"{prefix}_processed_manifest.tsv")

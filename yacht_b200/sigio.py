@@ -168,11 +168,11 @@ def sig_info(sig_file: str, ksize: int):
         return None
 
 
-def sig_info_from_text(text: str, sig_file: str, ksize: int):
-    """:func:`sig_info` for a signature document that is already in memory (`sig_file` is the path it was, or is
-    being, written to): same selection rule -- exactly one non-empty sketch of that k-mer size -- same tuple."""
+def sig_info_from_signatures(signatures: Sequence[Signature], sig_file: str, ksize: int):
+    """:func:`sig_info` for a signature document already parsed by :func:`parse_signature_json` (`sig_file` is the path
+    it was, or is being, written to): same selection rule -- exactly one non-empty sketch of that k-mer size -- same tuple."""
     try:
-        sigs = [s for s in parse_signature_json(text, sig_file) if s.ksize == ksize]
+        sigs = [s for s in signatures if s.ksize == ksize]
         if len(sigs) != 1 or len(sigs[0]) == 0:
             return None
         sig = sigs[0]

@@ -7,6 +7,7 @@ There is no CPU hashing path: without the library and a GPU these functions rais
 """
 from __future__ import annotations
 
+import argparse
 import gzip
 import os
 import queue
@@ -33,16 +34,29 @@ def _context() -> _lib.GpuContext:
     return _ctx
 
 
+def kmer_list(text: str):
+    """Type of `sketch ref --kmer`: one k-mer size ("31" -> 31) or a comma-separated list of them ("21,31,51" ->
+    [21, 31, 51]).  The option takes one command-line word, so `--kmer 21 31` stays an unrecognized argument."""
+    try:
+        sizes = [int(part) for part in text.split(",")]
+    except ValueError:
+        raise argparse.ArgumentTypeError(f"expected a k-mer size or a comma-separated list of sizes (21,31,51), got {text!r}")
+    return sizes[0] if len(sizes) == 1 else sizes
+
+
 def add_cli_arguments(parser, infile_help: str, nargs=None, multi_kmer: bool = False) -> None:
     """The four options both `yacht sketch` sub-commands take (names and defaults of the reference's wrappers).
-    With `multi_kmer`, --kmer takes one or more values and is always a list (default [31])."""
+    With `multi_kmer`, --kmer takes one or more values and is always a list (default [31]); without it, --kmer is one
+    word, a size or a comma-separated list of sizes (`kmer_list`)."""
     kw = {"nargs": nargs} if nargs else {}
     parser.add_argument("--infile", help=infile_help, required=True, **kw)
     if multi_kmer:
         parser.add_argument("--kmer", type=int, nargs="+", default=[31],
                             help="K-mer size(s). Several distinct sizes are sketched in one pass into one output file.")
     else:
-        parser.add_argument("--kmer", type=int, default=31, help="K-mer size.")
+        parser.add_argument("--kmer", type=kmer_list, default=31,
+                            help="K-mer size, or several comma-separated (21,31,51): every file is read once and sketched at "
+                                 "each size into one output file.")
     parser.add_argument("--scaled", type=int, default=1000, help="Scaled factor.")
     parser.add_argument("--outfile", help="Output file name.", required=True)
 
@@ -176,25 +190,39 @@ def sketch_stream(paths: Sequence[str], ksize, scaled: int, per_record: bool = F
     return [split(h, a, o) for h, a, o, _ in per_k], names
 
 
-def sketch_record_groups(groups: Sequence[Sequence[bytes]], ksize: int, scaled: int, seed: int = SEED):
+def kmer_sizes(kmer) -> List[int]:
+    """--kmer as a list (the command line gives one; a caller that builds the namespace itself may pass one int).
+    Refuses a size given twice."""
+    kmers = [int(k) for k in kmer] if isinstance(kmer, (list, tuple)) else [int(kmer)]
+    dup = sorted({k for k in kmers if kmers.count(k) > 1})
+    if dup:
+        raise ValueError(f"--kmer: k-mer size(s) {', '.join(map(str, dup))} given more than once.")
+    return kmers
+
+
+def sketch_record_groups(groups: Sequence[Sequence[bytes]], ksize, scaled: int, seed: int = SEED):
     """One sketch per group of records.  Returns [(mins uint64 ascending, abundances uint32)] in group order.
     Groups are packed into device calls of at most BATCH_BASES bytes; a group larger than that is split over calls and its
-    partial sketches are merged (hashes united, abundances added)."""
+    partial sketches are merged (hashes united, abundances added).
+    With a sequence of k-mer sizes for `ksize` every batch is joined and uploaded once and hashed at each size
+    (ygpu_sketch_sequences_k); the result is then [[(mins, abundances)] per group] per k, in the order given."""
     ctx = _context()
     max_hash = max_hash_for_scaled(scaled)
-    out: List[Optional[Tuple[np.ndarray, np.ndarray]]] = [None] * len(groups)
+    multi = not isinstance(ksize, (int, np.integer))
+    ks = list(ksize) if multi else [ksize]
+    out: List[List[Optional[Tuple[np.ndarray, np.ndarray]]]] = [[None] * len(groups) for _ in ks]
 
-    def merge(gi, mins, ab):
-        if out[gi] is None:
-            out[gi] = (mins, ab)
+    def merge(ki, gi, mins, ab):
+        if out[ki][gi] is None:
+            out[ki][gi] = (mins, ab)
             return
-        m0, a0 = out[gi]
+        m0, a0 = out[ki][gi]
         allm = np.concatenate([m0, mins])
         alla = np.concatenate([a0, ab]).astype(np.uint64)
         um, inv = np.unique(allm, return_inverse=True)
         ua = np.zeros(um.shape[0], dtype=np.uint64)
         np.add.at(ua, inv, alla)
-        out[gi] = (um, ua.astype(np.uint32))
+        out[ki][gi] = (um, ua.astype(np.uint32))
 
     batch_parts: List[bytes] = []
     batch_ids: List[int] = []          # group id of every sketch range of the batch
@@ -205,10 +233,15 @@ def sketch_record_groups(groups: Sequence[Sequence[bytes]], ksize: int, scaled: 
         nonlocal batch_parts, batch_ids, batch_offs, size
         if not batch_ids:
             return
-        hashes, abund, offs, _ = ctx.sketch_sequences(b"".join(batch_parts), batch_offs, ksize, max_hash, seed)
-        for j, gi in enumerate(batch_ids):
-            lo, hi = int(offs[j]), int(offs[j + 1])
-            merge(gi, hashes[lo:hi], abund[lo:hi])
+        bases = b"".join(batch_parts)
+        if multi:
+            per_k = ctx.sketch_sequences_k(bases, batch_offs, ks, max_hash, seed)
+        else:
+            per_k = [ctx.sketch_sequences(bases, batch_offs, ksize, max_hash, seed)]
+        for ki, (hashes, abund, offs, _) in enumerate(per_k):
+            for j, gi in enumerate(batch_ids):
+                lo, hi = int(offs[j]), int(offs[j + 1])
+                merge(ki, gi, hashes[lo:hi], abund[lo:hi])
         batch_parts, batch_ids, batch_offs, size = [], [], [0], 0
 
     for gi, recs in enumerate(groups):
@@ -231,26 +264,40 @@ def sketch_record_groups(groups: Sequence[Sequence[bytes]], ksize: int, scaled: 
         size = batch_offs[-1]
     flush()
     empty = (np.zeros(0, np.uint64), np.zeros(0, np.uint32))
-    return [o if o is not None else empty for o in out]
+    per_k = [[o if o is not None else empty for o in out_k] for out_k in out]
+    return per_k if multi else per_k[0]
 
 
-def sketch_files(paths: Sequence[str], ksize: int, scaled: int, singleton: bool = False, names: Optional[Sequence[str]] = None,
+def sketch_files(paths: Sequence[str], ksize, scaled: int, singleton: bool = False, names: Optional[Sequence[str]] = None,
                  threads: Optional[int] = None):
     """Sketch dicts ({name, filename, mins, abundances}) ready for sigio.write_sig_zip: one per file (all records together,
     like ``sourmash sketch fromfile`` / ``sketch dna``) or, with ``singleton``, one per record (``--singleton``).
-    Files are taken in chunks of ~CHUNK_FILE_BYTES on disk so that a large collection never sits in host memory at once."""
+    Files are taken in chunks of ~CHUNK_FILE_BYTES on disk so that a large collection never sits in host memory at once.
+    With a sequence of k-mer sizes for `ksize` every file is read once and there is one dict per (file or record, size),
+    file- or record-major and sizes in the order given, each with its own ``"ksize"``."""
     threads = max(1, int(threads or os.cpu_count() or 1))
+    multi = not isinstance(ksize, (int, np.integer))
     out: List[dict] = []
+
+    def emit(name, filename, per_k):
+        """per_k: [(mins, abundances)] per size (one entry for a single size)."""
+        if not multi:
+            [(mins, ab)] = per_k
+            out.append({"name": name, "filename": filename, "mins": mins, "abundances": ab})
+            return
+        out.extend({"name": name, "filename": filename, "mins": mins, "abundances": ab, "ksize": k}
+                   for k, (mins, ab) in zip(ksize, per_k))
+
     i = 0
     while i < len(paths):
         if is_streamed(paths[i]):       # a large file: parsed on the device, never held in host memory
             sketches, rec_names = sketch_stream([paths[i]], ksize, scaled, per_record=singleton)
+            per_k = sketches if multi else [sketches]     # [[(mins, ab)] per sketch] per size
             if singleton:
-                out.extend({"name": name, "filename": paths[i], "mins": mins, "abundances": ab}
-                           for name, (mins, ab) in zip(rec_names, sketches))
+                for r, name in enumerate(rec_names):
+                    emit(name, paths[i], [sk[r] for sk in per_k])
             else:
-                [(mins, ab)] = sketches
-                out.append({"name": names[i] if names is not None else "", "filename": paths[i], "mins": mins, "abundances": ab})
+                emit(names[i] if names is not None else "", paths[i], [sk[0] for sk in per_k])
             i += 1
             continue
         j, size = i, 0
@@ -277,8 +324,9 @@ def sketch_files(paths: Sequence[str], ksize: int, scaled: int, singleton: bool 
                 meta.append((names[i + k] if names is not None else "", path))
         del all_recs
         sketches = sketch_record_groups(groups, ksize, scaled)
-        out.extend({"name": name, "filename": filename, "mins": mins, "abundances": ab}
-                   for (name, filename), (mins, ab) in zip(meta, sketches))
+        per_k = sketches if multi else [sketches]
+        for g, (name, filename) in enumerate(meta):
+            emit(name, filename, [sk[g] for sk in per_k])
         i = j
     return out
 

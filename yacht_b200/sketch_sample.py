@@ -42,11 +42,7 @@ def main(args):
     files = list(args.infile)
     if len(files) not in (1, 2):
         raise ValueError("Please provide either one file for single-end reads or two files for paired-end reads.")
-    # the command line gives a list; a caller that builds the namespace itself may still pass one int
-    kmers = list(args.kmer) if isinstance(args.kmer, (list, tuple)) else [args.kmer]
-    dup = sorted({k for k in kmers if kmers.count(k) > 1})
-    if dup:
-        raise ValueError(f"--kmer: k-mer size(s) {', '.join(map(str, dup))} given more than once.")
+    kmers = sketch.kmer_sizes(args.kmer)
     kind = "a single-end FASTA/Q file" if len(files) == 1 else "paired-end FASTA/Q files"
     _log("INFO", f"Starting sketching {kind}: {' '.join(files)}")
     if len(kmers) == 1:

@@ -19,7 +19,7 @@ import shutil
 import sys
 from glob import glob
 from multiprocessing import Pool
-from typing import Dict, List, Optional, Tuple
+from typing import Collection, Dict, List, Optional, Tuple
 
 import numpy as np
 import pandas as pd
@@ -99,16 +99,25 @@ def _extract_chunk(args):
         with open(target, "wb") as f:
             f.write(raw)
         try:
-            text = raw.decode()
-        except UnicodeDecodeError:
-            text = None
-        info = sigio.sig_info_from_text(text, target, ksize) if text is not None else None
-        out.append((target, info))
+            sigs = sigio.parse_signature_json(raw.decode(), target)
+        except Exception:                                         # not text, not JSON, not a signature document
+            sigs = None
+        info = sigio.sig_info_from_signatures(sigs, target, ksize) if sigs is not None else None
+        other_size = bool(sigs) and all(sig.ksize != ksize for sig in sigs)
+        out.append((target, info, other_size))
     return out
 
 
 def extract_signatures_and_info(ref_zip: str, path_to_temp_dir: str, ksize: int, num_threads: int) -> Dict[str, Tuple[str, float, int, int, str]]:
     """Unzip + gunzip + collect_signature_info in one parallel pass; returns what collect_signature_info returns."""
+    return extract_signatures(ref_zip, path_to_temp_dir, ksize, num_threads)[0]
+
+
+def extract_signatures(ref_zip: str, path_to_temp_dir: str, ksize: int, num_threads: int):
+    """:func:`extract_signatures_and_info`, and the names (under signatures/) of the extracted files that are signatures
+    of other k-mer sizes only: they parse, hold at least one sketch and none of size `ksize`.  A zip sketched at several
+    sizes holds one such file per genome and extra size; :func:`run_yacht_train_core` leaves them out of the train core's
+    file list, which would otherwise compare them too."""
     with zipfile.ZipFile(ref_zip, "r") as z:
         names = z.namelist()
         sig_members = [n for n in names if n.startswith("signatures/") and not n.endswith("/") and "/" not in n[len("signatures/"):]]
@@ -128,13 +137,18 @@ def extract_signatures_and_info(ref_zip: str, path_to_temp_dir: str, ksize: int,
     else:
         parts = [_extract_chunk(j) for j in jobs]
     info = {}
+    other_size = set()
     for part in parts:
-        for target, sig in part:
+        for target, sig, other in part:
             if sig:
                 info[sig[1]] = (sig[2], sig[3], sig[4], sig[5], sig[0])
+            elif other:
+                other_size.add(os.path.basename(target))
             else:
                 _log("WARNING", f"CANNOT extract the relevant info from the signature file: {target}")
-    return info
+    if other_size:
+        _log("INFO", f"Leaving out {len(other_size)} signature files without a k-mer size {ksize} sketch (other k-mer sizes)")
+    return info, other_size
 
 
 def _gunzip_one(path: str) -> str:
@@ -159,11 +173,14 @@ def decompress_all_sig_files(sig_files: List[str], num_threads: int) -> None:
 
 def run_yacht_train_core(num_threads: int, ani_thresh: float, ksize: int, path_to_temp_dir: str,
                          sig_info_dict: Dict[str, Tuple[str, float, int, int, str]],
-                         num_genome_threshold: int = 1000000) -> pd.DataFrame:
+                         num_genome_threshold: int = 1000000, other_size_files: Collection[str] = ()) -> pd.DataFrame:
     """utils.py:112-197, verbatim semantics: write the file list, convert ANI to containment, launch
-    the core executable, move the pair files, keep the manifest rows of the selected genomes."""
+    the core executable, move the pair files, keep the manifest rows of the selected genomes.
+    `other_size_files` (names under signatures/, from :func:`extract_signatures`) stay out of the file list: the
+    signatures of other k-mer sizes of a multi-size zip, which the reference lists too and then fails on."""
     sig_files = pd.DataFrame(
-        [os.path.join(path_to_temp_dir, "signatures", file) for file in os.listdir(os.path.join(path_to_temp_dir, "signatures"))]
+        [os.path.join(path_to_temp_dir, "signatures", file) for file in os.listdir(os.path.join(path_to_temp_dir, "signatures"))
+         if file not in other_size_files]
     )
     sig_files_path = os.path.join(path_to_temp_dir, "training_sig_files.tsv")
     sig_files.to_csv(sig_files_path, header=False, index=False)
